@@ -28,6 +28,8 @@ Printed JSON (one line, rank 0):
   fused_rollout, sweep   extra measurements (in-kernel policy; other env counts, eager and CUDA-graph replay)
 `--impl reference` times the UNMODIFIED reference (byte-compiled in oracle/_ref) with one
 process per host core; it never touches CUDA.
+`--dump-outputs DIR` writes what the last timed step returned (rank 0's envs) as DIR/<name>.npy; the inputs depend
+on the arguments only, so two builds run with the same arguments can be compared array by array.
 """
 import argparse
 import json
@@ -48,6 +50,7 @@ UNIT = "env-steps/s"
 SCHED = dict(success_rate_threshold=0.3, window_size=15, min_episodes_before_progression=20, progression_steps=5)
 MAX_EPISODE_STEPS = 200
 SEED = 42
+DUMP_ROWS = 1 << 17                    # --dump-outputs: ~34 MB of arrays at this many envs, under the 64 MB budget
 
 
 def parse_args():
@@ -72,7 +75,13 @@ def parse_args():
                     help="reference arm: env-steps per process per bench step (0 = size from --ref-budget-seconds)")
     ap.add_argument("--ref-budget-seconds", type=float, default=120.0, help="reference arm: target wall time of the whole run")
     ap.add_argument("--ref-procs", type=int, default=0, help="reference arm: processes (0 = all host cores)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the observation, reward, flags and info arrays of the last timed step as DIR/<name>.npy "
+                         f"(rank 0's envs; a fixed, seeded sample of {DUMP_ROWS} envs above that count)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ------------------------------------------------------------------------------------ reference arm
@@ -268,6 +277,33 @@ class ClockSampler:
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": mx, "samples": len(sm), "reasons": sorted(reasons)}
 
 
+# ------------------------------------------------------------------------------------ output dump
+def dump_outputs(out_dir, step_out, n):
+    """Write what env.step() returned -- observation, reward, flags and every info array -- as <out_dir>/<name>.npy for
+    the same fixed, seeded sample of env rows (all n when n <= DUMP_ROWS; env_index.npy lists them).  float64 arrays
+    stay float64, the others are written as float32 (flags and counts are small integers, exact in float32)."""
+    import numpy as np
+    import torch
+    obs, reward, terminated, truncated, info = step_out
+    arrays = {"obs": obs, "reward": reward, "terminated": terminated, "truncated": truncated}
+
+    def add(prefix, d):
+        for k, v in d.items():
+            if isinstance(v, dict):
+                add(f"{prefix}{k}_", v)
+            else:
+                arrays[prefix + k] = v
+    add("info_", info)
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(SEED).choice(n, DUMP_ROWS, replace=False))
+    idx = torch.from_numpy(rows).to(obs.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), rows.astype(np.float64))
+    for name, t in arrays.items():
+        a = t.index_select(0, idx).cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
+    print(f"bench.py: wrote {len(arrays) + 1} arrays ({len(rows)} envs) to {out_dir}", file=sys.stderr)
+
+
 # ------------------------------------------------------------------------------------ b200 arm
 def run_b200(args):
     import torch
@@ -345,7 +381,7 @@ def run_b200(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for t in range(steps):
-            env.step(pool[t % len(pool)])
+            out = env.step(pool[t % len(pool)])
             maybe_poll(t)
         e1.record()
         barrier()
@@ -354,7 +390,7 @@ def run_b200(args):
             tms = torch.tensor([ms], device=dev, dtype=torch.float64)
             dist.all_reduce(tms, op=dist.ReduceOp.MAX)
             ms = float(tms.item())
-        return ms
+        return ms, out
 
     # ---- main timed region: API mode, device-resident actions -------------------------------------
     env, sched, drv = make_env(E, gid0=rank * E)
@@ -362,8 +398,10 @@ def run_b200(args):
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
-    ms = timed_api(env, drv, pool, args.steps, args.warmup, args.poll_every)
+    ms, last_out = timed_api(env, drv, pool, args.steps, args.warmup, args.poll_every)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_out, E)      # before any later step overwrites the output buffers
     value = E * n_gpus * args.steps / (ms * 1e-3)
     launches = args.steps
 
@@ -382,7 +420,7 @@ def run_b200(args):
     # sustained figure: the same loop continued for >= 400 steps (two full 200-step episode cycles with their reset
     # waves and curriculum polls), so that a short --steps window can neither flatter nor hide it
     sus_steps = max(int(args.sustained_steps), 1)
-    ms_sus = timed_api(env, drv, pool, sus_steps, 0, args.poll_every, preroll=False)
+    ms_sus, _ = timed_api(env, drv, pool, sus_steps, 0, args.poll_every, preroll=False)
     k_ms_sus = ms_sus / sus_steps
     # measured DRAM traffic of this kernel (ncu, per launch) -- only quoted while the library is still built from the
     # sources it was measured on
@@ -422,7 +460,7 @@ def run_b200(args):
     if not args.no_tracking_variant:
         env_t, _, drv_t = make_env(E, gid0=rank * E, track=True)
         t_steps = max(250, args.steps // 4)
-        ms_t = timed_api(env_t, drv_t, pool, t_steps, max(args.warmup, 3), args.poll_every)
+        ms_t, _ = timed_api(env_t, drv_t, pool, t_steps, max(args.warmup, 3), args.poll_every)
         tracking_full = {"value": E * n_gpus * t_steps / (ms_t * 1e-3), "ms_per_step": ms_t / t_steps, "steps": t_steps,
                          "roofline_frac": ALGO_BYTES_PER_ENV_STEP * E / (ms_t / t_steps * 1e-3) / 1e9 / peak,
                          "note": "track_episodes=True: +32 B/env-step of per-env return / history traffic that the "
@@ -591,7 +629,7 @@ def run_b200(args):
                 continue
             env_s, _, drv_s = make_env(n)
             pool_s = action_pool(n)
-            s_ms = timed_api(env_s, drv_s, pool_s, 300, 120, 100)
+            s_ms, _ = timed_api(env_s, drv_s, pool_s, 300, 120, 100)
             v = n * 300 / (s_ms * 1e-3)
             # the same API step replayed from a CUDA graph (8 steps per replay over the same four action tensors as the
             # eager loop, so that both see the same working set in L2): removes the host launch path

@@ -7,7 +7,7 @@ Run in the build container only (needs /root/reference or oracle/_ref):
 The reference is imported under oracle/gym_stub (gymnasium is not installed in the image);
 numpy 2.3.5 / NEP 50 promotion is part of the pinned behaviour (SURVEY.md Appendix A-16).
 Outputs (committed):
-    traj.npz     per-step obs / reward / components / flags for 32 trajectories
+    traj.npz     per-step obs / reward / components / flags for 30 trajectories
     noise.npz    CombinedNoiseWrapper trajectories with the wrapper's normal draws recorded
     labels.npz   both failure classifiers on synthetic episodes (ties included)
     episodes.npz Evaluator.evaluate_episode / run_episode records with the policy's actions
@@ -101,8 +101,14 @@ def gen_traj():
         terminated=np.asarray(out["terminated"], bool), truncated=np.asarray(out["truncated"], bool),
         num_contacts=np.asarray(out["num_contacts"], np.uint8), op_final=np.asarray(out["op_final"], np.float64),
         names=np.asarray(names))
+    # The seed-2 trajectories are left out to keep the file under 1 MB.  The other 30 still cover every configuration,
+    # both reward types, all four action styles, both episode limits and every reused-env (chained) episode.
+    keep = np.array([i for i, name in enumerate(names) if "/seed2/" not in name])
+    remap = {int(old): new for new, old in enumerate(keep)}
+    arr = {k: v[keep] for k, v in arr.items()}
+    arr["chain"] = np.asarray([remap[int(c)] if c >= 0 else -1 for c in arr["chain"]], np.int32)
     np.savez_compressed(os.path.join(HERE, "traj.npz"), **arr)
-    print("traj.npz:", len(names), "trajectories x", T_STEPS, "steps;",
+    print("traj.npz:", len(keep), "trajectories x", T_STEPS, "steps;",
           "terminated steps:", int(arr["terminated"].sum()), "truncated steps:", int(arr["truncated"].sum()))
 
 

@@ -1458,15 +1458,16 @@ def test_fuzz_extreme_inputs_match_oracle(dx):
                 np.testing.assert_allclose(r[fin], orr[fin], rtol=REWARD_RTOL, atol=REWARD_ATOL)
 
 
-def test_bench_b200_arm_prints_one_contract_line():
+def test_bench_b200_arm_prints_one_contract_line(tmp_path):
     """bench.py (a short run at a reduced env count): exactly one JSON line on stdout carrying every key of the
-    bench contract, the roofline and the end-to-end object."""
+    bench contract, the roofline and the end-to-end object; --dump-outputs writes the last timed step's arrays."""
     import json
     import subprocess
     import sys
     root = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
+    dump = tmp_path / "outputs"
     proc = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "20", "--warmup", "3", "--num-envs", "262144",
-                           "--e2e-steps", "3", "--no-sweep", "--no-cpu-baseline", "--no-tracking-variant"],
+                           "--e2e-steps", "3", "--no-sweep", "--no-cpu-baseline", "--no-tracking-variant", "--dump-outputs", str(dump)],
                           capture_output=True, text=True, timeout=300)
     assert proc.returncode == 0, proc.stderr[-2000:]
     lines = [ln for ln in proc.stdout.splitlines() if ln.strip()]
@@ -1490,6 +1491,41 @@ def test_bench_b200_arm_prints_one_contract_line():
     assert e["value"] > 0 and e["h2d_bytes_per_step"] == 262144 * 60 and e["d2h_bytes_per_step"] == 262144 * (32 * 4 + 8)
     assert e["all_rows_d2h_bytes_per_step"] == 262144 * (41 * 4 + 7) and e["copy_ceiling"]["value"] > e["value"] * 0.8
     assert e["value"] < d["value"]                       # host buffers cross PCIe: never faster than the device-resident loop
+    # one seeded sample of 131,072 of the 262,144 envs, the same rows in every array, float32 / float64 only, <= 64 MB
+    files = {p.stem: np.load(p) for p in dump.iterdir()}
+    rows = files["env_index"].astype(np.int64)
+    assert len(rows) == 131072 and np.all(np.diff(rows) > 0) and rows[-1] < 262144
+    assert files["obs"].shape == (131072, 45) and files["info_object_position"].shape == (131072, 3)
+    for name in ("reward", "terminated", "truncated", "info_num_contacts", "info_step_count", "info_finished"):
+        assert files[name].shape == (131072,), name
+    assert all(a.dtype in (np.float32, np.float64) for a in files.values())
+    assert sum(p.stat().st_size for p in dump.iterdir()) <= 64 << 20
+    assert files["info_step_count"].max() <= 200 and np.isfinite(files["obs"]).all()
+
+
+def test_bench_dump_outputs_repeat_and_come_from_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs at 4,096 envs (every env written, no sampling): two runs with the same arguments write
+    bit-identical arrays, and the step counters are those after the last timed step -- with no pre-roll, 2 warm-up and
+    3 timed steps the envs that have not reset yet stand at step 5."""
+    import subprocess
+    import sys
+    root = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
+    runs = []
+    for k in range(2):
+        dump = tmp_path / f"run{k}"
+        proc = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--num-envs", "4096", "--preroll-steps", "0",
+                               "--warmup", "2", "--steps", "3", "--sustained-steps", "10", "--e2e-steps", "3", "--no-strong",
+                               "--no-sweep", "--no-cpu-baseline", "--no-tracking-variant", "--dump-outputs", str(dump)],
+                              capture_output=True, text=True, timeout=300)
+        assert proc.returncode == 0, proc.stderr[-2000:]
+        runs.append({p.stem: np.load(p) for p in dump.iterdir()})
+    a, b = runs
+    assert sorted(a) == sorted(b) and len(a) >= 10
+    for name in a:
+        assert a[name].dtype == b[name].dtype and np.array_equal(a[name], b[name], equal_nan=True), name
+    assert np.array_equal(a["env_index"], np.arange(4096)) and a["obs"].shape == (4096, 45)
+    steps = a["info_step_count"]
+    assert steps.min() >= 0 and steps.max() == 2 + 3
 
 
 def test_object_position_attribute_follows_the_reference(dx):
