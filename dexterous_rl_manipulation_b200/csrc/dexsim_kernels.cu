@@ -1252,7 +1252,7 @@ int dexsim_fill_normal(const DexsimState* st, const DexsimParams* p, int32_t rng
     int rc = check_state(st);
     if (rc) return rc;
     if (!p || !out) return DEXSIM_E_NULL;
-    if (rng_stream != (int)STREAM_DYN && rng_stream != (int)STREAM_OBS) return DEXSIM_E_PARAM;
+    if (rng_stream < (int)STREAM_DYN || rng_stream > (int)STREAM_LEARNER_UPD) return DEXSIM_E_PARAM;
     if (rows != NJ && rows != NOBS) return DEXSIM_E_PARAM;
     if (st->n == 0) return 0;
     const int grid = (int)((st->n + 255) / 256 > 65535 ? 65535 : (st->n + 255) / 256);

@@ -321,7 +321,8 @@ int dexsim_step_single(const DexsimState* st, const DexsimParams* p, const Dexsi
 int dexsim_fill_policy_actions(const DexsimState* st, const DexsimParams* p, int32_t policy_kind,
                                float* actions /* [15, ld] for each env's CURRENT (episode, step) */,
                                void* stream);
-int dexsim_fill_normal(const DexsimState* st, const DexsimParams* p, int32_t rng_stream /* 2 dyn, 3 obs */,
+int dexsim_fill_normal(const DexsimState* st, const DexsimParams* p,
+                       int32_t rng_stream /* 2 dyn, 3 obs, 4 learner exploration, 5 learner update */,
                        int32_t rows /* 15 or 45 */, float sigma, float* out /* [rows, ld] */, void* stream);
 
 /* ---- failure labels from episode summaries: replaces EvaluationMetrics.classify_failure

@@ -360,7 +360,8 @@ int32_t dexo_classify_taxonomy(int32_t success, int32_t episode_steps, int32_t n
  * Philox4x32-10 (Salmon et al., SC'11; same constants as Random123 / cuRAND).  The device
  * implements this specification independently; DESIGN.md "RNG" is the shared definition.
  *   key = (seed lo, seed hi);  counter = (env global id, episode, step, stream | block << 8)
- *   streams: 0 reset, 1 policy, 2 dynamics noise, 3 observation noise, 4 learner          */
+ *   streams: 0 reset, 1 policy, 2 dynamics noise, 3 observation noise, 4 learner exploration,
+ *   5 learner update                                                                        */
 void dexo_philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]) {
     uint32_t c0 = ctr[0], c1 = ctr[1], c2 = ctr[2], c3 = ctr[3];
     uint32_t k0 = key[0], k1 = key[1];
@@ -421,6 +422,37 @@ void dexo_policy_action(uint64_t seed, uint32_t env_gid, uint32_t episode, uint3
             action[j] = clip_f32(-0.5f + noise, -1.0f, 1.0f);
         } else {
             action[j] = u;
+        }
+    }
+}
+
+/* Box-Muller normals (streams 2-5), in double precision on the spec's exact inputs (DESIGN.md "RNG"):
+ *   u1 = ((wa >> 8) + 1)·2^-24 in (0, 1],  u2 = (wb >> 8)·2^-24,  theta = 2·pi·(u2 - 1/2)
+ *   z0 = sqrt(-2 ln u1)·cos(theta),  z1 = sqrt(-2 ln u1)·sin(theta)
+ * The device evaluates the same formula in float32 with the hardware log / sin / cos; tests bound the difference. */
+void dexo_normal_pair_ref(const uint32_t* wa, const uint32_t* wb, int64_t n, double* z0, double* z1) {
+    const double two_pi = 6.283185307179586476925286766559;
+    for (int64_t i = 0; i < n; ++i) {
+        const double u1 = ((double)(wa[i] >> 8) + 1.0) * 0x1p-24;
+        const double u2 = (double)(wb[i] >> 8) * 0x1p-24;
+        const double r = sqrt(-2.0 * log(u1)), theta = two_pi * (u2 - 0.5);
+        z0[i] = r * cos(theta);
+        z1[i] = r * sin(theta);
+    }
+}
+
+/* sigma·N(0,1) rows of one env: Philox block b of counter (gid, episode, step, stream | b << 8) gives rows
+ * 4b .. 4b+3 from the word pairs (x, y) and (z, w). */
+void dexo_normal_rows_ref(uint64_t seed, const uint32_t* env_gid, const uint32_t* episode, const uint32_t* step,
+                          int64_t n, uint32_t stream, int32_t rows, double sigma, double* out) {
+    for (int64_t i = 0; i < n; ++i) {
+        for (int32_t b = 0; 4 * b < rows; ++b) {
+            uint32_t w[4];
+            double z[4];
+            philox_block(seed, env_gid[i], episode[i], step[i], stream, (uint32_t)b, w);
+            dexo_normal_pair_ref(&w[0], &w[1], 1, &z[0], &z[1]);
+            dexo_normal_pair_ref(&w[2], &w[3], 1, &z[2], &z[3]);
+            for (int k = 0; k < 4 && 4 * b + k < rows; ++k) out[i * rows + 4 * b + k] = sigma * z[k];
         }
     }
 }

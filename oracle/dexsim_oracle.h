@@ -118,6 +118,11 @@ void dexo_reset_draws(uint64_t seed, uint32_t env_gid, uint32_t episode, const d
                       float* pos /* [3] */);
 void dexo_policy_action(uint64_t seed, uint32_t env_gid, uint32_t episode, uint32_t step,
                         int32_t policy_kind /* 1 random, 2 heuristic */, float* action /* [15] */);
+/* Box-Muller on Philox words in double precision (the spec the device's float32 draws approximate) */
+void dexo_normal_pair_ref(const uint32_t* wa, const uint32_t* wb, int64_t n, double* z0 /* [n] */, double* z1 /* [n] */);
+void dexo_normal_rows_ref(uint64_t seed, const uint32_t* env_gid, const uint32_t* episode, const uint32_t* step,
+                          int64_t n /* envs */, uint32_t stream /* 2..5 */, int32_t rows, double sigma,
+                          double* out /* [n, rows] */);
 
 /* ---- fused rollout restatement (auto-reset, in-"kernel" policy, counters) -------------- */
 typedef struct {

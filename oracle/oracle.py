@@ -232,6 +232,27 @@ def philox(ctr, key):
     return out
 
 
+def normal_pair_ref(wa, wb):
+    """Float64 Box-Muller (z0, z1) of Philox words wa, wb (arrays of uint32) -- DESIGN.md "RNG"."""
+    wa, wb = np.broadcast_arrays(np.asarray(wa, np.uint32), np.asarray(wb, np.uint32))
+    shape = wa.shape
+    wa, wb = np.ascontiguousarray(wa).ravel(), np.ascontiguousarray(wb).ravel()
+    z0, z1 = np.empty(wa.size), np.empty(wa.size)
+    lib().dexo_normal_pair_ref(_p(wa), _p(wb), C.c_int64(wa.size), _p(z0), _p(z1))
+    return z0.reshape(shape), z1.reshape(shape)
+
+
+def normal_rows_ref(seed, env_gid, episode, step, stream, rows, sigma):
+    """Float64 sigma * N(0,1) [n, rows] that dexsim_fill_normal draws for envs with these (gid, episode, step) words
+    (arrays, broadcast; each taken modulo 2^32 like the device's counter words)."""
+    gid, ep, st = (np.ascontiguousarray(np.asarray(a, np.int64) & 0xFFFFFFFF, np.uint32)
+                   for a in np.broadcast_arrays(env_gid, episode, step))
+    out = np.empty((gid.size, rows))
+    lib().dexo_normal_rows_ref(C.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), _p(gid), _p(ep), _p(st), C.c_int64(gid.size),
+                               C.c_uint32(stream), C.c_int32(rows), C.c_double(sigma), _p(out))
+    return out
+
+
 def np_var_counts(counts):
     counts = np.ascontiguousarray(counts, np.uint8)
     return lib().dexo_np_var_counts(_p(counts), C.c_int64(counts.size))
