@@ -14,18 +14,14 @@
 #include <cstring>
 #include <atomic>
 #include <mutex>
+#include <type_traits>
 
 #include "dexsim_core.cuh"
 
 namespace dexsim {
 
-#ifndef DEXSIM_STEP_MIN_BLOCKS
-#define DEXSIM_STEP_MIN_BLOCKS 2
-#endif
+constexpr int STEP_MIN_BLOCKS = 2;
 constexpr int STEP_THREADS = 256;
-#ifndef DEXSIM_PDL_DEFAULT
-#define DEXSIM_PDL_DEFAULT(n) 1      // measured on B200 (tools/time_small.py): 14.3 -> 12.1 us at 131,072 envs, 70.0 -> 67.7 us at 1 Mi
-#endif
 
 constexpr int SMEM_GROUPS_MAX = 64;     // group table + block counters are staged in smem up to this many groups
 
@@ -263,7 +259,7 @@ __global__ void pack_env_kernel(const DexsimState st, const DexsimStepIO io, con
 // EXTRAS: noise, reward components, episode tracking, auto-reset -- the plain path carries none
 // of their registers or branches.
 template <bool DENSE, bool AOS, bool EXTRAS>
-__global__ void __launch_bounds__(STEP_THREADS, DEXSIM_STEP_MIN_BLOCKS)
+__global__ void __launch_bounds__(STEP_THREADS, STEP_MIN_BLOCKS)
 step_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
             const uint16_t* __restrict__ group_of_env, const DexsimStepIO io,
             double* __restrict__ pack_out = nullptr, const double pack_tag = 0.0) {
@@ -501,14 +497,10 @@ reset_philox_kernel(const DexsimState st, const DexsimParams p, const DexsimGrou
 }
 
 // ---- fused rollout ------------------------------------------------------------------------------------
-#ifndef DEXSIM_ROLLOUT_MIN_BLOCKS
-#define DEXSIM_ROLLOUT_MIN_BLOCKS 2
-#endif
-#ifndef DEXSIM_ROLLOUT_THREADS
-#define DEXSIM_ROLLOUT_THREADS 256      // CTA shape of the fused rollout for large batches (x MIN_BLOCKS resident CTAs per SM)
-#endif
+constexpr int ROLLOUT_MIN_BLOCKS = 2;
+constexpr int ROLLOUT_THREADS = 256;      // CTA shape of the fused rollout for large batches (x MIN_BLOCKS resident CTAs per SM)
 template <bool DENSE, bool LEARNER>
-__global__ void __launch_bounds__(DEXSIM_ROLLOUT_THREADS, DEXSIM_ROLLOUT_MIN_BLOCKS)
+__global__ void __launch_bounds__(ROLLOUT_THREADS, ROLLOUT_MIN_BLOCKS)
 rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
                const uint16_t* __restrict__ group_of_env, const int k_steps, const int policy_kind,
                const DexsimRolloutIO rio) {
@@ -741,7 +733,7 @@ static int query_device(DeviceInfo& d) {
     if (err != cudaSuccess) return -(int)err;
     err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&d.step_ctas, step_kernel<true, false, false>, STEP_THREADS, 0);
     if (err != cudaSuccess) return -(int)err;
-    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&d.rollout_ctas, rollout_kernel<true, false>, DEXSIM_ROLLOUT_THREADS, 0);
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&d.rollout_ctas, rollout_kernel<true, false>, ROLLOUT_THREADS, 0);
     if (err != cudaSuccess) return -(int)err;
     d.valid = true;
     return 0;
@@ -808,30 +800,6 @@ static void launch_step_variant(bool extras, int grid, cudaStream_t s, const Dex
     else        step_kernel<DENSE, AOS, false><<<grid, STEP_THREADS, 0, s>>>(st, p, groups, goe, io);
 }
 
-// Programmatic dependent launch of the pipelined step kernel: DEXSIM_PDL=0 never, =1 always, unset = default policy.
-static int pdl_choice(int64_t n) {
-    static int forced = -2;
-    if (forced == -2) {
-        const char* e = getenv("DEXSIM_PDL");
-        forced = e ? atoi(e) : -1;
-    }
-    if (forced >= 0) return forced ? 1 : 0;
-    return DEXSIM_PDL_DEFAULT(n);
-}
-
-// The programmatic edge is kept inside captured graphs as well (DEXSIM_PDL_GRAPH=0 drops it, for experiments): measured on
-// B200 with capture_step(steps=8), us per step with / without: 65,536 envs 9.4 / 10.6, 131,072 12.6 / 13.6, 1 Mi 69.2 / 70.0.
-// Eager stepping with PDL (9.3 / 12.1 / 67.1) is as fast as a graph replay once the GPU, not the host, is the bound
-// (>= 65,536 envs); at 4,096 envs the replay wins (6.5 vs 7.5, the eager loop runs at the host's issue rate).
-static bool pdl_in_graphs() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("DEXSIM_PDL_GRAPH");
-        v = (e && !atoi(e)) ? 0 : 1;
-    }
-    return v == 1;
-}
-
 template <bool DENSE, bool AOS, int TRACK, bool EXTRA, int STAGES, int TILE_>
 static int launch_tma_variant(int sm_count, cudaStream_t s, const DexsimState& st, const DexsimParams& p,
                               const DexsimGroup* groups, const uint16_t* goe, const DexsimStepIO& io,
@@ -856,70 +824,61 @@ static int launch_tma_variant(int sm_count, cudaStream_t s, const DexsimState& s
     }
     int grid = sm_count * ctas_per_sm;
     if (grid > num_tiles) grid = num_tiles;
-    // Programmatic dependent launch for back-to-back steps of batches whose step is launch-latency bound: this grid may
-    // start (barrier init, counter staging) while the previous step's grid drains and blocks in griddepcontrol.wait
-    // until that grid has completed -- stream order is preserved for every access.  All CTAs of a launch are resident
-    // at once (grid <= SMs x CTAs per SM), so a waiting grid can never keep its predecessor's CTAs off the SMs.
-    int pdl = pdl_choice(st.n);
-    if (pdl && !pdl_in_graphs()) {
-        // inside a stream capture the kernel nodes of consecutive steps already launch back to back
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        if (cudaStreamIsCapturing(s, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone) pdl = 0;
-    }
-    if (pdl) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(TMA_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = s;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        return cuda_rc(cudaLaunchKernelEx(&cfg, kern, st, p, groups, goe, io, maps, num_tiles, pdl));
-    }
-    kern<<<grid, TMA_THREADS, smem, s>>>(st, p, groups, goe, io, maps, num_tiles, 0);
-    return cuda_rc(cudaGetLastError());
+    // Programmatic dependent launch, eagerly and inside captured graphs: this grid may start (barrier init, counter
+    // staging) while the previous step's grid drains and blocks in griddepcontrol.wait until that grid has completed --
+    // stream order is preserved for every access.  All CTAs of a launch are resident at once (grid <= SMs x CTAs per SM),
+    // so a waiting grid can never keep its predecessor's CTAs off the SMs.  Measured on B200, us per step with / without:
+    // eager (tools/time_small.py) 131,072 envs 12.1 / 14.3, 1 Mi 67.7 / 70.0; replayed from capture_step(steps=8)
+    // (tools/time_graph.py) 65,536 envs 9.4 / 10.6, 131,072 12.6 / 13.6, 1 Mi 69.2 / 70.0.  Eager stepping with PDL
+    // (9.3 / 12.1 / 67.1) is as fast as a graph replay once the GPU, not the host, is the bound (>= 65,536 envs); at
+    // 4,096 envs the replay wins (6.5 vs 7.5, the eager loop runs at the host's issue rate).
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(TMA_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = s;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr; cfg.numAttrs = 1;
+    return cuda_rc(cudaLaunchKernelEx(&cfg, kern, st, p, groups, goe, io, maps, num_tiles, /*pdl=*/1));
 }
 
-// 0 = auto (TMA pipeline when eligible), 1 = register-resident kernel only, 2 = TMA pipeline required.
-// Initialised from DEXSIM_STEP_IMPL (v1 | v2), changeable at run time with dexsim_set_step_impl().
+// Step kernel (dexsim_set_step_impl): 0 = auto (TMA pipeline when eligible), 1 = register-resident kernel only,
+// 2 = TMA pipeline required.
 static int g_rollout_impl = 0;
-static int g_step_impl = -1;
-static int step_impl_choice() {
-    if (g_step_impl < 0) {
-        const char* e = getenv("DEXSIM_STEP_IMPL");
-        g_step_impl = (e && !strcmp(e, "v1")) ? 1 : (e && !strcmp(e, "v2")) ? 2 : 0;
-    }
-    return g_step_impl;
+static int g_step_impl = 0;
+
+// Tile width of the pipelined kernel (dexsim_set_step_tile): 0 = auto, 1 = narrow (128 envs, three CTAs of four compute
+// warps per SM) only, 2 = wide (224 envs, two CTAs of seven compute warps per SM) wherever it exists.  Identical results
+// either way.
+static int g_step_tile = 0;
+
+static bool aligned16(const void* ptr) { return !(reinterpret_cast<uintptr_t>(ptr) & 15u); }
+
+// What a step call asks of the kernel beyond the plain step.  track: 0 = plain step, 1 = full episode tracking (returns
+// + history summaries -> labels), 2 = counts only.  extra: noise, reward components or the float64 reward.
+static int step_track(const DexsimState& st, const DexsimParams& p, const DexsimStepIO& io) {
+    if (!p.auto_reset && st.ep_return == nullptr && io.finished == nullptr) return 0;
+    return st.ep_return != nullptr ? 1 : 2;
+}
+static bool step_extra_io(const DexsimStepIO& io) {
+    return io.dyn_noise || io.obs_noise || io.reward_comps || io.reward64 || io.sigma_dyn != 0.0f || io.sigma_obs != 0.0f;
 }
 
-// Smallest batch the auto choice sends down the TMA pipeline (DEXSIM_TMA_MIN_ENVS overrides it for experiments).
-// Measured on B200 (tools/time_small.py, us per step, register-resident kernel vs pipeline, hard curriculum, 400 steps):
-//   without programmatic dependent launch the register-resident kernel won below ~80k envs (65,536 envs, counts:
-//   10.2 vs 11.4) -- with it (the default, see pdl_choice) the pipeline's prologue overlaps the previous step's tail:
+// Whether the pipelined kernel takes a step call (`single`: dexsim_step_single, which packs its env in the same launch).
+// It needs 16-byte aligned bases for everything its bulk copies touch; noise / reward-component / float64-reward calls
+// ride it too (their rows are accessed directly) when the actions are [n,15].  Every batch of at least one tile takes
+// it: measured on B200 (tools/time_small.py, us per step, register-resident kernel vs pipeline, hard curriculum,
+// 400 steps), without programmatic dependent launch the register-resident kernel won below ~80k envs (65,536 envs,
+// counts: 10.2 vs 11.4) -- with it the pipeline's prologue overlaps the previous step's tail:
 //   counts:  4,096 envs 7.6 vs 6.3;  16,384 8.4 vs 7.0;  65,536 10.2 vs 9.3;  131,072 15.1 vs 12.0;  196,608 20.2 vs 14.4
 //   tracked: 4,096 8.7 vs 7.1;  65,536 11.1 vs 10.7;  131,072 16.8 vs 14.2;  196,608 22.5 vs 17.2
 //   plain:   16,384 6.2 vs 4.9;  65,536 6.2 vs 7.0 (both at the ~5 us host issue rate);  131,072 10.3 vs 9.0
-// so every batch of at least one tile takes the pipeline.
-static int64_t tma_min_envs(int track, bool extra) {
-    (void)track; (void)extra;
-    static int64_t forced = -2;
-    if (forced == -2) {
-        const char* e = getenv("DEXSIM_TMA_MIN_ENVS");
-        forced = e ? atoll(e) : -1;
-    }
-    const int64_t v = forced >= 0 ? forced : TILE;
-    return v < TILE ? TILE : v;
-}
-
-// Tile width of the pipelined kernel: 0 = auto, 1 = narrow (128 envs, three CTAs of four compute warps per SM) only,
-// 2 = wide (224 envs, two CTAs of seven compute warps per SM) wherever it exists.  Initialised from DEXSIM_STEP_TILE
-// (narrow | wide), changeable at run time with dexsim_set_step_tile().  Identical results either way.
-static int g_step_tile = -1;
-static int step_tile_choice() {
-    if (g_step_tile < 0) {
-        const char* e = getenv("DEXSIM_STEP_TILE");
-        g_step_tile = (e && !strcmp(e, "narrow")) ? 1 : (e && !strcmp(e, "wide")) ? 2 : 0;
-    }
-    return g_step_tile;
+static bool pipeline_eligible(const DexsimState& st, const DexsimStepIO& io, int track, bool extra_io, bool single) {
+    return (!extra_io || io.action_layout == 1) && !single && st.n >= TILE && st.n < (int64_t)0x7FFFFF00 &&
+           aligned16(io.action) && aligned16(io.reward) && aligned16(st.thr) && aligned16(st.damp) &&
+           aligned16(st.step_count) && aligned16(st.cmask) && aligned16(io.terminated) && aligned16(io.truncated) &&
+           aligned16(io.num_contacts) && aligned16(st.episode) && aligned16(io.finished) &&
+           (track != 1 || (aligned16(st.ep_return) && aligned16(st.ep_stats))) &&
+           g_step_impl != 1 && get_encode_fn() != nullptr;
 }
 
 // A step of a batch whose state sits in L2 (below ~256 Ki envs) is bound by how many env-warps an SM can run side by side
@@ -931,8 +890,7 @@ static int step_tile_choice() {
 // HBM-bound batches gain nothing, so they stay on the narrow tile (more CTAs for the dynamic tile hand-out to balance).
 static bool use_wide_tile(int64_t n, int track, int sm_count) {
     if (track == 1 || n < TILE_WIDE || TILE != 128) return false;       // full tracking: its stages only fit the narrow tile
-    const int choice = step_tile_choice();
-    if (choice) return choice == 2;
+    if (g_step_tile) return g_step_tile == 2;
     if (n >= (int64_t)1 << 18) return false;
     // tiles per resident CTA, rounded up -- a handful of CTAs with one tile more (5 % of a round) do not count as a round:
     // the dynamic hand-out spreads them over the SMs
@@ -942,7 +900,6 @@ static bool use_wide_tile(int64_t n, int track, int sm_count) {
     return depth_wide < depth_narrow;
 }
 
-// track: 0 = plain step, 1 = full episode tracking (returns + history summaries -> labels), 2 = counts only
 static int launch_step_tma(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups, const uint16_t* goe,
                            const DexsimStepIO* io, cudaStream_t s, int track, bool extra, int sm_count) {
     // Tensor maps are pure functions of (base pointers, n, ld): a stepping loop re-encodes nothing.  One cached set
@@ -974,30 +931,36 @@ static int launch_step_tma(const DexsimState* st, const DexsimParams* p, const D
     }
     const StepMaps& maps = cache.maps;
     const int num_tiles = (int)((st->n + tile - 1) / tile);
-    const bool dense = p->reward_type == 1;
-#define DEXSIM_TMA_CASE(D, A, T, X)                                                                                 \
-    if (dense == D && aos == A && track == T && extra == X)                                                         \
-        return launch_tma_variant<D, A, T, X, DEXSIM_TMA_STAGES, TILE>(sm_count, s, *st, *p, groups, goe, *io, maps, num_tiles);
-#define DEXSIM_TMA_WIDE_CASE(D, A, T, X)                                                                            \
-    if (wide && dense == D && aos == A && track == T && extra == X)                                                 \
-        return launch_tma_variant<D, A, T, X, 2, TILE_WIDE>(sm_count, s, *st, *p, groups, goe, *io, maps, num_tiles);
-    // wide tile: plain and counts-only steps
-    DEXSIM_TMA_WIDE_CASE(true, true, 0, false) DEXSIM_TMA_WIDE_CASE(true, true, 2, false)
-    DEXSIM_TMA_WIDE_CASE(true, false, 0, false) DEXSIM_TMA_WIDE_CASE(true, false, 2, false)
-    DEXSIM_TMA_WIDE_CASE(false, true, 0, false) DEXSIM_TMA_WIDE_CASE(false, true, 2, false)
-    DEXSIM_TMA_WIDE_CASE(false, false, 0, false) DEXSIM_TMA_WIDE_CASE(false, false, 2, false)
-    DEXSIM_TMA_WIDE_CASE(true, true, 0, true) DEXSIM_TMA_WIDE_CASE(true, true, 2, true)
-    DEXSIM_TMA_WIDE_CASE(false, true, 0, true) DEXSIM_TMA_WIDE_CASE(false, true, 2, true)
-    DEXSIM_TMA_CASE(true, true, 0, false) DEXSIM_TMA_CASE(true, true, 1, false) DEXSIM_TMA_CASE(true, true, 2, false)
-    DEXSIM_TMA_CASE(true, false, 0, false) DEXSIM_TMA_CASE(true, false, 1, false) DEXSIM_TMA_CASE(true, false, 2, false)
-    DEXSIM_TMA_CASE(false, true, 0, false) DEXSIM_TMA_CASE(false, true, 1, false) DEXSIM_TMA_CASE(false, true, 2, false)
-    DEXSIM_TMA_CASE(false, false, 0, false) DEXSIM_TMA_CASE(false, false, 1, false) DEXSIM_TMA_CASE(false, false, 2, false)
-    // noise / reward components: the reference's [n,15] action layout only (SoA callers take the register kernel)
-    DEXSIM_TMA_CASE(true, true, 0, true) DEXSIM_TMA_CASE(true, true, 1, true) DEXSIM_TMA_CASE(true, true, 2, true)
-    DEXSIM_TMA_CASE(false, true, 0, true) DEXSIM_TMA_CASE(false, true, 1, true) DEXSIM_TMA_CASE(false, true, 2, true)
-#undef DEXSIM_TMA_WIDE_CASE
-#undef DEXSIM_TMA_CASE
-    return 1;
+    // runtime (dense, aos, track, extra) -> template arguments: each call hands its value on as a std::integral_constant
+    const auto as_bool = [](bool b, auto&& f) { return b ? f(std::true_type{}) : f(std::false_type{}); };
+    const auto as_track = [](int t, auto&& f) {
+        using std::integral_constant;
+        return t == 1 ? f(integral_constant<int, 1>{}) : t == 2 ? f(integral_constant<int, 2>{}) : f(integral_constant<int, 0>{});
+    };
+    return as_bool(p->reward_type == 1, [&](auto dense) {
+        return as_bool(aos, [&](auto aos_) {
+            return as_track(track, [&](auto track_) {
+                return as_bool(extra, [&](auto extra_) -> int {
+                    constexpr bool DENSE = decltype(dense)::value, AOS = decltype(aos_)::value, EXTRA = decltype(extra_)::value;
+                    constexpr int TRACK = decltype(track_)::value;
+                    // The instantiations: noise / reward components only with the reference's [n,15] action layout (SoA
+                    // callers take the register kernel), and the wide tile only without full tracking (its stages have no
+                    // room for the per-env return / history arrays).
+                    if constexpr (EXTRA && !AOS) {
+                        return 1;
+                    } else {
+                        if constexpr (TRACK != 1) {
+                            if (wide)
+                                return launch_tma_variant<DENSE, AOS, TRACK, EXTRA, 2, TILE_WIDE>(sm_count, s, *st, *p, groups,
+                                                                                                  goe, *io, maps, num_tiles);
+                        }
+                        return launch_tma_variant<DENSE, AOS, TRACK, EXTRA, DEXSIM_TMA_STAGES, TILE>(sm_count, s, *st, *p, groups,
+                                                                                                     goe, *io, maps, num_tiles);
+                    }
+                });
+            });
+        });
+    });
 }
 
 static int launch_step(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
@@ -1020,26 +983,13 @@ static int launch_step(const DexsimState* st, const DexsimParams* p, const Dexsi
     DeviceInfo di;
     rc = device_info_cached(di);
     if (rc) return rc;
-    // TMA pipeline: needs 16-byte aligned bases for everything its bulk copies touch; noise / reward-component /
-    // float64-reward calls ride it too (their rows are accessed directly) when the actions are [n,15]
-    const int impl = step_impl_choice();
-    const bool extra_io = io->dyn_noise || io->obs_noise || io->reward_comps || io->reward64 || fused_dyn || fused_obs;
-    const bool tracked = (p && p->auto_reset) || st->ep_return != nullptr || io->finished != nullptr;
-    const int track = !tracked ? 0 : (st->ep_return != nullptr ? 1 : 2);
-    const bool tma_ok = (!extra_io || io->action_layout == 1) && pack_out == nullptr &&
-                        st->n >= TILE && st->n < (int64_t)0x7FFFFF00 &&
-                        !(reinterpret_cast<uintptr_t>(io->action) & 15u) && !(reinterpret_cast<uintptr_t>(io->reward) & 15u) &&
-                        !(reinterpret_cast<uintptr_t>(st->thr) & 15u) && !(reinterpret_cast<uintptr_t>(st->damp) & 15u) &&
-                        !(reinterpret_cast<uintptr_t>(st->step_count) & 15u) && !(reinterpret_cast<uintptr_t>(st->cmask) & 15u) &&
-                        !(reinterpret_cast<uintptr_t>(io->terminated) & 15u) && !(reinterpret_cast<uintptr_t>(io->truncated) & 15u) &&
-                        !(reinterpret_cast<uintptr_t>(io->num_contacts) & 15u) && !(reinterpret_cast<uintptr_t>(st->episode) & 15u) &&
-                        (track != 1 || (!(reinterpret_cast<uintptr_t>(st->ep_return) & 15u) && !(reinterpret_cast<uintptr_t>(st->ep_stats) & 15u))) &&
-                        !(reinterpret_cast<uintptr_t>(io->finished) & 15u);
-    if (impl != 1 && tma_ok && (impl == 2 || st->n >= tma_min_envs(track, extra_io))) {
+    const int track = step_track(*st, *p, *io);
+    const bool extra_io = step_extra_io(*io);
+    if (pipeline_eligible(*st, *io, track, extra_io, pack_out != nullptr)) {
         rc = launch_step_tma(st, p, groups, goe, io, s, track, extra_io, di.sm_count);
-        if (rc <= 0) return rc;                      // launched (0) or CUDA error (< 0); 1 = not available
+        if (rc <= 0) return rc;                      // launched (0) or CUDA error (< 0); 1 = a tensor map was rejected
     }
-    if (impl == 2) return DEXSIM_E_PARAM;            // TMA pipeline was demanded but is not eligible
+    if (g_step_impl == 2) return DEXSIM_E_PARAM;     // TMA pipeline was demanded but is not eligible
     if (io->flags & DEXSIM_STEP_HOST_ALL_ROWS) return DEXSIM_E_PARAM;   // only the pipelined kernel mirrors every row
     const int grid = grid_for(st->n, STEP_THREADS, di.step_ctas, di.sm_count);
     const bool dense = p->reward_type == 1, aos = io->action_layout == 1;
@@ -1181,7 +1131,7 @@ int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGro
     // Small batches are latency-bound: spread warps over as many SM sub-partitions as possible
     // (4 per SM) by shrinking the CTA; large batches use full 256-thread CTAs.
     const int64_t warps = (st->n + 31) / 32;
-    int threads = DEXSIM_ROLLOUT_THREADS;
+    int threads = ROLLOUT_THREADS;
     while (threads > 32 && warps * 32 / threads < (int64_t)di.sm_count * 4) threads = (threads / 2 + 31) / 32 * 32;
     const int64_t blocks = (st->n + threads - 1) / threads;
     if (blocks > 0x7FFFFFFFll) return DEXSIM_E_SIZE;
@@ -1284,12 +1234,9 @@ struct HostPipe {
     cudaStream_t streams[HOST_STREAMS];
     cudaStream_t small;                // per-env vectors (reward, flags) of the WHOLE batch: a few large copies instead of
                                        // one small copy per vector per chunk
-    cudaStream_t upload;               // every chunk's action upload, back to back: the uploads run ahead of the downloads
-                                       // instead of queueing behind an earlier chunk's download in the same stream
     cudaEvent_t fork_ev;
-    cudaEvent_t join_ev[HOST_STREAMS + 2];
+    cudaEvent_t join_ev[HOST_STREAMS + 1];
     cudaEvent_t kdone[HOST_MAX_CHUNKS];
-    cudaEvent_t up_ev[HOST_MAX_CHUNKS];
 };
 HostPipe g_pipes[64];
 std::mutex g_pipes_mutex;      // first use from several host threads at once
@@ -1309,16 +1256,12 @@ int get_pipe(HostPipe** out) {
         }
         err = cudaStreamCreateWithFlags(&hp.small, cudaStreamNonBlocking);
         if (err != cudaSuccess) return -(int)err;
-        err = cudaStreamCreateWithFlags(&hp.upload, cudaStreamNonBlocking);
-        if (err != cudaSuccess) return -(int)err;
-        for (int k = 0; k < HOST_STREAMS + 2; ++k) {
+        for (int k = 0; k < HOST_STREAMS + 1; ++k) {
             err = cudaEventCreateWithFlags(&hp.join_ev[k], cudaEventDisableTiming);
             if (err != cudaSuccess) return -(int)err;
         }
         for (int k = 0; k < HOST_MAX_CHUNKS; ++k) {
             err = cudaEventCreateWithFlags(&hp.kdone[k], cudaEventDisableTiming);
-            if (err != cudaSuccess) return -(int)err;
-            err = cudaEventCreateWithFlags(&hp.up_ev[k], cudaEventDisableTiming);
             if (err != cudaSuccess) return -(int)err;
         }
         err = cudaEventCreateWithFlags(&hp.fork_ev, cudaEventDisableTiming);
@@ -1329,17 +1272,6 @@ int get_pipe(HostPipe** out) {
     return 0;
 }
 }  // namespace
-
-// DEXSIM_HOST_UPLOAD_STREAM=1: all action uploads of a host step on one dedicated stream, running ahead of the downloads
-// (experiment; default 0 = each chunk uploads on its own stream, behind the previous download of that stream).
-static bool upload_stream_choice() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("DEXSIM_HOST_UPLOAD_STREAM");
-        v = (e && atoi(e)) ? 1 : 0;
-    }
-    return v == 1;
-}
 
 // DEXSIM_HOST_TRACE=1: device-side timeline of every tenth chunked dexsim_step_host call on stderr (experiments): when each
 // chunk's upload, kernel and row download finished, relative to the call's fork point (profiles/r02_host_step_timeline.txt).
@@ -1366,17 +1298,6 @@ struct HostTrace {               // one set of timing events, owned by the first
 };
 static HostTrace g_trace;
 static std::atomic<int> g_trace_calls{0};
-
-// zero-copy transport: 1 = the step kernel reads the actions from mapped host memory itself (no copy at all),
-// 0 = the copy engine uploads them chunk by chunk
-static bool zc_kernel_upload() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("DEXSIM_ZC_KERNEL_UPLOAD");
-        v = (e && atoi(e)) ? 1 : 0;
-    }
-    return v == 1;
-}
 
 int dexsim_expand_contact_rows(float* h_obs, const uint8_t* h_contact_mask, int64_t n, int64_t ld) {
     if (!h_obs || !h_contact_mask) return DEXSIM_E_NULL;
@@ -1406,13 +1327,14 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
     // mask as three more bulk rows, x / y and their velocities when a reset changes them (h_obs must be current, as for
     // DEXSIM_HOST_STATIC_ROWS) -- so nothing is downloaded by the copy engine: no per-copy hand-over times, no pipeline
     // fill, and the download of a tile starts the moment it is computed.  The contact rows follow from the mask
-    // (PACKED_CONTACTS semantics; EXPAND_CONTACTS as below).  The actions either come up chunk by chunk on the copy engine (default:
-    // uploads of chunk k+1 overlap the PCIe writes of chunk k's kernel) or are read from host memory by the kernel's own
-    // bulk loads (DEXSIM_ZC_KERNEL_UPLOAD=1: no copies at all).  Not eligible (a buffer that is not mapped, fewer envs
-    // than a tile, DEXSIM_STEP_IMPL=register): the copy transport below runs instead.
+    // (PACKED_CONTACTS semantics; EXPAND_CONTACTS as below).  The actions come up chunk by chunk on the copy engine: uploads
+    // of chunk k+1 overlap the PCIe writes of chunk k's kernel.  The transport is decided here, once, for the whole batch:
+    // chunk offsets are multiples of 1,024 envs, so every chunk keeps the batch's alignment, and the fold rule below keeps
+    // every chunk at one tile or more.  Not eligible (a buffer that is not mapped, fewer envs than a tile, the register
+    // kernel selected): the copy transport below runs instead.
     DexsimStepIO zio = *io;
     bool zc = false;
-    if ((flags & DEXSIM_HOST_ZERO_COPY) && (flags & DEXSIM_HOST_PACKED_CONTACTS) && h_obs && n >= TILE) {
+    if ((flags & DEXSIM_HOST_ZERO_COPY) && (flags & DEXSIM_HOST_PACKED_CONTACTS) && h_obs) {
         auto alias = [](const void* h) -> void* {
             if (!h) return nullptr;
             cudaPointerAttributes attr;
@@ -1428,12 +1350,8 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
         if (h_num_contacts) zio.num_contacts = static_cast<uint8_t*>(alias(h_num_contacts));
         zio.host_cmask = static_cast<uint8_t*>(alias(h_contact_mask));
         zio.flags |= DEXSIM_STEP_HOST_ALL_ROWS;
-        zc = zio.host_static_rows && zio.reward && zio.terminated && zio.truncated && zio.num_contacts && zio.host_cmask;
-        if (zc && zc_kernel_upload()) {
-            const float* a = static_cast<const float*>(alias(h_action));
-            if (a) { zio.action = a; chunks = 1; }
-            else zc = false;
-        }
+        zc = zio.host_static_rows && zio.reward && zio.terminated && zio.truncated && zio.num_contacts && zio.host_cmask &&
+             pipeline_eligible(*st, zio, step_track(*st, *p, zio), step_extra_io(zio), /*single=*/false);
     }
     // chunk boundaries are multiples of 1024 envs (tile- and alignment-friendly)
     if (chunks > HOST_MAX_CHUNKS) chunks = HOST_MAX_CHUNKS;
@@ -1466,8 +1384,6 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
             err = cudaStreamWaitEvent(hp->streams[k], hp->fork_ev, 0);
             if (err != cudaSuccess) return -(int)err;
         }
-        err = cudaStreamWaitEvent(hp->upload, hp->fork_ev, 0);
-        if (err != cudaSuccess) return -(int)err;
     }
     // observation rows that travel: all 45, or without the constant quaternion rows 33-36 (SKIP_QUAT), and without the
     // five 0/1 contact rows 40-44 when the 1-byte contact mask is sent instead (PACKED_CONTACTS)
@@ -1505,8 +1421,7 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
         }
         return 0;
     };
-    auto enqueue_chunks = [&]() -> int {
-    for (int c = 0; c < nchunks; ++c) {
+    for (int c = 0; c < nchunks && rc == 0; ++c) {
         const int64_t lo = (int64_t)c * per, hi = chunk_hi(c), m = hi - lo;
         cudaStream_t s = nchunks > 1 ? hp->streams[c % HOST_STREAMS] : user;
         DexsimState sub = *st;
@@ -1518,9 +1433,8 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
         DexsimParams sp = *p;
         sp.env_gid0 = p->env_gid0 + lo;
         DexsimStepIO sio = zc ? zio : *io;
-        const bool kernel_upload = zc && zio.action != io->action;       // the kernel reads the actions from host memory
         float* d_action = const_cast<float*>(io->action) + (aos ? lo * NJ : lo);
-        sio.action = kernel_upload ? zio.action + (aos ? lo * NJ : lo) : d_action;
+        sio.action = d_action;
         sio.reward += lo; sio.terminated += lo; sio.truncated += lo; sio.num_contacts += lo;
         if (sio.reward_comps) sio.reward_comps += lo;
         if (sio.reward64) sio.reward64 += lo;
@@ -1528,35 +1442,25 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
         if (sio.sched) sio.sched = (2 * (c + 1) + 1 < DEXSIM_SCHED_WORDS) ? io->sched + 2 * (c + 1) : nullptr;   // chunks run concurrently
         if (zc) { sio.host_static_rows = zio.host_static_rows + lo; if (sio.host_cmask) sio.host_cmask += lo; }
         else if (mirror) sio.host_static_rows = mirror + lo;
-        cudaError_t err = cudaSuccess;
-        cudaStream_t up = (nchunks > 1 && upload_stream_choice()) ? hp->upload : s;
-        if (kernel_upload) up = s;
-        else if (aos) err = cudaMemcpyAsync(d_action, h_action + lo * NJ, (size_t)m * NJ * sizeof(float), cudaMemcpyHostToDevice, up);
-        else err = cudaMemcpy2DAsync(d_action, (size_t)ld * 4, h_action + lo, (size_t)ld * 4, (size_t)m * 4, NJ, cudaMemcpyHostToDevice, up);
-        if (err != cudaSuccess) return -(int)err;
-        if (up != s) {                                   // the chunk's stream picks up where the upload stream got to
-            err = cudaEventRecord(hp->up_ev[c], up);
-            if (err == cudaSuccess) err = cudaStreamWaitEvent(s, hp->up_ev[c], 0);
-            if (err != cudaSuccess) return -(int)err;
-        }
+        cudaError_t err;
+        if (aos) err = cudaMemcpyAsync(d_action, h_action + lo * NJ, (size_t)m * NJ * sizeof(float), cudaMemcpyHostToDevice, s);
+        else err = cudaMemcpy2DAsync(d_action, (size_t)ld * 4, h_action + lo, (size_t)ld * 4, (size_t)m * 4, NJ, cudaMemcpyHostToDevice, s);
+        if (err != cudaSuccess) { rc = -(int)err; break; }
         if (tracing) cudaEventRecord(g_trace.up[c], s);
         rc = launch_step(&sub, &sp, groups, group_of_env ? group_of_env + lo : nullptr, &sio, s);
-        if (rc) return rc;
+        if (rc) break;
         if (tracing) cudaEventRecord(g_trace.k[c], s);
         if (zc) {                                        // every result is already on its way to the host buffers
-            if (nchunks > 1) {
-                err = cudaEventRecord(hp->kdone[c], s);
-                if (err != cudaSuccess) return -(int)err;
-            }
+            if (nchunks > 1) rc = cuda_rc(cudaEventRecord(hp->kdone[c], s));
             continue;
         }
         if (nchunks > 1) {
             if (expand_on_host) {                        // the chunk's contact masks first: the host expands them while its rows travel
                 err = cudaMemcpyAsync(h_contact_mask + lo, st->cmask + lo, (size_t)m, cudaMemcpyDeviceToHost, s);
-                if (err != cudaSuccess) return -(int)err;
+                if (err != cudaSuccess) { rc = -(int)err; break; }
             }
             err = cudaEventRecord(hp->kdone[c], s);      // this chunk's kernel has run: its per-env vectors are final
-            if (err != cudaSuccess) return -(int)err;
+            if (err != cudaSuccess) { rc = -(int)err; break; }
         }
         if (h_obs) {
             auto rows = [&](int r0, int r1) -> cudaError_t {       // observation rows [r0, r1) of this chunk
@@ -1582,33 +1486,18 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
                 err = cudaMemcpy2DAsync(h_obs + lo, (size_t)ld * 4, st->obs + lo, (size_t)ld * 4, (size_t)m * 4, rows_hi,
                                         cudaMemcpyDeviceToHost, s);
             }
-            if (err != cudaSuccess) return -(int)err;
+            if (err != cudaSuccess) { rc = -(int)err; break; }
             if (tracing) cudaEventRecord(g_trace.down[c], s);
         }
-        if (nchunks == 1) {
-            rc = copy_vectors(s, 0, n);
-            if (rc) return rc;
-        }
+        if (nchunks == 1) rc = copy_vectors(s, 0, n);
     }
-    if (nchunks > 1 && !zc) {
+    if (rc == 0 && nchunks > 1 && !zc) {
         // reward / flags of the whole batch in one copy per vector (5 copies instead of 5 per chunk: every copy costs
         // the DMA engine a few microseconds whatever its size), on their own stream once every chunk's kernel has run --
         // the kernels finish long before the observation downloads do, so these ride along with them
-        for (int c = 0; c < nchunks; ++c) {
-            cudaError_t err = cudaStreamWaitEvent(hp->small, hp->kdone[c], 0);
-            if (err != cudaSuccess) return -(int)err;
-        }
-        rc = copy_vectors(hp->small, 0, n);
-        if (rc) return rc;
-        if (tracing) cudaEventRecord(g_trace.small, hp->small);
-    }
-    return 0;
-    };
-    rc = enqueue_chunks();
-    if (zc && rc == DEXSIM_E_PARAM) {
-        // the pipelined kernel is not available for this call (nothing has been launched): copy transport
-        zc = false;
-        rc = enqueue_chunks();
+        for (int c = 0; c < nchunks && rc == 0; ++c) rc = cuda_rc(cudaStreamWaitEvent(hp->small, hp->kdone[c], 0));
+        if (rc == 0) rc = copy_vectors(hp->small, 0, n);
+        if (rc == 0 && tracing) cudaEventRecord(g_trace.small, hp->small);
     }
     if (zc && rc == 0) g_zero_copy_steps.fetch_add(1, std::memory_order_relaxed);
     if (nchunks > 1) {
@@ -1617,13 +1506,9 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
             if (err == cudaSuccess) err = cudaStreamWaitEvent(user, hp->join_ev[k], 0);
             if (err != cudaSuccess && rc == 0) rc = -(int)err;
         }
-        {
-            cudaError_t err = cudaEventRecord(hp->join_ev[HOST_STREAMS], hp->small);
-            if (err == cudaSuccess) err = cudaStreamWaitEvent(user, hp->join_ev[HOST_STREAMS], 0);
-            if (err == cudaSuccess) err = cudaEventRecord(hp->join_ev[HOST_STREAMS + 1], hp->upload);
-            if (err == cudaSuccess) err = cudaStreamWaitEvent(user, hp->join_ev[HOST_STREAMS + 1], 0);
-            if (err != cudaSuccess && rc == 0) rc = -(int)err;
-        }
+        cudaError_t err = cudaEventRecord(hp->join_ev[HOST_STREAMS], hp->small);
+        if (err == cudaSuccess) err = cudaStreamWaitEvent(user, hp->join_ev[HOST_STREAMS], 0);
+        if (err != cudaSuccess && rc == 0) rc = -(int)err;
         enqueue_lock.unlock();
     }
     if ((flags & DEXSIM_HOST_ASYNC) && rc == 0) return 0;          // the caller synchronizes `stream` before reading

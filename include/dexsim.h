@@ -14,8 +14,10 @@
  *     pointers (pinned for full speed) and are documented as such.
  *   - `stream` is a cudaStream_t passed as void* (0 = legacy default stream).  Calls are
  *     asynchronous on that stream unless stated; no allocation and no per-call global state
- *     (the only process-wide switches are dexsim_set_step_impl / dexsim_set_rollout_impl, for tests
- *     and profiling) => thread-safe per (device, stream).  dexsim_step_host forks onto a few internal
+ *     (the only process-wide switches are dexsim_set_step_impl / dexsim_set_step_tile /
+ *     dexsim_set_rollout_impl, for tests and profiling, and the environment variable DEXSIM_HOST_TRACE=1,
+ *     which prints a device-side timeline of every tenth chunked dexsim_step_host call to stderr)
+ *     => thread-safe per (device, stream).  dexsim_step_host forks onto a few internal
  *     streams per device, joins them into `stream` and (unless DEXSIM_HOST_ASYNC) synchronizes it before
  *     returning; concurrent callers on the SAME device are serialised while they enqueue.
  *   - Return value: 0 = ok; negative cudaError_t (-e) for CUDA failures; DEXSIM_E_* for
@@ -347,7 +349,10 @@ int dexsim_classify_summary(const DexsimEpisodeSummary* s, const uint8_t* counts
  *      obs / reward / flags back to HOST memory, synchronous on return unless DEXSIM_HOST_ASYNC.  Pinned buffers make
  *      the copies asynchronous DMA; pageable buffers work but stage through the driver.  With chunks > 1
  *      the envs are split into that many ranges whose H2D copy, kernel and D2H copies overlap on
- *      internal streams (created once per device, forked from / joined into `stream`).
+ *      internal streams (created once per device, forked from / joined into `stream`).  The transport
+ *      (DEXSIM_HOST_ZERO_COPY or the copies) is decided once per call, before anything is enqueued; if a launch
+ *      still fails (e.g. the tensor-map encoder rejects a map), the call joins its streams and returns the error
+ *      without enqueueing anything again.
  *      This is what a caller that keeps NumPy-side policies uses in place of
  *      `obs, r, term, trunc, info = env.step(action)` (envs/manipulation_env.py:184). ------------------ */
 #define DEXSIM_HOST_SKIP_QUAT 1        /* do not copy obs rows 33-36 (constant quaternion, already in h_obs) */

@@ -33,6 +33,18 @@ def test_library_exports_every_declared_symbol():
     assert L.dexsim_version() == _lib.ABI_VERSION
 
 
+def test_only_environment_switch_is_the_host_trace():
+    """include/dexsim.h promises that the dexsim_set_* functions and DEXSIM_HOST_TRACE are the only process-wide state:
+    the library reads no other environment variable."""
+    csrc = os.path.join(ROOT, "dexterous_rl_manipulation_b200", "csrc")
+    names = []
+    for f in sorted(os.listdir(csrc)):
+        src = open(os.path.join(csrc, f)).read()
+        assert not re.search(r"getenv\s*\(\s*[^\s\"]", src), f"{f}: getenv with a name that is not a string literal"
+        names += re.findall(r"getenv\s*\(\s*\"([^\"]*)\"", src)
+    assert names == ["DEXSIM_HOST_TRACE"]
+
+
 def test_struct_layouts():
     L = _lib.lib()
     assert L.dexsim_sizeof_state() == C.sizeof(_lib.DexsimState) == 14 * 8

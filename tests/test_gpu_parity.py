@@ -788,11 +788,20 @@ def test_step_host_matches_device_step(dx, n, chunks, track):
     assert torch.equal(a_env._obs, b_env._obs)
 
 
-@pytest.mark.parametrize("n,track", [(5000, True), (70_001, True), (4096, False)])
-def test_step_host_zero_copy_launch(dx, n, track):
+@pytest.mark.parametrize("n,track,chunks,impl", [
+    pytest.param(5000, True, None, "auto", id="5000-True"),
+    pytest.param(70_001, True, None, "auto", id="70001-True"),
+    pytest.param(4096, False, None, "auto", id="4096-False"),
+    # three chunks of 1,024 envs and one of 50: the last one, below a tile, is folded into its neighbour
+    pytest.param(3122, True, 4, "auto", id="fold"),
+    # the register-resident kernel selected: not eligible, every call takes the copy transport
+    pytest.param(5000, True, 3, "register", id="ineligible"),
+])
+def test_step_host_zero_copy_launch(dx, n, track, chunks, impl):
     """DEXSIM_HOST_ZERO_COPY: once the pinned buffers are current and the actions are pinned too, a synchronous step_host
-    is ONE kernel launch that reads the actions from, and writes every result into, host memory -- same results as the
-    device-tensor API, entry by entry, through resets, and the device-side state stays identical."""
+    uploads the actions with the copy engine and is then ONE kernel launch per chunk that writes every result into host
+    memory -- same results as the device-tensor API, entry by entry, through resets, and the device-side state stays
+    identical.  A call the pipelined kernel does not take runs the copy transport with the same results."""
     from dexterous_rl_manipulation_b200 import _lib
     L = _lib.lib()
     CC = dx.CurriculumConfig
@@ -805,37 +814,41 @@ def test_step_host_zero_copy_launch(dx, n, track):
     b_env.host_zero_copy = True                      # (default "auto": on up to 160K envs)
     rng = np.random.default_rng(4)
     pins = [torch.empty(n, 15).pin_memory() for _ in range(2)]
-    before = int(L.dexsim_host_zero_copy_steps())
-    for t in range(50):
-        act = rng.uniform(-1.2, 1.2, (n, 15)).astype(np.float32)
-        if t == 23:                                   # a device-side step behind the host buffer: next call re-primes
-            a_env.step(torch.from_numpy(act).cuda()); b_env.step(torch.from_numpy(act).cuda())
+    _lib.set_step_impl(impl)
+    try:
+        before = int(L.dexsim_host_zero_copy_steps())
+        for t in range(50):
             act = rng.uniform(-1.2, 1.2, (n, 15)).astype(np.float32)
-        if t == 31:
-            a_env.reset(seed=6); b_env.reset(seed=6)
-        pins[t % 2].copy_(torch.from_numpy(act))
-        o1, r1, te1, tr1, i1 = a_env.step(torch.from_numpy(act).cuda())
-        o2, r2, te2, tr2, i2 = b_env.step_host(pins[t % 2])
-        assert torch.equal(o1.cpu(), o2), (t, (o1.cpu() != o2).nonzero()[:5])
-        assert torch.equal(r1.cpu(), r2) and torch.equal(te1.cpu(), te2) and torch.equal(tr1.cpu(), tr2), t
-        assert torch.equal(i1["num_contacts"].cpu(), i2["num_contacts"]), t
-        assert torch.equal(i2["contact_mask"], a_env._cmask[:n].cpu()), t
-    # 50 calls, three of them priming downloads (first call, after the device-side step, after the reset)
-    assert int(L.dexsim_host_zero_copy_steps()) - before == 47
-    assert torch.equal(a_env._obs, b_env._obs) and torch.equal(a_env._op64, b_env._op64)
-    assert torch.equal(a_env._episode, b_env._episode) and torch.equal(a_env._cmask, b_env._cmask)
-    if track:
-        assert torch.equal(a_env.counters, b_env.counters) and int(a_env.counters[:, 0].sum()) > 0
-    # switched off: the copy transport, same results
-    b_env.host_zero_copy = False
-    before = int(L.dexsim_host_zero_copy_steps())
-    for t in range(5):
-        act = rng.uniform(-1.2, 1.2, (n, 15)).astype(np.float32)
-        pins[t % 2].copy_(torch.from_numpy(act))
-        o1, r1, te1, tr1, i1 = a_env.step(torch.from_numpy(act).cuda())
-        o2, r2, te2, tr2, i2 = b_env.step_host(pins[t % 2])
-        assert torch.equal(o1.cpu(), o2) and torch.equal(r1.cpu(), r2), t
-    assert int(L.dexsim_host_zero_copy_steps()) == before
+            if t == 23:                                   # a device-side step behind the host buffer: next call re-primes
+                a_env.step(torch.from_numpy(act).cuda()); b_env.step(torch.from_numpy(act).cuda())
+                act = rng.uniform(-1.2, 1.2, (n, 15)).astype(np.float32)
+            if t == 31:
+                a_env.reset(seed=6); b_env.reset(seed=6)
+            pins[t % 2].copy_(torch.from_numpy(act))
+            o1, r1, te1, tr1, i1 = a_env.step(torch.from_numpy(act).cuda())
+            o2, r2, te2, tr2, i2 = b_env.step_host(pins[t % 2], chunks=chunks)
+            assert torch.equal(o1.cpu(), o2), (t, (o1.cpu() != o2).nonzero()[:5])
+            assert torch.equal(r1.cpu(), r2) and torch.equal(te1.cpu(), te2) and torch.equal(tr1.cpu(), tr2), t
+            assert torch.equal(i1["num_contacts"].cpu(), i2["num_contacts"]), t
+            assert torch.equal(i2["contact_mask"], a_env._cmask[:n].cpu()), t
+        # 50 calls, three of them priming downloads (first call, after the device-side step, after the reset)
+        assert int(L.dexsim_host_zero_copy_steps()) - before == (0 if impl == "register" else 47)
+        assert torch.equal(a_env._obs, b_env._obs) and torch.equal(a_env._op64, b_env._op64)
+        assert torch.equal(a_env._episode, b_env._episode) and torch.equal(a_env._cmask, b_env._cmask)
+        if track:
+            assert torch.equal(a_env.counters, b_env.counters) and int(a_env.counters[:, 0].sum()) > 0
+        # switched off: the copy transport, same results
+        b_env.host_zero_copy = False
+        before = int(L.dexsim_host_zero_copy_steps())
+        for t in range(5):
+            act = rng.uniform(-1.2, 1.2, (n, 15)).astype(np.float32)
+            pins[t % 2].copy_(torch.from_numpy(act))
+            o1, r1, te1, tr1, i1 = a_env.step(torch.from_numpy(act).cuda())
+            o2, r2, te2, tr2, i2 = b_env.step_host(pins[t % 2], chunks=chunks)
+            assert torch.equal(o1.cpu(), o2) and torch.equal(r1.cpu(), r2), t
+        assert int(L.dexsim_host_zero_copy_steps()) == before
+    finally:
+        _lib.set_step_impl("auto")
 
 
 class _PatternPolicy:

@@ -1,9 +1,10 @@
 """Short, deterministic launch sequence for ncu (never a source of bench numbers).
 
-    python tools/profile_step.py [num_envs] [variant]
+    python tools/profile_step.py [num_envs] [variant] [auto|narrow|wide]
 
 variant: api (step kernel, plain), api_counts (auto-reset + counters, the bench path), api_track (auto-reset +
 full episode tracking), api_noisy (sigma_obs 0.05 + sigma_dyn 0.1 drawn in-kernel), fused (rollout kernel).
+The last argument sets the tile width of the pipelined step kernel (default auto).
 8 warm-up launches, then 6 profiled-range launches.
 """
 import os
@@ -14,9 +15,11 @@ import torch
 sys.path.insert(0, os.path.abspath(os.path.join(os.path.dirname(__file__), "..")))
 
 import dexterous_rl_manipulation_b200 as dx
+from dexterous_rl_manipulation_b200 import _lib
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 1 << 20
 variant = sys.argv[2] if len(sys.argv) > 2 else "api_track"
+_lib.set_step_tile(sys.argv[3] if len(sys.argv) > 3 else "auto")
 CC = dx.CurriculumConfig
 kw = dict(max_episode_steps=200, reward_type="dense", curriculum_config=CC.hard(), seed=42)
 if variant == "api":

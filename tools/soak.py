@@ -1,5 +1,8 @@
 """Long-run consistency soak (not a benchmark): the TMA pipeline kernel vs the register kernel over many
-thousands of back-to-back launches with auto-reset, counters and ragged tiles; then the chunked host path."""
+thousands of back-to-back launches with auto-reset, counters and ragged tiles; then the chunked host path.
+
+    python tools/soak.py [num_envs] [steps] [full|counts] [auto|narrow|wide]
+"""
 import os
 import sys
 import time
@@ -13,6 +16,7 @@ from dexterous_rl_manipulation_b200 import _lib  # noqa: E402
 CC = dx.CurriculumConfig
 n, steps = int(sys.argv[1]) if len(sys.argv) > 1 else 300_007, int(sys.argv[2]) if len(sys.argv) > 2 else 20_000
 full = (sys.argv[3] if len(sys.argv) > 3 else "full") == "full"       # "counts": auto-reset + counters only
+_lib.set_step_tile(sys.argv[4] if len(sys.argv) > 4 else "auto")       # tile width of the pipelined kernel
 kw = dict(max_episode_steps=60, reward_type="dense", auto_reset=True, respawn=True, loop_max_steps=60, track_episodes=full,
           groups=[CC.easy(), CC.medium(), CC.hard()], seed=77)
 envs = {impl: dx.BatchedManipulationEnv(n, "cuda", **kw) for impl in ("register", "tma")}

@@ -34,5 +34,5 @@ for n in (int(a) for a in (sys.argv[1:] or ["4096", "65536", "131072", "262144",
     e1.record()
     torch.cuda.synchronize()
     graph = e0.elapsed_time(e1) / 400 * 1e3
-    print(f"{os.environ.get('DEXSIM_PDL_GRAPH', '0')} n={n:8d} eager {eager:7.2f} us/step  graph replay {graph:7.2f} us/step", flush=True)
+    print(f"n={n:8d} eager {eager:7.2f} us/step  graph replay {graph:7.2f} us/step", flush=True)
     del env, replay

@@ -34,7 +34,7 @@ for chunks in (8, 16):
     dt = (time.perf_counter() - t0) / 20
     print(f"async chunks {chunks:3d}: {dt * 1e3:6.3f} ms/step  {n / dt / 1e6:7.1f} M env-steps/s", flush=True)
 
-# zero-copy: one launch, actions read from / results written to pinned host memory by the kernel itself
+# zero-copy: actions uploaded by the copy engine, results written to pinned host memory by the kernel itself
 env.host_zero_copy = True
 from dexterous_rl_manipulation_b200 import _lib  # noqa: E402
 L = _lib.lib()
@@ -48,5 +48,5 @@ for packed in (False, True):
             env.step_host(pool[t % 2], chunks=chunks, packed_contacts=packed)
         dt = (time.perf_counter() - t0) / 20
         print(f"zero-copy chunks {chunks:3d} packed={int(packed)}: {dt * 1e3:6.3f} ms/step  {n / dt / 1e6:7.1f} M env-steps/s  "
-              f"(zero-copy launches {int(L.dexsim_host_zero_copy_steps()) - z0}/20, kernel upload {os.environ.get('DEXSIM_ZC_KERNEL_UPLOAD', '0')})",
+              f"(zero-copy launches {int(L.dexsim_host_zero_copy_steps()) - z0}/20)",
               flush=True)

@@ -1,7 +1,8 @@
-"""Pipelined step kernel only, per batch size and variant: CUDA-event time per step.  Run once per experiment build
-(DEXSIM_LIB_PATH=exp/lib....so) to compare tile widths / CTA shapes (experiments only, not a bench number source).
+"""Pipelined step kernel only, per batch size and variant: CUDA-event time per step.  Run once per tile width, or once per
+experiment build (DEXSIM_LIB_PATH=exp/lib....so), to compare tile widths / CTA shapes (experiments only, not a bench
+number source).
 
-    python tools/time_tile.py [sizes,comma,separated] [reps] [variants,comma,separated]
+    python tools/time_tile.py [sizes,comma,separated] [reps] [variants,comma,separated] [auto|narrow|wide]
 """
 import os
 import sys
@@ -16,8 +17,10 @@ CC = dx.CurriculumConfig
 sizes = [int(x) for x in sys.argv[1].split(",")] if len(sys.argv) > 1 else [32768, 65536, 131072, 196608, 262144, 524288, 1048576]
 reps = int(sys.argv[2]) if len(sys.argv) > 2 else 300
 variants = sys.argv[3].split(",") if len(sys.argv) > 3 else ["plain", "counts", "track"]
+tile = sys.argv[4] if len(sys.argv) > 4 else "auto"
 _lib.set_step_impl("tma")
-print("lib", os.environ.get("DEXSIM_LIB_PATH", "default"), flush=True)
+_lib.set_step_tile(tile)
+print("lib", os.environ.get("DEXSIM_LIB_PATH", "default"), "tile", tile, flush=True)
 for n in sizes:
     g = torch.Generator(device="cuda").manual_seed(0)
     pool = [torch.rand(n, 15, device="cuda", generator=g) * 2 - 1 for _ in range(4)]
