@@ -11,7 +11,7 @@ import numpy as _np
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("DEXSIM_LIB_PATH") or os.path.join(HERE, "libdexsim_b200.so")   # env override: kernel experiments only
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 NJ, NF, OBS = 15, 5, 45
 NCOUNTERS = 18
 MAX_GROUPS = 256
@@ -102,6 +102,7 @@ EXPORTS = (
     "dexsim_device_info", "dexsim_set_step_impl", "dexsim_set_step_tile", "dexsim_set_rollout_impl", "dexsim_reset_predrawn",
     "dexsim_reset_philox", "dexsim_step", "dexsim_rollout", "dexsim_fill_policy_actions",
     "dexsim_fill_normal", "dexsim_classify_summary", "dexsim_step_host", "dexsim_pack_env", "dexsim_pack_env_tagged", "dexsim_step_single",
+    "dexsim_step_final",
     "dexsim_expand_contact_rows",
     "dexsim_host_zero_copy_steps",
 )
@@ -140,6 +141,7 @@ def lib():
     L.dexsim_reset_predrawn.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, vp, vp, vp, vp, vp]
     L.dexsim_reset_philox.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, vp, i32, vp]
     L.dexsim_step.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, C.POINTER(DexsimStepIO), vp]
+    L.dexsim_step_final.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, C.POINTER(DexsimStepIO), vp, vp]
     L.dexsim_rollout.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, i32, i32,
                                  C.POINTER(DexsimRolloutIO), vp]
     L.dexsim_fill_policy_actions.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, vp, vp]

@@ -8,6 +8,8 @@
 //                    state in registers for the whole launch, episodes auto-reset, per-group
 //                    counters aggregated in shared memory and flushed with one atomic per counter.
 //   reset_*_kernel   episode (re)initialisation from pre-drawn or Philox draws.
+//   finish_reset_kernel  the second launch of dexsim_step_final: episode end + reset of the envs a step without
+//                    auto-reset finished, after copying their terminal observation out.
 // No CPU fallback exists: every entry point launches CUDA work or returns an error code.
 #include <cstdio>
 #include <cstdlib>
@@ -493,6 +495,104 @@ reset_philox_kernel(const DexsimState st, const DexsimParams p, const DexsimGrou
         st.size[i] = size; st.mass[i] = mass; st.friction[i] = friction;
         if (st.ep_return) st.ep_return[i] = 0.0;
         if (st.ep_stats) { st.ep_stats[i] = 0u; st.ep_stats[ld + i] = 0u; }
+    }
+}
+
+// ---- finish-and-reset pass (dexsim_step_final) ----------------------------------------------------------
+// Runs after a step launched with auto_reset = 0 and no finished / counters / ret_sums outputs, and does what the step
+// kernels' in-kernel auto-reset does, from the arrays that step left behind: `done` from the flags and the step count,
+// `finished`, the episode end (counters staged per CTA as in step_kernel, labels when tracking), the reset through
+// load_env -> finish_and_reset -> store_env_full, and the reset observation's noise.  Before the reset, the column the
+// step returned (noisy_obs when observation noise is on, obs otherwise) is copied into `final_obs`; columns of envs
+// that did not finish are not written.  One thread per env of a grid-stride loop: a warp without a finished lane moves
+// on after one ballot.  `pdl`: launched as a programmatic dependent of the step (see launch_finish_reset).
+__global__ void __launch_bounds__(STEP_THREADS)
+finish_reset_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
+                    const uint16_t* __restrict__ group_of_env, const DexsimStepIO io, float* __restrict__ final_obs,
+                    const int pdl) {
+    __shared__ unsigned long long sh_cnt[SMEM_GROUPS_MAX * DEXSIM_NCOUNTERS];
+    __shared__ double sh_rs[SMEM_GROUPS_MAX * 2];
+    const bool count_episodes = io.counters != nullptr;
+    const bool staged = count_episodes && p.num_groups <= SMEM_GROUPS_MAX;
+    if (staged) {
+        for (int w = threadIdx.x; w < p.num_groups * DEXSIM_NCOUNTERS; w += STEP_THREADS) sh_cnt[w] = 0ull;
+        for (int w = threadIdx.x; w < p.num_groups * 2; w += STEP_THREADS) sh_rs[w] = 0.0;
+        __syncthreads();
+    }
+    // every global access below comes after the step grid has completed and flushed
+    if (pdl) asm volatile("griddepcontrol.wait;" ::: "memory");
+    const int64_t n = st.n, ld = st.ld;
+    const bool tracking = st.ep_return != nullptr && st.ep_stats != nullptr;
+    const bool noisy = io.noisy_obs && (io.obs_noise || io.sigma_obs != 0.0f);
+    const bool fused_obs = !io.obs_noise && io.noisy_obs && io.sigma_obs != 0.0f;
+    const float* __restrict__ returned = noisy ? io.noisy_obs : st.obs;
+    for (int64_t base = (int64_t)blockIdx.x * STEP_THREADS; base < n; base += (int64_t)gridDim.x * STEP_THREADS) {
+        const int64_t i = base + threadIdx.x;
+        bool done = false;
+        if (i < n) {
+            const int sc = st.step_count[i];
+            done = io.terminated[i] || io.truncated[i] || (p.loop_max_steps > 0 && sc >= p.loop_max_steps);
+            io.finished[i] = done ? 1 : 0;
+        }
+        if (__ballot_sync(0xffffffffu, done) == 0u) continue;
+        if (!done) continue;
+
+#pragma unroll
+        for (int row = 0; row < NOBS; ++row) final_obs[row * ld + i] = returned[row * ld + i];
+
+        EnvRegs e;
+        load_env(st, i, e);
+        const int64_t gid = p.env_gid0 + i;
+        const int g = group_index(group_of_env, i, gid, p.num_groups);
+        uint32_t episode = st.episode[i];
+        double ep_return = 0.0;
+        EpStats es{0u, 0u};
+        if (tracking) { ep_return = st.ep_return[i]; es.w0 = st.ep_stats[i]; es.w1 = st.ep_stats[ld + i]; }
+        unsigned long long* cnt = nullptr;
+        double* rs = nullptr;
+        if (count_episodes) {
+            cnt = (staged ? sh_cnt : reinterpret_cast<unsigned long long*>(io.counters)) + (int64_t)g * DEXSIM_NCOUNTERS;
+            if (io.ret_sums) rs = (staged ? sh_rs : io.ret_sums) + 2 * g;
+        }
+        double size, mass, friction;
+        finish_and_reset(e, p, groups[g], (uint32_t)gid, episode, ep_return, es, io.terminated[i] != 0, (int)io.num_contacts[i],
+                         cnt, rs, size, mass, friction, nullptr, /*classify=*/tracking);
+        st.episode[i] = episode;
+        st.size[i] = size; st.mass[i] = mass; st.friction[i] = friction;
+        store_env_full(st, i, e);
+        if (tracking) {
+            st.ep_return[i] = ep_return;
+            st.ep_stats[i] = es.w0; st.ep_stats[ld + i] = es.w1;
+        }
+        // the observation noise of the reset state, as the in-kernel reset draws it
+        float* __restrict__ out = io.noisy_obs;
+        if (io.noisy_obs && io.obs_noise) {
+#pragma unroll
+            for (int row = 0; row < NOBS; ++row) out[row * ld + i] = __fadd_rn(obs_entry(e, row), __ldg(io.obs_noise + row * ld + i));
+        } else if (fused_obs) {
+            const float sigma = io.sigma_obs > 0.0f ? io.sigma_obs : groups[g].sigma_obs;
+#pragma unroll
+            for (int b = 0; b < (NOBS + 3) / 4; ++b) {
+                const U4 o = rng_block(p.seed, (uint32_t)gid, episode, (uint32_t)e.sc, STREAM_OBS, (uint32_t)b);
+                float z[4];
+                normal_pair(o.x, o.y, z[0], z[1]);
+                normal_pair(o.z, o.w, z[2], z[3]);
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    const int row = 4 * b + k;
+                    if (row < NOBS) out[row * ld + i] = __fadd_rn(obs_entry(e, row), __fmul_rn(sigma, z[k]));
+                }
+            }
+        }
+    }
+    if (staged) {
+        __syncthreads();
+        unsigned long long* gc = reinterpret_cast<unsigned long long*>(io.counters);
+        for (int w = threadIdx.x; w < p.num_groups * DEXSIM_NCOUNTERS; w += STEP_THREADS)
+            if (sh_cnt[w]) atomicAdd(&gc[w], sh_cnt[w]);
+        if (io.ret_sums)
+            for (int w = threadIdx.x; w < p.num_groups * 2; w += STEP_THREADS)
+                if (sh_rs[w] != 0.0) atomicAdd(&io.ret_sums[w], sh_rs[w]);
     }
 }
 
@@ -1000,6 +1100,31 @@ static int launch_step(const DexsimState* st, const DexsimParams* p, const Dexsi
     return cuda_rc(cudaGetLastError());
 }
 
+// The pass of dexsim_step_final: one resident wave of CTAs, launched as a programmatic dependent of the step, so that its
+// launch and counter staging overlap the step's tail (griddepcontrol.wait orders every global access behind the step).
+static int launch_finish_reset(const DexsimState& st, const DexsimParams& p, const DexsimGroup* groups, const uint16_t* goe,
+                               const DexsimStepIO& io, float* final_obs, cudaStream_t s, int sm_count) {
+    static thread_local int occupancy[64] = {0};
+    int dev = 0;
+    cudaError_t err = cudaGetDevice(&dev);
+    if (err != cudaSuccess) return -(int)err;
+    int uncached = 0;
+    int& ctas_per_sm = (dev >= 0 && dev < 64) ? occupancy[dev] : uncached;
+    if (ctas_per_sm == 0) {
+        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, finish_reset_kernel, STEP_THREADS, 0);
+        if (err != cudaSuccess) return -(int)err;
+        if (ctas_per_sm < 1) ctas_per_sm = 1;
+    }
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)grid_for(st.n, STEP_THREADS, ctas_per_sm, sm_count));
+    cfg.blockDim = dim3(STEP_THREADS); cfg.dynamicSmemBytes = 0; cfg.stream = s;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr; cfg.numAttrs = 1;
+    return cuda_rc(cudaLaunchKernelEx(&cfg, finish_reset_kernel, st, p, groups, goe, io, final_obs, /*pdl=*/1));
+}
+
 }  // namespace dexsim
 
 namespace dexsim {
@@ -1106,6 +1231,30 @@ int dexsim_step_single(const DexsimState* st, const DexsimParams* p, const Dexsi
                        const uint16_t* group_of_env, const DexsimStepIO* io, double* out64, double tag, void* stream) {
     if (!p || !out64) return DEXSIM_E_NULL;
     return launch_step(st, p, groups, group_of_env, io, (cudaStream_t)stream, out64, tag);
+}
+
+int dexsim_step_final(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                      const uint16_t* group_of_env, const DexsimStepIO* io, float* final_obs, void* stream) {
+    if (!p || !io) return DEXSIM_E_NULL;
+    if (!p->auto_reset || io->host_static_rows || (io->flags & DEXSIM_STEP_HOST_ALL_ROWS)) return DEXSIM_E_PARAM;
+    if (!final_obs || !io->finished) return DEXSIM_E_NULL;
+    int rc = check_state(st);
+    if (rc) return rc;
+    // the limits of an auto-reset call (the step below runs without auto-reset and would not check them)
+    rc = check_params(p, true, groups, st->ep_return != nullptr);
+    if (rc) return rc;
+    // the step without the reset: it leaves the observation of the step that ended an episode in obs / noisy_obs
+    DexsimParams sp = *p;
+    sp.auto_reset = 0;
+    DexsimStepIO sio = *io;
+    sio.finished = nullptr; sio.counters = nullptr; sio.ret_sums = nullptr;
+    const cudaStream_t s = (cudaStream_t)stream;
+    rc = launch_step(st, &sp, groups, group_of_env, &sio, s);
+    if (rc || st->n == 0) return rc;
+    DeviceInfo di;
+    rc = device_info_cached(di);
+    if (rc) return rc;
+    return launch_finish_reset(*st, *p, groups, group_of_env, *io, final_obs, s, di.sm_count);
 }
 
 int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,

@@ -120,11 +120,19 @@ class BatchedManipulationEnv:
         group_of_env=None,
         observation_noise_std: float = 0.0,
         dynamics_noise_std: float = 0.0,
+        final_observation: bool = False,
     ):
         if num_fingers != 5 or joints_per_finger != 3:
             raise _lib.DexsimError(-1006, "BatchedManipulationEnv")
         if num_envs < 1:
             raise ValueError("num_envs must be >= 1")
+        self.final_observation = bool(final_observation)
+        if self.final_observation and not auto_reset:
+            raise ValueError("final_observation=True needs auto_reset=True: without it step() does not reset, and the "
+                             "returned observation is already the final one")
+        if self.final_observation and int(num_envs) == 1:
+            raise NotImplementedError("final_observation is for batched envs; num_envs == 1 mirrors the reference, "
+                                      "which has no auto-reset")
         self._lib = _lib.lib()
         self.device = torch.device(device)
         if self.device.type != "cuda":
@@ -195,6 +203,8 @@ class BatchedManipulationEnv:
         self._truncated = z(ld, dtype=torch.uint8)
         self._num_contacts = z(ld, dtype=torch.uint8)
         self._finished = z(ld, dtype=torch.uint8) if self.auto_reset else None
+        # terminal observation of every episode a step ends (dexsim_step_final), read where info["finished"]
+        self._final_obs = z(45, ld, dtype=torch.float32) if self.final_observation else None
         self._action_dev = z(n, 15, dtype=torch.float32)
         self._sched = z(_L.SCHED_WORDS, dtype=torch.int32)      # dynamic tile scheduler words of the pipelined step kernel
         self._noisy_obs = None
@@ -233,6 +243,7 @@ class BatchedManipulationEnv:
         self._h_primed_slot = None                       # result slot whose pinned observation is current (see step_host)
         self._state_ref, self._params_ref, self._io_ref = C.byref(self._state), C.byref(self._params), C.byref(self._io)
         self._goe_ptr = self._ptr(self._goe)
+        self._final_obs_ptr = self._ptr(self._final_obs)
         self._step_out = None
         if not self.single:
             self._step_out = (self._obs_view, self._reward[:n], self._terminated[:n].view(torch.bool),
@@ -584,10 +595,14 @@ class BatchedManipulationEnv:
                 io.dyn_noise = io.obs_noise = io.noisy_obs = None
                 io.sigma_dyn = io.sigma_obs = 0.0
                 self._io_has_noise = False
-            rc = self._lib.dexsim_step(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
-                                       self._io_ref, _raw_stream(self.device.index))
+            if self._final_obs is None:
+                rc = self._lib.dexsim_step(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
+                                           self._io_ref, _raw_stream(self.device.index))
+            else:
+                rc = self._lib.dexsim_step_final(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
+                                                 self._io_ref, self._final_obs_ptr, _raw_stream(self.device.index))
             if rc:
-                raise _lib.DexsimError(rc, "dexsim_step")
+                raise _lib.DexsimError(rc, "dexsim_step_final" if self._final_obs is not None else "dexsim_step")
             return self._step_out
         if (self.single and dyn_noise is None and obs_noise is None and not self._noisy_env
                 and not (isinstance(action, torch.Tensor) and action.is_cuda)
@@ -658,6 +673,9 @@ class BatchedManipulationEnv:
             io.sigma_obs = self.observation_noise_std if self.observation_noise_std > 0.0 else -1.0
             io.noisy_obs = self._noisy_obs.data_ptr()
         post_step_noise = want_obs and obs_noise is None and not fused and self.observation_noise_std > 0.0
+        if post_step_noise and self._final_obs is not None:
+            raise NotImplementedError("final_observation needs the observation noise drawn inside the step kernel "
+                                      "(fused_noise=True)")
         if self.single and not post_step_noise:
             # one launch: the step and the packed read-back of what step() returns (dexsim_step_single)
             tag = self._next_pack_tag()
@@ -665,8 +683,7 @@ class BatchedManipulationEnv:
                                                     self._io_ref, self._pack_host.data_ptr(), tag, self._stream()),
                        "dexsim_step_single")
             return self._single_wait_decode(tag, after_reset=False)
-        _lib.check(self._lib.dexsim_step(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
-                                         self._io_ref, self._stream()), "dexsim_step")
+        self._launch_step()
         if post_step_noise:
             # Philox observation noise is keyed by (episode, step count AFTER the step), so it is
             # drawn once the step has run (evaluation/robustness_tests.py:204-205)
@@ -729,9 +746,17 @@ class BatchedManipulationEnv:
         io.action, io.action_layout = action_soa.data_ptr(), 0
         io.dyn_noise = io.obs_noise = io.noisy_obs = None
         io.sigma_dyn = io.sigma_obs = 0.0
-        _lib.check(self._lib.dexsim_step(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
-                                         self._io_ref, self._stream()), "dexsim_step")
+        self._launch_step()
         return self._step_out
+
+    def _launch_step(self):
+        """dexsim_step, or dexsim_step_final when the env returns final observations."""
+        if self._final_obs is None:
+            _lib.check(self._lib.dexsim_step(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
+                                             self._io_ref, self._stream()), "dexsim_step")
+        else:
+            _lib.check(self._lib.dexsim_step_final(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
+                                                   self._io_ref, self._final_obs_ptr, self._stream()), "dexsim_step_final")
 
     def _reset_outputs(self):
         obs = self._emit_obs(reset=True)          # also draws the reset observation's noise when enabled
@@ -828,12 +853,16 @@ class BatchedManipulationEnv:
                     "closure": self._comps[2, :n], "stability": self._comps[3, :n]}
             if self._finished is not None:
                 self._info["finished"] = self._finished[:n].view(torch.bool)
+            if self._final_obs is not None:
+                # batch first like obs; row i is the observation that ended env i's episode, valid where info["finished"]
+                self._info["final_observation"] = self._final_obs[:, :n].t()
             if self.info_success:
                 self._info["success"] = self._terminated[:n].view(torch.bool)
         if after_reset:
             info = dict(self._info)
             info["num_contacts"] = sum(((self._cmask[:n] >> f) & 1) for f in range(5)).to(torch.uint8)
             info.pop("reward_components", None)
+            info.pop("final_observation", None)
             return info
         return self._info
 
@@ -873,6 +902,9 @@ class BatchedManipulationEnv:
         (-11 % download bytes).  ``expand_contacts_host(slot)`` fills the columns in on the host when needed."""
         if not self._did_reset:
             raise RuntimeError("call reset() before step_host()")
+        if self.final_observation:
+            raise NotImplementedError("step_host() does not return final observations: step a final_observation env "
+                                      "with step()")
         n = self.num_envs
         b = self._host_buffers(slot)
         a = action_host if isinstance(action_host, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(action_host, np.float32))

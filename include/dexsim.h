@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define DEXSIM_ABI_VERSION 3
+#define DEXSIM_ABI_VERSION 4
 #define DEXSIM_NJ 15      /* joints            envs/manipulation_env.py:52 */
 #define DEXSIM_NF 5       /* fingers           envs/manipulation_env.py:50 */
 #define DEXSIM_OBS 45     /* observation width envs/manipulation_env.py:96-106 */
@@ -242,6 +242,21 @@ int dexsim_reset_philox(const DexsimState* st, const DexsimParams* p, const Dexs
  *      and CombinedNoiseWrapper.step (evaluation/robustness_tests.py:177-207) ---------------- */
 int dexsim_step(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
                 const uint16_t* group_of_env, const DexsimStepIO* io, void* stream);
+
+/* dexsim_step with auto-reset that also returns the terminal observation of every episode it ends (what a trainer
+ * bootstraps a value estimate from at truncation; Gymnasium's info["final_observation"]).  Same arguments as
+ * dexsim_step plus `final_obs`, device float32 [45, ld].  Two launches on `stream`: the step without the reset, then a
+ * finish-and-reset pass over the envs whose episode ended.
+ *   - For every env with io->finished[i] == 1 after the call, column i of final_obs is bit for bit what dexsim_step with
+ *     auto_reset = 0 would have left in st->obs -- or in io->noisy_obs when observation noise is on -- for the same
+ *     inputs.  Other columns of final_obs are not written.
+ *   - Every other state array and output equals what dexsim_step with auto-reset produces; io->ret_sums is a float64
+ *     atomic sum and equal only up to summation order.
+ *   - Returns, before anything touches the device: DEXSIM_E_PARAM when p->auto_reset == 0, io->host_static_rows is set
+ *     or io->flags has DEXSIM_STEP_HOST_ALL_ROWS; DEXSIM_E_NULL when final_obs or io->finished is NULL. */
+int dexsim_step_final(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                      const uint16_t* group_of_env, const DexsimStepIO* io,
+                      float* final_obs /* device [45, ld] */, void* stream);
 
 /* ---- fused rollout: replaces the caller loops training/episode_utils.py:42-53,
  *      evaluation/evaluator.py:135-158, evaluation/robustness_tests.py:292-304 with the policy
