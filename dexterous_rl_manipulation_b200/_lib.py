@@ -11,7 +11,7 @@ import numpy as _np
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("DEXSIM_LIB_PATH") or os.path.join(HERE, "libdexsim_b200.so")   # env override: kernel experiments only
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 NJ, NF, OBS = 15, 5, 45
 NCOUNTERS = 18
 MAX_GROUPS = 256
@@ -102,7 +102,7 @@ EXPORTS = (
     "dexsim_device_info", "dexsim_set_step_impl", "dexsim_set_step_tile", "dexsim_set_rollout_impl", "dexsim_reset_predrawn",
     "dexsim_reset_philox", "dexsim_step", "dexsim_rollout", "dexsim_fill_policy_actions",
     "dexsim_fill_normal", "dexsim_classify_summary", "dexsim_step_host", "dexsim_pack_env", "dexsim_pack_env_tagged", "dexsim_step_single",
-    "dexsim_step_final",
+    "dexsim_step_final", "dexsim_step_host_final",
     "dexsim_expand_contact_rows",
     "dexsim_host_zero_copy_steps",
 )
@@ -154,6 +154,8 @@ def lib():
                                           C.POINTER(i32), C.POINTER(i32)]
     L.dexsim_step_host.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, C.POINTER(DexsimStepIO),
                                    vp, vp, vp, vp, vp, vp, vp, i32, i32, vp]
+    L.dexsim_step_host_final.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, C.POINTER(DexsimStepIO),
+                                         vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, vp]
     L.dexsim_expand_contact_rows.argtypes = [vp, vp, i64, i64]
     L.dexsim_host_zero_copy_steps.argtypes = []
     L.dexsim_host_zero_copy_steps.restype = C.c_int64

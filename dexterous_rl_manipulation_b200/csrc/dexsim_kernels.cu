@@ -8,8 +8,8 @@
 //                    state in registers for the whole launch, episodes auto-reset, per-group
 //                    counters aggregated in shared memory and flushed with one atomic per counter.
 //   reset_*_kernel   episode (re)initialisation from pre-drawn or Philox draws.
-//   finish_reset_kernel  the second launch of dexsim_step_final: episode end + reset of the envs a step without
-//                    auto-reset finished, after copying their terminal observation out.
+//   finish_reset_kernel  the second launch of dexsim_step_final and dexsim_step_host_final: episode end + reset of
+//                    the envs a step without auto-reset finished, after copying their terminal observation out.
 // No CPU fallback exists: every entry point launches CUDA work or returns an error code.
 #include <cstdio>
 #include <cstdlib>
@@ -506,10 +506,27 @@ reset_philox_kernel(const DexsimState st, const DexsimParams p, const DexsimGrou
 // step returned (noisy_obs when observation noise is on, obs otherwise) is copied into `final_obs`; columns of envs
 // that did not finish are not written.  One thread per env of a grid-stride loop: a warp without a finished lane moves
 // on after one ballot.  `pdl`: launched as a programmatic dependent of the step (see launch_finish_reset).
+//
+// HOST (dexsim_step_host_final): the outputs of `hf` instead of `final_obs`, all of them device aliases of the caller's
+// mapped page-locked buffers, offset to the chunk.
+struct FinishHost {
+    float* final_obs;       // [n, 45] batch-first: row i <- the returned observation of env i, finished envs only
+    float* obs;             // the host observation [45, ld] or NULL: rows 30, 31, 37, 38 of a reset env (the static-row
+                            // mirror); with `zero_copy` also every other row the zero-copy step writes (0-32, 37-39)
+    uint8_t* cmask;         // zero_copy: the host contact masks (of reset envs)
+    uint8_t* terminated;    // zero_copy: the flags of every env, which the step left on the device for this pass
+    uint8_t* truncated;
+    uint8_t* num_contacts;  // (NULL: the caller has no buffer for them)
+    uint8_t* finished;
+    int zero_copy;
+};
+constexpr int FINISH_HOST_SMEM = STEP_THREADS * NOBS * 4;      // one [32 envs, 45] record block per warp
+
+template <bool HOST>
 __global__ void __launch_bounds__(STEP_THREADS)
 finish_reset_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
                     const uint16_t* __restrict__ group_of_env, const DexsimStepIO io, float* __restrict__ final_obs,
-                    const int pdl) {
+                    const int pdl, const FinishHost hf) {
     __shared__ unsigned long long sh_cnt[SMEM_GROUPS_MAX * DEXSIM_NCOUNTERS];
     __shared__ double sh_rs[SMEM_GROUPS_MAX * 2];
     const bool count_episodes = io.counters != nullptr;
@@ -533,12 +550,46 @@ finish_reset_kernel(const DexsimState st, const DexsimParams p, const DexsimGrou
             const int sc = st.step_count[i];
             done = io.terminated[i] || io.truncated[i] || (p.loop_max_steps > 0 && sc >= p.loop_max_steps);
             io.finished[i] = done ? 1 : 0;
+            if (HOST && hf.zero_copy) {              // consecutive lanes, consecutive bytes: one PCIe write per warp and vector
+                hf.terminated[i] = io.terminated[i];
+                hf.truncated[i] = io.truncated[i];
+                if (hf.num_contacts) hf.num_contacts[i] = io.num_contacts[i];
+                hf.finished[i] = done ? 1 : 0;
+            }
         }
-        if (__ballot_sync(0xffffffffu, done) == 0u) continue;
+        const unsigned fin = __ballot_sync(0xffffffffu, done);
+        if (fin == 0u) continue;
+        if (HOST) {
+            // Records leave from consecutive lanes: 4-byte writes scattered over host memory would cost a PCIe transaction
+            // each.  The finished lanes stage their columns in the warp's block of shared memory; the warp then writes
+            // each record as 45 contiguous floats (two stores), or, when every lane finished, 32 x 45 contiguous floats.
+            extern __shared__ float sh_rec[];
+            const int lane = threadIdx.x & 31;
+            float* rec = sh_rec + (threadIdx.x - lane) * NOBS;
+            if (done) {
+#pragma unroll
+                for (int row = 0; row < NOBS; ++row) rec[lane * NOBS + row] = returned[row * ld + i];
+            }
+            __syncwarp();
+            float* dst = hf.final_obs + (i - lane) * NOBS;
+            if (fin == 0xffffffffu) {
+#pragma unroll
+                for (int k = 0; k < NOBS; ++k) dst[k * 32 + lane] = rec[k * 32 + lane];
+            } else {
+                for (unsigned m = fin; m; m &= m - 1u) {
+                    const int j = __ffs(m) - 1;
+                    dst[j * NOBS + lane] = rec[j * NOBS + lane];
+                    if (lane < NOBS - 32) dst[j * NOBS + 32 + lane] = rec[j * NOBS + 32 + lane];
+                }
+            }
+            __syncwarp();
+        }
         if (!done) continue;
 
+        if (!HOST) {
 #pragma unroll
-        for (int row = 0; row < NOBS; ++row) final_obs[row * ld + i] = returned[row * ld + i];
+            for (int row = 0; row < NOBS; ++row) final_obs[row * ld + i] = returned[row * ld + i];
+        }
 
         EnvRegs e;
         load_env(st, i, e);
@@ -559,7 +610,19 @@ finish_reset_kernel(const DexsimState st, const DexsimParams p, const DexsimGrou
                          cnt, rs, size, mass, friction, nullptr, /*classify=*/tracking);
         st.episode[i] = episode;
         st.size[i] = size; st.mass[i] = mass; st.friction[i] = friction;
-        store_env_full(st, i, e);
+        store_env_full(st, i, e, HOST ? hf.obs : nullptr);
+        if (HOST && hf.zero_copy) {
+            // the zero-copy step sent this env's pre-reset rows and mask to the host: overwrite them with the reset state
+            float* __restrict__ h = hf.obs;
+#pragma unroll
+            for (int j = 0; j < NJ; ++j) {
+                h[(DEXSIM_ROW_JP + j) * ld + i] = e.jp[j];
+                h[(DEXSIM_ROW_JV + j) * ld + i] = e.jv[j];
+            }
+            h[(DEXSIM_ROW_OP + 2) * ld + i] = (float)e.op[2];
+            h[(DEXSIM_ROW_OV + 2) * ld + i] = e.ov[2];
+            hf.cmask[i] = (uint8_t)e.cmask;
+        }
         if (tracking) {
             st.ep_return[i] = ep_return;
             st.ep_stats[i] = es.w0; st.ep_stats[ld + i] = es.w1;
@@ -1100,10 +1163,14 @@ static int launch_step(const DexsimState* st, const DexsimParams* p, const Dexsi
     return cuda_rc(cudaGetLastError());
 }
 
-// The pass of dexsim_step_final: one resident wave of CTAs, launched as a programmatic dependent of the step, so that its
-// launch and counter staging overlap the step's tail (griddepcontrol.wait orders every global access behind the step).
+// The pass of dexsim_step_final (HOST: of dexsim_step_host_final): one resident wave of CTAs, launched as a programmatic
+// dependent of the step, so that its launch and counter staging overlap the step's tail (griddepcontrol.wait orders every
+// global access behind the step).
+template <bool HOST>
 static int launch_finish_reset(const DexsimState& st, const DexsimParams& p, const DexsimGroup* groups, const uint16_t* goe,
-                               const DexsimStepIO& io, float* final_obs, cudaStream_t s, int sm_count) {
+                               const DexsimStepIO& io, float* final_obs, const FinishHost& hf, cudaStream_t s, int sm_count) {
+    auto kern = finish_reset_kernel<HOST>;
+    const int smem = HOST ? FINISH_HOST_SMEM : 0;
     static thread_local int occupancy[64] = {0};
     int dev = 0;
     cudaError_t err = cudaGetDevice(&dev);
@@ -1111,18 +1178,22 @@ static int launch_finish_reset(const DexsimState& st, const DexsimParams& p, con
     int uncached = 0;
     int& ctas_per_sm = (dev >= 0 && dev < 64) ? occupancy[dev] : uncached;
     if (ctas_per_sm == 0) {
-        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, finish_reset_kernel, STEP_THREADS, 0);
+        if (HOST) {                 // the record blocks and the static counter arrays together exceed the default 48 KB
+            err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+            if (err != cudaSuccess) return -(int)err;
+        }
+        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kern, STEP_THREADS, smem);
         if (err != cudaSuccess) return -(int)err;
         if (ctas_per_sm < 1) ctas_per_sm = 1;
     }
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid_for(st.n, STEP_THREADS, ctas_per_sm, sm_count));
-    cfg.blockDim = dim3(STEP_THREADS); cfg.dynamicSmemBytes = 0; cfg.stream = s;
+    cfg.blockDim = dim3(STEP_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = s;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    return cuda_rc(cudaLaunchKernelEx(&cfg, finish_reset_kernel, st, p, groups, goe, io, final_obs, /*pdl=*/1));
+    return cuda_rc(cudaLaunchKernelEx(&cfg, kern, st, p, groups, goe, io, final_obs, /*pdl=*/1, hf));
 }
 
 }  // namespace dexsim
@@ -1254,7 +1325,7 @@ int dexsim_step_final(const DexsimState* st, const DexsimParams* p, const Dexsim
     DeviceInfo di;
     rc = device_info_cached(di);
     if (rc) return rc;
-    return launch_finish_reset(*st, *p, groups, group_of_env, *io, final_obs, s, di.sm_count);
+    return launch_finish_reset<false>(*st, *p, groups, group_of_env, *io, final_obs, FinishHost{}, s, di.sm_count);
 }
 
 int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
@@ -1457,19 +1528,45 @@ int dexsim_expand_contact_rows(float* h_obs, const uint8_t* h_contact_mask, int6
 
 int64_t dexsim_host_zero_copy_steps(void) { return g_zero_copy_steps.load(std::memory_order_relaxed); }
 
-int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
-                     const uint16_t* group_of_env, const DexsimStepIO* io, const float* h_action, float* h_obs,
-                     float* h_reward, uint8_t* h_terminated, uint8_t* h_truncated, uint8_t* h_num_contacts,
-                     uint8_t* h_contact_mask, int32_t chunks, int32_t flags, void* stream) {
+static void* mapped_alias(const void* h) {       // device alias of mapped page-locked host memory, else NULL
+    if (!h) return nullptr;
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, h) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer)
+        return attr.devicePointer;
+    (void)cudaGetLastError();
+    return nullptr;
+}
+
+// dexsim_step_host and, with final outputs (h_final_obs != NULL, argument checks done by the caller),
+// dexsim_step_host_final: per chunk, the step without the reset and then the finish-and-reset pass, after which
+// everything that chunk moves to the host is enqueued.
+static int step_host_impl(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                          const uint16_t* group_of_env, const DexsimStepIO* io, const float* h_action, float* h_obs,
+                          float* h_reward, uint8_t* h_terminated, uint8_t* h_truncated, uint8_t* h_num_contacts,
+                          uint8_t* h_contact_mask, uint8_t* h_finished, float* h_final_obs, int32_t chunks, int32_t flags,
+                          void* stream) {
     int rc = check_state(st);
     if (rc) return rc;
     if (!p || !io || !io->action || !h_action || !h_reward || !h_terminated || !h_truncated) return DEXSIM_E_NULL;
     if ((flags & DEXSIM_HOST_PACKED_CONTACTS) && !h_contact_mask) return DEXSIM_E_NULL;
     if (io->dyn_noise || io->obs_noise || io->noisy_obs || io->sigma_dyn != 0.0f || io->sigma_obs != 0.0f)
         return DEXSIM_E_PARAM;   // noise: use dexsim_step
+    const bool final = h_final_obs != nullptr;
+    float* d_final = nullptr;                    // device alias of h_final_obs
+    if (final) {
+        d_final = static_cast<float*>(mapped_alias(h_final_obs));
+        if (!d_final) return DEXSIM_E_PARAM;
+    }
     cudaStream_t user = (cudaStream_t)stream;
     const int64_t n = st->n, ld = st->ld;
     if (n == 0) return 0;
+    int sm_count = 0;
+    if (final) {
+        DeviceInfo di;
+        rc = device_info_cached(di);
+        if (rc) return rc;
+        sm_count = di.sm_count;
+    }
     const bool aos = io->action_layout == 1;
     // Zero-copy transport (DEXSIM_HOST_ZERO_COPY): the pipelined kernel itself writes every result into the caller's mapped
     // page-locked buffers -- the joint rows as a second bulk tensor store per tile, object z, its velocity and the contact
@@ -1481,25 +1578,27 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
     // chunk offsets are multiples of 1,024 envs, so every chunk keeps the batch's alignment, and the fold rule below keeps
     // every chunk at one tile or more.  Not eligible (a buffer that is not mapped, fewer envs than a tile, the register
     // kernel selected): the copy transport below runs instead.
+    // With final outputs the step leaves its flags on the device, where the pass reads them; the pass writes them, and
+    // `finished`, to the host (zflags).
     DexsimStepIO zio = *io;
     bool zc = false;
+    FinishHost zflags = {};
     if ((flags & DEXSIM_HOST_ZERO_COPY) && (flags & DEXSIM_HOST_PACKED_CONTACTS) && h_obs) {
-        auto alias = [](const void* h) -> void* {
-            if (!h) return nullptr;
-            cudaPointerAttributes attr;
-            if (cudaPointerGetAttributes(&attr, h) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer)
-                return attr.devicePointer;
-            (void)cudaGetLastError();
-            return nullptr;
-        };
-        zio.host_static_rows = static_cast<float*>(alias(h_obs));
-        zio.reward = static_cast<float*>(alias(h_reward));
-        zio.terminated = static_cast<uint8_t*>(alias(h_terminated));
-        zio.truncated = static_cast<uint8_t*>(alias(h_truncated));
-        if (h_num_contacts) zio.num_contacts = static_cast<uint8_t*>(alias(h_num_contacts));
-        zio.host_cmask = static_cast<uint8_t*>(alias(h_contact_mask));
+        zio.host_static_rows = static_cast<float*>(mapped_alias(h_obs));
+        zio.reward = static_cast<float*>(mapped_alias(h_reward));
+        zflags.terminated = static_cast<uint8_t*>(mapped_alias(h_terminated));
+        zflags.truncated = static_cast<uint8_t*>(mapped_alias(h_truncated));
+        zflags.num_contacts = h_num_contacts ? static_cast<uint8_t*>(mapped_alias(h_num_contacts)) : nullptr;
+        zio.host_cmask = static_cast<uint8_t*>(mapped_alias(h_contact_mask));
         zio.flags |= DEXSIM_STEP_HOST_ALL_ROWS;
-        zc = zio.host_static_rows && zio.reward && zio.terminated && zio.truncated && zio.num_contacts && zio.host_cmask &&
+        if (final) {
+            zflags.finished = static_cast<uint8_t*>(mapped_alias(h_finished));
+        } else {
+            zio.terminated = zflags.terminated; zio.truncated = zflags.truncated;
+            if (h_num_contacts) zio.num_contacts = zflags.num_contacts;
+        }
+        zc = zio.host_static_rows && zio.reward && zflags.terminated && zflags.truncated &&
+             (h_num_contacts ? zflags.num_contacts : io->num_contacts) && zio.host_cmask && (!final || zflags.finished) &&
              pipeline_eligible(*st, zio, step_track(*st, *p, zio), step_extra_io(zio), /*single=*/false);
     }
     // chunk boundaries are multiples of 1024 envs (tile- and alignment-friendly)
@@ -1568,6 +1667,10 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
             err = cudaMemcpyAsync(h_contact_mask + lo, st->cmask + lo, (size_t)m, cudaMemcpyDeviceToHost, s);
             if (err != cudaSuccess) return -(int)err;
         }
+        if (final) {
+            err = cudaMemcpyAsync(h_finished + lo, io->finished + lo, (size_t)m, cudaMemcpyDeviceToHost, s);
+            if (err != cudaSuccess) return -(int)err;
+        }
         return 0;
     };
     for (int c = 0; c < nchunks && rc == 0; ++c) {
@@ -1596,7 +1699,28 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
         else err = cudaMemcpy2DAsync(d_action, (size_t)ld * 4, h_action + lo, (size_t)ld * 4, (size_t)m * 4, NJ, cudaMemcpyHostToDevice, s);
         if (err != cudaSuccess) { rc = -(int)err; break; }
         if (tracing) cudaEventRecord(g_trace.up[c], s);
-        rc = launch_step(&sub, &sp, groups, group_of_env ? group_of_env + lo : nullptr, &sio, s);
+        const uint16_t* goe = group_of_env ? group_of_env + lo : nullptr;
+        if (!final) {
+            rc = launch_step(&sub, &sp, groups, goe, &sio, s);
+        } else {
+            // as dexsim_step_final: the step without the reset, then the pass, which resets, counts and writes the records
+            DexsimParams np = sp;
+            np.auto_reset = 0;
+            DexsimStepIO nio = sio;
+            nio.finished = nullptr; nio.counters = nullptr; nio.ret_sums = nullptr;
+            rc = launch_step(&sub, &np, groups, goe, &nio, s);
+            if (rc) break;
+            FinishHost hf = {};
+            hf.final_obs = d_final + lo * NOBS;
+            hf.obs = sio.host_static_rows;
+            if (zc) {
+                hf.zero_copy = 1;
+                hf.cmask = sio.host_cmask;
+                hf.terminated = zflags.terminated + lo; hf.truncated = zflags.truncated + lo; hf.finished = zflags.finished + lo;
+                hf.num_contacts = zflags.num_contacts ? zflags.num_contacts + lo : nullptr;
+            }
+            rc = launch_finish_reset<true>(sub, sp, groups, goe, sio, nullptr, hf, s, sm_count);
+        }
         if (rc) break;
         if (tracing) cudaEventRecord(g_trace.k[c], s);
         if (zc) {                                        // every result is already on its way to the host buffers
@@ -1687,6 +1811,31 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
         fprintf(stderr, "  per-env vectors down %8.1f\n", v * 1e3);
     }
     return rc ? rc : sync_rc;
+}
+
+int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                     const uint16_t* group_of_env, const DexsimStepIO* io, const float* h_action, float* h_obs,
+                     float* h_reward, uint8_t* h_terminated, uint8_t* h_truncated, uint8_t* h_num_contacts,
+                     uint8_t* h_contact_mask, int32_t chunks, int32_t flags, void* stream) {
+    return step_host_impl(st, p, groups, group_of_env, io, h_action, h_obs, h_reward, h_terminated, h_truncated,
+                          h_num_contacts, h_contact_mask, nullptr, nullptr, chunks, flags, stream);
+}
+
+int dexsim_step_host_final(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                           const uint16_t* group_of_env, const DexsimStepIO* io, const float* h_action, float* h_obs,
+                           float* h_reward, uint8_t* h_terminated, uint8_t* h_truncated, uint8_t* h_num_contacts,
+                           uint8_t* h_contact_mask, uint8_t* h_finished, float* h_final_obs, int32_t chunks, int32_t flags,
+                           void* stream) {
+    if (!p || !io) return DEXSIM_E_NULL;
+    if (!p->auto_reset) return DEXSIM_E_PARAM;
+    if (!h_finished || !h_final_obs || !io->finished) return DEXSIM_E_NULL;
+    int rc = check_state(st);
+    if (rc) return rc;
+    // the limits of an auto-reset call (the step runs without auto-reset and would not check them)
+    rc = check_params(p, true, groups, st->ep_return != nullptr);
+    if (rc) return rc;
+    return step_host_impl(st, p, groups, group_of_env, io, h_action, h_obs, h_reward, h_terminated, h_truncated,
+                          h_num_contacts, h_contact_mask, h_finished, h_final_obs, chunks, flags, stream);
 }
 
 }  // extern "C"

@@ -879,6 +879,10 @@ class BatchedManipulationEnv:
                  "cmask": pin(ld, dtype=torch.uint8)}
             b["obs"][_L.ROW_QUAT].fill_(1.0)          # constant quaternion rows are never re-copied
             b["info"] = {"num_contacts": b["nc"][:n], "contact_mask": b["cmask"][:n]}
+            if self.final_observation:
+                # written by the finish-and-reset pass through the mapped buffer: ~180 bytes per FINISHED env cross PCIe
+                b["fin"], b["final"] = pin(ld, dtype=torch.uint8), pin(n, 45, dtype=torch.float32)
+                b["info"].update(finished=b["fin"][:n].view(torch.bool), final_observation=b["final"])
             b["out"] = (b["obs"][:, :n].t(), b["reward"][:n], b["term"][:n].view(torch.bool), b["trunc"][:n].view(torch.bool),
                         b["info"])
             bufs[slot] = b
@@ -899,12 +903,15 @@ class BatchedManipulationEnv:
         next step (or of another env group) with this step's download.
         ``packed_contacts=True``: the five 0/1 contact columns of the observation (obs[:, 40:45]) are NOT downloaded;
         ``info["contact_mask"]`` (uint8, bit f = finger f) carries the same information in one byte per env
-        (-11 % download bytes).  ``expand_contacts_host(slot)`` fills the columns in on the host when needed."""
+        (-11 % download bytes).  ``expand_contacts_host(slot)`` fills the columns in on the host when needed.
+
+        ``final_observation=True`` envs (dexsim_step_host_final): ``info["finished"]`` (bool [num_envs]) marks the envs
+        whose episode ended in this step and was reset, and ``info["final_observation"]`` (float32 [num_envs, 45]) holds,
+        where ``info["finished"]``, the observation that ended it -- all 45 entries, also with ``packed_contacts``.  Its
+        other rows keep stale values.  Both are pinned buffers of the ``slot`` like the other outputs; the GPU writes the
+        rows of finished envs only, straight into the buffer."""
         if not self._did_reset:
             raise RuntimeError("call reset() before step_host()")
-        if self.final_observation:
-            raise NotImplementedError("step_host() does not return final observations: step a final_observation env "
-                                      "with step()")
         n = self.num_envs
         b = self._host_buffers(slot)
         a = action_host if isinstance(action_host, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(action_host, np.float32))
@@ -934,11 +941,15 @@ class BatchedManipulationEnv:
             io.action, io.action_layout = self._action_dev.data_ptr(), 1
             io.dyn_noise = io.obs_noise = io.noisy_obs = None
             io.sigma_dyn = io.sigma_obs = 0.0
-            _lib.check(self._lib.dexsim_step_host(
-                C.byref(self._state), C.byref(self._params), self._ptr(self._groups_dev), self._ptr(self._goe),
-                C.byref(io), a.data_ptr(), b["obs"].data_ptr(), b["reward"].data_ptr(), b["term"].data_ptr(),
-                b["trunc"].data_ptr(), b["nc"].data_ptr(), b["cmask"].data_ptr(),
-                int(chunks) if chunks is not None else max(1, min(8, n // 8192)), flags, self._stream()), "dexsim_step_host")
+            args = (C.byref(self._state), C.byref(self._params), self._ptr(self._groups_dev), self._ptr(self._goe),
+                    C.byref(io), a.data_ptr(), b["obs"].data_ptr(), b["reward"].data_ptr(), b["term"].data_ptr(),
+                    b["trunc"].data_ptr(), b["nc"].data_ptr(), b["cmask"].data_ptr())
+            tail = (int(chunks) if chunks is not None else max(1, min(8, n // 8192)), flags, self._stream())
+            if self.final_observation:
+                _lib.check(self._lib.dexsim_step_host_final(*args, b["fin"].data_ptr(), b["final"].data_ptr(), *tail),
+                           "dexsim_step_host_final")
+            else:
+                _lib.check(self._lib.dexsim_step_host(*args, *tail), "dexsim_step_host")
         # this slot's observation is current now; any other entry point that touches the state resets the marker
         self._h_primed_slot = slot if sync else None
         if not sync:

@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define DEXSIM_ABI_VERSION 4
+#define DEXSIM_ABI_VERSION 5
 #define DEXSIM_NJ 15      /* joints            envs/manipulation_env.py:52 */
 #define DEXSIM_NF 5       /* fingers           envs/manipulation_env.py:50 */
 #define DEXSIM_OBS 45     /* observation width envs/manipulation_env.py:96-106 */
@@ -403,7 +403,33 @@ int dexsim_step_host(const DexsimState* st, const DexsimParams* p, const DexsimG
                      uint8_t* h_contact_mask /* host [ld]: filled whenever given; required with DEXSIM_HOST_PACKED_CONTACTS */,
                      int32_t chunks, int32_t flags, void* stream);
 
-/* Diagnostic: how many dexsim_step_host calls of this process were served by the DEXSIM_HOST_ZERO_COPY launch. */
+/* dexsim_step_host with auto-reset that also returns the terminal observation of every episode it ends (what a trainer
+ * bootstraps a value estimate from at truncation; Gymnasium's info["final_observation"]).  Same arguments as
+ * dexsim_step_host plus `h_finished` and `h_final_obs`.  Per chunk, the step runs without the reset and a
+ * finish-and-reset pass follows it (as in dexsim_step_final); everything the chunk moves to the host is enqueued after the
+ * pass.  The pass writes each finished env's record straight into h_final_obs (about 180 bytes per finished env cross
+ * PCIe, nothing per unfinished one).
+ *   - Every output, state array and counter equals what dexsim_step_host with auto-reset produces for the same inputs,
+ *     flags and chunk count; io->ret_sums is a float64 atomic sum and equal only up to summation order.
+ *   - h_finished[i] == 1 where env i's episode ended in this step and the env was reset.  For every such env, row i of
+ *     h_final_obs is bit for bit column i of final_obs from dexsim_step_final: the observation a step without auto-reset
+ *     returns, all 45 entries (the five contact floats too, under DEXSIM_HOST_PACKED_CONTACTS).  Other rows are not
+ *     written.
+ *   - DEXSIM_HOST_ZERO_COPY is served as by dexsim_step_host (counted by dexsim_host_zero_copy_steps); h_finished is one
+ *     of the buffers that must be mapped for it.  In this mode io->terminated / truncated / num_contacts on the device
+ *     are written as well.
+ *   - Returns, before anything touches the device: DEXSIM_E_PARAM when p->auto_reset == 0, when noise is requested (as
+ *     dexsim_step_host) or when h_final_obs is not mapped page-locked memory; DEXSIM_E_NULL when h_finished, h_final_obs
+ *     or io->finished is NULL. */
+int dexsim_step_host_final(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                           const uint16_t* group_of_env, const DexsimStepIO* io, const float* h_action,
+                           float* h_obs, float* h_reward, uint8_t* h_terminated, uint8_t* h_truncated,
+                           uint8_t* h_num_contacts, uint8_t* h_contact_mask,
+                           uint8_t* h_finished /* host [ld]: 1 where the episode ended this step and the env was reset */,
+                           float* h_final_obs /* mapped page-locked host [n, 45], batch-first */,
+                           int32_t chunks, int32_t flags, void* stream);
+
+/* Diagnostic: how many dexsim_step_host / dexsim_step_host_final calls of this process were served by the DEXSIM_HOST_ZERO_COPY launch. */
 int64_t dexsim_host_zero_copy_steps(void);
 
 /* HOST function: observation rows 40-44 (the five 0/1 contact floats, envs/manipulation_env.py:262) of envs [0, n) of a
