@@ -102,7 +102,7 @@ EXPORTS = (
     "dexsim_device_info", "dexsim_set_step_impl", "dexsim_set_step_tile", "dexsim_set_rollout_impl", "dexsim_reset_predrawn",
     "dexsim_reset_philox", "dexsim_step", "dexsim_rollout", "dexsim_fill_policy_actions",
     "dexsim_fill_normal", "dexsim_classify_summary", "dexsim_step_host", "dexsim_pack_env", "dexsim_pack_env_tagged", "dexsim_step_single",
-    "dexsim_step_final", "dexsim_step_host_final",
+    "dexsim_step_final", "dexsim_step_host_final", "dexsim_step_next_reset",
     "dexsim_expand_contact_rows",
     "dexsim_host_zero_copy_steps",
 )
@@ -142,6 +142,7 @@ def lib():
     L.dexsim_reset_philox.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, vp, i32, vp]
     L.dexsim_step.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, C.POINTER(DexsimStepIO), vp]
     L.dexsim_step_final.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, C.POINTER(DexsimStepIO), vp, vp]
+    L.dexsim_step_next_reset.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, C.POINTER(DexsimStepIO), vp]
     L.dexsim_rollout.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, i32, i32,
                                  C.POINTER(DexsimRolloutIO), vp]
     L.dexsim_fill_policy_actions.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, vp, vp]

@@ -195,6 +195,30 @@ __device__ __forceinline__ void finish_and_reset(EnvRegs& e, const DexsimParams&
     es.w0 = 0u; es.w1 = 0u;
 }
 
+// ---- next-step auto-reset (dexsim_step_next_reset) -------------------------------------------------------------------
+// An env has a pending reset when its stored state is what a step that ended its episode left behind: the step kernels'
+// `done` evaluated on that state (terminated: the contact count of the stored mask; truncated: the step before the last
+// one was at max_episode_steps; the loop bound).  Every reset leaves sc == 0, so a freshly reset env is never pending.
+// Derived from the state alone, it survives state_dict() / load_state_dict() and needs no array of its own.
+__device__ __forceinline__ bool pending_reset(const EnvRegs& e, const DexsimParams& p) {
+    return e.sc > 0 && (__popc(e.cmask) >= p.success_threshold || e.sc > p.max_episode_steps ||
+                        (p.loop_max_steps > 0 && e.sc >= p.loop_max_steps));
+}
+
+// The reset of a pending env, in place of its step: what finish_and_reset does after the episode end (counted by the step
+// that ended it), and the outputs of a reset step -- reward 0, both flags 0, the contact count of the reset state.
+__device__ __forceinline__ void next_step_reset(EnvRegs& e, const DexsimParams& p, const DexsimGroup& grp, uint32_t gid,
+                                                uint32_t& episode, const DexsimState& st, int64_t i, StepResult& r) {
+    double ep_return = 0.0, size, mass, friction;
+    EpStats es{0u, 0u};
+    finish_and_reset(e, p, grp, gid, episode, ep_return, es, false, 0, nullptr, nullptr, size, mass, friction);
+    st.episode[i] = episode;
+    st.size[i] = size; st.mass[i] = mass; st.friction[i] = friction;
+    r.total = r.distance = r.contact = r.closure = r.stability = 0.0;
+    r.n_c = __popc(e.cmask);
+    r.terminated = r.truncated = false;
+}
+
 // Observation entry `row` (envs/manipulation_env.py:254-264) of an env held in registers; `row` is a compile-time
 // constant wherever this is called from an unrolled loop.
 __device__ __forceinline__ float obs_entry(const EnvRegs& e, const int row) {
@@ -260,11 +284,13 @@ __global__ void pack_env_kernel(const DexsimState st, const DexsimStepIO io, con
 // memory with coalesced float4 reads (15 is odd, so the per-thread reads are bank-conflict free).
 // EXTRAS: noise, reward components, episode tracking, auto-reset -- the plain path carries none
 // of their registers or branches.
-template <bool DENSE, bool AOS, bool EXTRAS>
+// NEXT: next-step auto-reset (dexsim_step_next_reset, see pending_reset); only with EXTRAS.
+template <bool DENSE, bool AOS, bool EXTRAS, bool NEXT>
 __global__ void __launch_bounds__(STEP_THREADS, STEP_MIN_BLOCKS)
 step_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
             const uint16_t* __restrict__ group_of_env, const DexsimStepIO io,
             double* __restrict__ pack_out = nullptr, const double pack_tag = 0.0) {
+    static_assert(!NEXT || EXTRAS, "next-step auto-reset needs the auto-reset path");
     __shared__ __align__(16) float sh_act[AOS ? STEP_THREADS * NJ : 4];
     // Finished episodes are counted per CTA in shared memory and flushed with one global atomic per
     // non-zero counter at the end: thousands of episodes end per step and would otherwise serialise
@@ -311,6 +337,8 @@ step_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __res
 #pragma unroll
         for (int k = 0; k < 3; ++k) { h.op_old[k] = e.op[k]; h.ov_old[k] = e.ov[k]; }
         h.cmask_old = e.cmask;
+        bool pending = false;
+        if constexpr (NEXT) pending = pending_reset(e, p);
 
         // in-kernel Philox noise (DexsimStepIO.sigma_*): needs the env's identity before the step
         const bool fused_dyn = EXTRAS && !io.dyn_noise && io.sigma_dyn != 0.0f;
@@ -326,7 +354,7 @@ step_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __res
 #pragma unroll
             for (int j = 0; j < NJ; ++j)
                 a[j] = clip_f32(__fadd_rn(a[j], __ldg(io.dyn_noise + j * ld + i)), -1.0f, 1.0f);
-        } else if (fused_dyn) {
+        } else if (fused_dyn && !pending) {
             const float sigma = io.sigma_dyn > 0.0f ? io.sigma_dyn : groups[g].sigma_dyn;
             if (sigma > 0.0f) {
                 float nz[NJ];
@@ -337,7 +365,17 @@ step_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __res
         }
 
         StepResult r;
-        env_step<DENSE>(e, a, p, r);
+        if constexpr (NEXT) {
+            if (pending) {          // the reset the previous step left for this env, instead of a step: the action is ignored
+                g = group_index(group_of_env, i, gid, p.num_groups);
+                episode = st.episode[i];
+                next_step_reset(e, p, groups[g], (uint32_t)gid, episode, st, i, r);
+            } else {
+                env_step<DENSE>(e, a, p, r);
+            }
+        } else {
+            env_step<DENSE>(e, a, p, r);
+        }
 
         io.reward[i] = (float)r.total;
         io.terminated[i] = r.terminated ? 1 : 0;
@@ -359,11 +397,12 @@ step_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __res
         const bool tracking = st.ep_return != nullptr && st.ep_stats != nullptr;
         double ep_return = 0.0;
         EpStats es{0u, 0u};
-        if (tracking) {
+        if (tracking && !pending) {                                    // a pending env's episode starts now: both stay 0
             ep_return = __dadd_rn(st.ep_return[i], r.total);           // evaluator.py:144
             es.w0 = st.ep_stats[i]; es.w1 = st.ep_stats[ld + i];
             epstats_push(es, e.sc - 1, r.n_c);                         // evaluator.py:148-150
         }
+        // (never true for a pending env: its reset left step count 0 and both flags 0)
         const bool done = r.terminated || r.truncated || (p.loop_max_steps > 0 && e.sc >= p.loop_max_steps);
         bool finished = false;
         if (p.auto_reset && done) {
@@ -377,10 +416,18 @@ step_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __res
                 cnt = (staged ? sh_cnt : reinterpret_cast<unsigned long long*>(io.counters)) + (int64_t)g * DEXSIM_NCOUNTERS;
                 if (io.ret_sums) rs = (staged ? sh_rs : io.ret_sums) + 2 * g;
             }
-            finish_and_reset(e, p, groups[g], (uint32_t)gid, episode, ep_return, es, r.terminated, r.n_c,
-                             cnt, rs, size, mass, friction, nullptr, /*classify=*/tracking);
-            st.episode[i] = episode;
-            st.size[i] = size; st.mass[i] = mass; st.friction[i] = friction;
+            if constexpr (NEXT) {   // counted and flagged now, reset by the env's next step
+                finish_episode(e, p, (uint32_t)gid, episode, ep_return, es, r.terminated, r.n_c, cnt, rs, nullptr,
+                               /*classify=*/tracking);
+                store_env_step(st, i, e, h, io.host_static_rows);
+            } else {
+                finish_and_reset(e, p, groups[g], (uint32_t)gid, episode, ep_return, es, r.terminated, r.n_c,
+                                 cnt, rs, size, mass, friction, nullptr, /*classify=*/tracking);
+                st.episode[i] = episode;
+                st.size[i] = size; st.mass[i] = mass; st.friction[i] = friction;
+                store_env_full(st, i, e, io.host_static_rows);
+            }
+        } else if (pending) {
             store_env_full(st, i, e, io.host_static_rows);
         } else {
             store_env_step(st, i, e, h, io.host_static_rows);
@@ -894,7 +941,7 @@ static int query_device(DeviceInfo& d) {
     if (err != cudaSuccess) return -(int)err;
     err = cudaDeviceGetAttribute(&d.sm_count, cudaDevAttrMultiProcessorCount, dev);
     if (err != cudaSuccess) return -(int)err;
-    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&d.step_ctas, step_kernel<true, false, false>, STEP_THREADS, 0);
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&d.step_ctas, step_kernel<true, false, false, false>, STEP_THREADS, 0);
     if (err != cudaSuccess) return -(int)err;
     err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&d.rollout_ctas, rollout_kernel<true, false>, ROLLOUT_THREADS, 0);
     if (err != cudaSuccess) return -(int)err;
@@ -956,18 +1003,19 @@ static int grid_for(int64_t n, int threads, int ctas_per_sm, int sm_count) {
 static inline int cuda_rc(cudaError_t e) { return e == cudaSuccess ? 0 : -(int)e; }
 
 template <bool DENSE, bool AOS>
-static void launch_step_variant(bool extras, int grid, cudaStream_t s, const DexsimState& st, const DexsimParams& p,
+static void launch_step_variant(bool extras, bool next, int grid, cudaStream_t s, const DexsimState& st, const DexsimParams& p,
                                 const DexsimGroup* groups, const uint16_t* goe, const DexsimStepIO& io,
                                 double* pack_out, double pack_tag) {
-    if (extras) step_kernel<DENSE, AOS, true><<<grid, STEP_THREADS, 0, s>>>(st, p, groups, goe, io, pack_out, pack_tag);
-    else        step_kernel<DENSE, AOS, false><<<grid, STEP_THREADS, 0, s>>>(st, p, groups, goe, io);
+    if (next)        step_kernel<DENSE, AOS, true, true><<<grid, STEP_THREADS, 0, s>>>(st, p, groups, goe, io, pack_out, pack_tag);
+    else if (extras) step_kernel<DENSE, AOS, true, false><<<grid, STEP_THREADS, 0, s>>>(st, p, groups, goe, io, pack_out, pack_tag);
+    else             step_kernel<DENSE, AOS, false, false><<<grid, STEP_THREADS, 0, s>>>(st, p, groups, goe, io);
 }
 
-template <bool DENSE, bool AOS, int TRACK, bool EXTRA, int STAGES, int TILE_>
+template <bool DENSE, bool AOS, int TRACK, bool EXTRA, int STAGES, int TILE_, bool NEXT>
 static int launch_tma_variant(int sm_count, cudaStream_t s, const DexsimState& st, const DexsimParams& p,
                               const DexsimGroup* groups, const uint16_t* goe, const DexsimStepIO& io,
                               const StepMaps& maps, int num_tiles) {
-    auto kern = step_tma_kernel<DENSE, AOS, TRACK, EXTRA, STAGES, TILE_>;
+    auto kern = step_tma_kernel<DENSE, AOS, TRACK, EXTRA, STAGES, TILE_, NEXT>;
     constexpr int TMA_THREADS = TILE_ + 32;            // one compute thread per env of a tile + the producer warp
     const size_t smem = (size_t)STAGES * StageLayout<TILE_>::stage_bytes(TRACK) + 2 * STAGES * (sizeof(uint64_t) + sizeof(int)) +
                         (TRACK ? TMA_GROUPS_MAX * (DEXSIM_NCOUNTERS * sizeof(unsigned long long) + 2 * sizeof(double)) : 0);
@@ -1064,7 +1112,7 @@ static bool use_wide_tile(int64_t n, int track, int sm_count) {
 }
 
 static int launch_step_tma(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups, const uint16_t* goe,
-                           const DexsimStepIO* io, cudaStream_t s, int track, bool extra, int sm_count) {
+                           const DexsimStepIO* io, cudaStream_t s, int track, bool extra, bool next, int sm_count) {
     // Tensor maps are pure functions of (base pointers, n, ld): a stepping loop re-encodes nothing.  One cached set
     // per host thread; the SoA action map is keyed by the action pointer too (AoS actions use 1-D bulk copies).
     struct MapCache { const void* obs; const void* op64; const void* act; const void* host; int64_t n, ld; int tile; bool valid; StepMaps maps; };
@@ -1094,7 +1142,7 @@ static int launch_step_tma(const DexsimState* st, const DexsimParams* p, const D
     }
     const StepMaps& maps = cache.maps;
     const int num_tiles = (int)((st->n + tile - 1) / tile);
-    // runtime (dense, aos, track, extra) -> template arguments: each call hands its value on as a std::integral_constant
+    // runtime (dense, aos, track, extra, next) -> template arguments: each call hands its value on as a std::integral_constant
     const auto as_bool = [](bool b, auto&& f) { return b ? f(std::true_type{}) : f(std::false_type{}); };
     const auto as_track = [](int t, auto&& f) {
         using std::integral_constant;
@@ -1103,32 +1151,39 @@ static int launch_step_tma(const DexsimState* st, const DexsimParams* p, const D
     return as_bool(p->reward_type == 1, [&](auto dense) {
         return as_bool(aos, [&](auto aos_) {
             return as_track(track, [&](auto track_) {
-                return as_bool(extra, [&](auto extra_) -> int {
-                    constexpr bool DENSE = decltype(dense)::value, AOS = decltype(aos_)::value, EXTRA = decltype(extra_)::value;
-                    constexpr int TRACK = decltype(track_)::value;
-                    // The instantiations: noise / reward components only with the reference's [n,15] action layout (SoA
-                    // callers take the register kernel), and the wide tile only without full tracking (its stages have no
-                    // room for the per-env return / history arrays).
-                    if constexpr (EXTRA && !AOS) {
-                        return 1;
-                    } else {
-                        if constexpr (TRACK != 1) {
-                            if (wide)
-                                return launch_tma_variant<DENSE, AOS, TRACK, EXTRA, 2, TILE_WIDE>(sm_count, s, *st, *p, groups,
-                                                                                                  goe, *io, maps, num_tiles);
+                return as_bool(extra, [&](auto extra_) {
+                    return as_bool(next, [&](auto next_) -> int {
+                        constexpr bool DENSE = decltype(dense)::value, AOS = decltype(aos_)::value, EXTRA = decltype(extra_)::value;
+                        constexpr int TRACK = decltype(track_)::value;
+                        constexpr bool NEXT = decltype(next_)::value;
+                        // The instantiations: noise / reward components only with the reference's [n,15] action layout
+                        // (SoA callers take the register kernel), the wide tile only without full tracking (its stages
+                        // have no room for the per-env return / history arrays), and next-step auto-reset only with the
+                        // episode bookkeeping (an auto-reset call always has TRACK 1 or 2).
+                        if constexpr ((EXTRA && !AOS) || (NEXT && TRACK == 0)) {
+                            return 1;
+                        } else {
+                            if constexpr (TRACK != 1) {
+                                if (wide)
+                                    return launch_tma_variant<DENSE, AOS, TRACK, EXTRA, 2, TILE_WIDE, NEXT>(sm_count, s, *st, *p,
+                                                                                                            groups, goe, *io, maps,
+                                                                                                            num_tiles);
+                            }
+                            return launch_tma_variant<DENSE, AOS, TRACK, EXTRA, DEXSIM_TMA_STAGES, TILE, NEXT>(sm_count, s, *st, *p,
+                                                                                                               groups, goe, *io,
+                                                                                                               maps, num_tiles);
                         }
-                        return launch_tma_variant<DENSE, AOS, TRACK, EXTRA, DEXSIM_TMA_STAGES, TILE>(sm_count, s, *st, *p, groups,
-                                                                                                     goe, *io, maps, num_tiles);
-                    }
+                    });
                 });
             });
         });
     });
 }
 
+// next: next-step auto-reset (dexsim_step_next_reset; the caller has checked its arguments).
 static int launch_step(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
                        const uint16_t* goe, const DexsimStepIO* io, cudaStream_t s,
-                       double* pack_out = nullptr, double pack_tag = 0.0) {
+                       double* pack_out = nullptr, double pack_tag = 0.0, bool next = false) {
     int rc = check_state(st);
     if (rc) return rc;
     if (!io || !io->action || !io->reward || !io->terminated || !io->truncated || !io->num_contacts) return DEXSIM_E_NULL;
@@ -1149,17 +1204,17 @@ static int launch_step(const DexsimState* st, const DexsimParams* p, const Dexsi
     const int track = step_track(*st, *p, *io);
     const bool extra_io = step_extra_io(*io);
     if (pipeline_eligible(*st, *io, track, extra_io, pack_out != nullptr)) {
-        rc = launch_step_tma(st, p, groups, goe, io, s, track, extra_io, di.sm_count);
+        rc = launch_step_tma(st, p, groups, goe, io, s, track, extra_io, next, di.sm_count);
         if (rc <= 0) return rc;                      // launched (0) or CUDA error (< 0); 1 = a tensor map was rejected
     }
     if (g_step_impl == 2) return DEXSIM_E_PARAM;     // TMA pipeline was demanded but is not eligible
     if (io->flags & DEXSIM_STEP_HOST_ALL_ROWS) return DEXSIM_E_PARAM;   // only the pipelined kernel mirrors every row
     const int grid = grid_for(st->n, STEP_THREADS, di.step_ctas, di.sm_count);
     const bool dense = p->reward_type == 1, aos = io->action_layout == 1;
-    if (dense) { if (aos) launch_step_variant<true, true>(extras, grid, s, *st, *p, groups, goe, *io, pack_out, pack_tag);
-                 else     launch_step_variant<true, false>(extras, grid, s, *st, *p, groups, goe, *io, pack_out, pack_tag); }
-    else       { if (aos) launch_step_variant<false, true>(extras, grid, s, *st, *p, groups, goe, *io, pack_out, pack_tag);
-                 else     launch_step_variant<false, false>(extras, grid, s, *st, *p, groups, goe, *io, pack_out, pack_tag); }
+    if (dense) { if (aos) launch_step_variant<true, true>(extras, next, grid, s, *st, *p, groups, goe, *io, pack_out, pack_tag);
+                 else     launch_step_variant<true, false>(extras, next, grid, s, *st, *p, groups, goe, *io, pack_out, pack_tag); }
+    else       { if (aos) launch_step_variant<false, true>(extras, next, grid, s, *st, *p, groups, goe, *io, pack_out, pack_tag);
+                 else     launch_step_variant<false, false>(extras, next, grid, s, *st, *p, groups, goe, *io, pack_out, pack_tag); }
     return cuda_rc(cudaGetLastError());
 }
 
@@ -1326,6 +1381,14 @@ int dexsim_step_final(const DexsimState* st, const DexsimParams* p, const Dexsim
     rc = device_info_cached(di);
     if (rc) return rc;
     return launch_finish_reset<false>(*st, *p, groups, group_of_env, *io, final_obs, FinishHost{}, s, di.sm_count);
+}
+
+int dexsim_step_next_reset(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                           const uint16_t* group_of_env, const DexsimStepIO* io, void* stream) {
+    if (!p || !io) return DEXSIM_E_NULL;
+    if (!p->auto_reset || io->host_static_rows || (io->flags & DEXSIM_STEP_HOST_ALL_ROWS)) return DEXSIM_E_PARAM;
+    if (!io->finished) return DEXSIM_E_NULL;
+    return launch_step(st, p, groups, group_of_env, io, (cudaStream_t)stream, nullptr, 0.0, /*next=*/true);
 }
 
 int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,

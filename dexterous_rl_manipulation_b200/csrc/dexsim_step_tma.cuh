@@ -141,7 +141,10 @@ __device__ __forceinline__ uint32_t tile_cols(int64_t n, int64_t base) {
 // tile is its block index, every further one comes from a global counter.  SMs do not progress at the same rate (ncu,
 // round 2: 125k .. 152k active cycles per SM under the static round-robin, the launch lasting as long as the slowest),
 // and tiles with episode resets take longer than others; with the counter every SM works until the batch is done.
-template <bool DENSE, bool AOS, int TRACK, bool EXTRA, int STAGES, int TILE_>
+// NEXT: next-step auto-reset (dexsim_step_next_reset).  An env whose stored state is what a step that ended its episode
+// left behind (pending_reset) is reset on its owning lane instead of stepped, and shares the tail below with a stepped
+// env; an episode that ends is counted and flagged `finished` but not reset.
+template <bool DENSE, bool AOS, int TRACK, bool EXTRA, int STAGES, int TILE_, bool NEXT>
 __global__ void __launch_bounds__(TILE_ + 32, (STAGES == 2) ? (TILE_ <= 96 ? 4 : (TILE_ >= 192 ? 2 : 3)) : (STAGES == 1 ? 4 : 2))
 step_tma_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
                 const uint16_t* __restrict__ group_of_env, const DexsimStepIO io,
@@ -149,6 +152,7 @@ step_tma_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* _
     // this instantiation's tile width (shadows the namespace-level narrow width) and stage layout
     constexpr int TILE = TILE_;
     static_assert(TRACK != 1 || TILE_ <= 128, "the full-tracking arrays only fit the narrow tile's stages");
+    static_assert(!NEXT || TRACK != 0, "next-step auto-reset needs the episode bookkeeping of TRACK 1 or 2");
     using SL = StageLayout<TILE_>;
     constexpr int OFF_JPJV = SL::OFF_JPJV, OFF_OV = SL::OFF_OV, OFF_OP64 = SL::OFF_OP64, OFF_THR = SL::OFF_THR, OFF_ACT = SL::OFF_ACT,
                   OFF_DAMP = SL::OFF_DAMP, OFF_SC = SL::OFF_SC, OFF_REWARD = SL::OFF_REWARD, OFF_CMASK = SL::OFF_CMASK,
@@ -329,6 +333,8 @@ step_tma_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* _
                 e.damp = reinterpret_cast<const float*>(sp + OFF_DAMP)[col];
                 e.sc = reinterpret_cast<const int*>(sp + OFF_SC)[col];
                 e.cmask = reinterpret_cast<const uint8_t*>(sp + OFF_CMASK)[col];
+                bool pending = false;
+                if constexpr (NEXT) pending = pending_reset(e, p);
                 float a[NJ];
                 const float* s_act = reinterpret_cast<const float*>(sp + OFF_ACT);
                 if (AOS) {
@@ -357,7 +363,7 @@ step_tma_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* _
 #pragma unroll
                         for (int j = 0; j < NJ; ++j)
                             a[j] = clip_f32(__fadd_rn(a[j], __ldg(io.dyn_noise + j * ld + i)), -1.0f, 1.0f);
-                    } else if (fused_dyn) {
+                    } else if (fused_dyn && !pending) {
                         const float sigma = io.sigma_dyn > 0.0f ? io.sigma_dyn : groups[g].sigma_dyn;
                         if (sigma > 0.0f) {
                             float nz[NJ];
@@ -373,7 +379,19 @@ step_tma_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* _
                 const unsigned cmask_old = e.cmask;
 
                 StepResult r;
-                env_step<DENSE>(e, a, p, r);
+                if constexpr (NEXT) {
+                    if (pending) {
+                        // the reset the previous step left for this env, instead of a step: the action is ignored
+                        g = group_of_env ? (int)group_of_env[i] : (int)((uint32_t)gid % (uint32_t)p.num_groups);
+                        episode = reinterpret_cast<const uint32_t*>(sp + OFF_EPISODE)[col];     // load_episode is on with auto-reset
+                        next_step_reset(e, p, groups[g], (uint32_t)gid, episode, st, i, r);
+                        st.thr[i] = e.thr; st.damp[i] = e.damp;
+                    } else {
+                        env_step<DENSE>(e, a, p, r);
+                    }
+                } else {
+                    env_step<DENSE>(e, a, p, r);
+                }
 
                 reinterpret_cast<float*>(sp + OFF_REWARD)[col] = (float)r.total;
                 (sp + OFF_TERM)[col] = r.terminated ? 1 : 0;
@@ -392,12 +410,13 @@ step_tma_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* _
                 if (TRACK) {
                     double ep_return = 0.0;
                     EpStats es{0u, 0u};
-                    if (TRACK == 1) {
+                    if (TRACK == 1 && !pending) {       // a pending env's episode starts now: return and summary stay 0
                         ep_return = __dadd_rn(reinterpret_cast<double*>(sp + OFF_EPRET)[col], r.total);
                         es.w0 = reinterpret_cast<uint32_t*>(sp + OFF_EPST0)[col];
                         es.w1 = reinterpret_cast<uint32_t*>(sp + OFF_EPST1)[col];
                         epstats_push(es, e.sc - 1, r.n_c);
                     }
+                    // (never true for a pending env: its reset left step count 0 and both flags 0)
                     const bool done = r.terminated || r.truncated || (p.loop_max_steps > 0 && e.sc >= p.loop_max_steps);
                     if (p.auto_reset && done) {
                         // episode end on the owning lane (counters, labels)
@@ -409,6 +428,12 @@ step_tma_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* _
                             cnt = (staged_cnt ? sh_cnt : reinterpret_cast<unsigned long long*>(io.counters)) + (int64_t)g * DEXSIM_NCOUNTERS;
                             if (io.ret_sums) rs = (staged_cnt ? sh_rs : io.ret_sums) + 2 * g;
                         }
+                        if constexpr (NEXT) {
+                            // counted and flagged now, reset by the env's next step
+                            finish_episode(e, p, (uint32_t)gid, episode, ep_return, es, r.terminated, r.n_c, cnt, rs, nullptr,
+                                           /*classify=*/TRACK == 1);
+                            lane_reset = true;
+                        } else
                         // the owning lane draws all of its env's Philox blocks (reset_draws + env_reset, dexsim_core.cuh)
                         {
                             double size, mass, friction;

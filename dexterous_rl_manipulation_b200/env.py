@@ -121,6 +121,7 @@ class BatchedManipulationEnv:
         observation_noise_std: float = 0.0,
         dynamics_noise_std: float = 0.0,
         final_observation: bool = False,
+        autoreset_mode: str = "same_step",
     ):
         if num_fingers != 5 or joints_per_finger != 3:
             raise _lib.DexsimError(-1006, "BatchedManipulationEnv")
@@ -133,6 +134,22 @@ class BatchedManipulationEnv:
         if self.final_observation and int(num_envs) == 1:
             raise NotImplementedError("final_observation is for batched envs; num_envs == 1 mirrors the reference, "
                                       "which has no auto-reset")
+        # "same_step": a step that ends an episode resets the env in the same launch and returns the new episode's first
+        # observation.  "next_step" (Gymnasium's AutoresetMode.NEXT_STEP, dexsim_step_next_reset): that step returns the
+        # terminal observation and info["finished"]; the env's next step ignores its action and resets it instead,
+        # returning the first observation, reward 0 and both flags False.
+        if autoreset_mode not in ("same_step", "next_step"):
+            raise ValueError("autoreset_mode must be 'same_step' or 'next_step'")
+        self.autoreset_mode = autoreset_mode
+        self._next_step = autoreset_mode == "next_step"
+        if self._next_step and not auto_reset:
+            raise ValueError("autoreset_mode='next_step' needs auto_reset=True")
+        if self._next_step and self.final_observation:
+            raise ValueError("autoreset_mode='next_step' already returns the terminal observation from step(); "
+                             "final_observation=True is for the same-step reset")
+        if self._next_step and int(num_envs) == 1:
+            raise NotImplementedError("autoreset_mode='next_step' is for batched envs; num_envs == 1 mirrors the "
+                                      "reference, which has no auto-reset")
         self._lib = _lib.lib()
         self.device = torch.device(device)
         if self.device.type != "cuda":
@@ -244,6 +261,9 @@ class BatchedManipulationEnv:
         self._state_ref, self._params_ref, self._io_ref = C.byref(self._state), C.byref(self._params), C.byref(self._io)
         self._goe_ptr = self._ptr(self._goe)
         self._final_obs_ptr = self._ptr(self._final_obs)
+        # the one-launch step entry of this env (dexsim_step_final is called where _final_obs is set)
+        self._step_entry = self._lib.dexsim_step_next_reset if self._next_step else self._lib.dexsim_step
+        self._step_entry_name = "dexsim_step_next_reset" if self._next_step else "dexsim_step"
         self._step_out = None
         if not self.single:
             self._step_out = (self._obs_view, self._reward[:n], self._terminated[:n].view(torch.bool),
@@ -596,13 +616,13 @@ class BatchedManipulationEnv:
                 io.sigma_dyn = io.sigma_obs = 0.0
                 self._io_has_noise = False
             if self._final_obs is None:
-                rc = self._lib.dexsim_step(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
-                                           self._io_ref, _raw_stream(self.device.index))
+                rc = self._step_entry(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
+                                      self._io_ref, _raw_stream(self.device.index))
             else:
                 rc = self._lib.dexsim_step_final(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
                                                  self._io_ref, self._final_obs_ptr, _raw_stream(self.device.index))
             if rc:
-                raise _lib.DexsimError(rc, "dexsim_step_final" if self._final_obs is not None else "dexsim_step")
+                raise _lib.DexsimError(rc, "dexsim_step_final" if self._final_obs is not None else self._step_entry_name)
             return self._step_out
         if (self.single and dyn_noise is None and obs_noise is None and not self._noisy_env
                 and not (isinstance(action, torch.Tensor) and action.is_cuda)
@@ -750,10 +770,11 @@ class BatchedManipulationEnv:
         return self._step_out
 
     def _launch_step(self):
-        """dexsim_step, or dexsim_step_final when the env returns final observations."""
+        """dexsim_step (dexsim_step_next_reset in next-step mode), or dexsim_step_final when the env returns final
+        observations."""
         if self._final_obs is None:
-            _lib.check(self._lib.dexsim_step(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
-                                             self._io_ref, self._stream()), "dexsim_step")
+            _lib.check(self._step_entry(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
+                                        self._io_ref, self._stream()), self._step_entry_name)
         else:
             _lib.check(self._lib.dexsim_step_final(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
                                                    self._io_ref, self._final_obs_ptr, self._stream()), "dexsim_step_final")
@@ -909,7 +930,11 @@ class BatchedManipulationEnv:
         whose episode ended in this step and was reset, and ``info["final_observation"]`` (float32 [num_envs, 45]) holds,
         where ``info["finished"]``, the observation that ended it -- all 45 entries, also with ``packed_contacts``.  Its
         other rows keep stale values.  Both are pinned buffers of the ``slot`` like the other outputs; the GPU writes the
-        rows of finished envs only, straight into the buffer."""
+        rows of finished envs only, straight into the buffer.
+
+        Not available in ``autoreset_mode="next_step"`` (its per-env outputs carry no ``finished`` vector)."""
+        if self._next_step:
+            raise NotImplementedError("step_host() does not support autoreset_mode='next_step'; use step()")
         if not self._did_reset:
             raise RuntimeError("call reset() before step_host()")
         n = self.num_envs
@@ -1021,7 +1046,12 @@ class BatchedManipulationEnv:
         (caller loops of training/episode_utils.py:42-53 / evaluation/evaluator.py:135-158).
         Returns (counters [G, 18] int64, ret_sums [G, 2] float64) device tensors (accumulated).
         ``one_episode=True``: every env stops at the end of its first episode and is left un-reset
-        (run_episode / evaluate_episode semantics); otherwise finished episodes auto-reset."""
+        (run_episode / evaluate_episode semantics); otherwise finished episodes auto-reset.
+        Not available in ``autoreset_mode="next_step"``: the fused rollout resets in the same step, and an episode a
+        step() left pending would be counted twice."""
+        if self._next_step:
+            raise NotImplementedError("rollout() resets finished episodes in the same step; it does not support "
+                                      "autoreset_mode='next_step'")
         if not self._did_reset:
             raise RuntimeError("call reset() before rollout()")
         self._h_primed_slot = None

@@ -258,6 +258,29 @@ int dexsim_step_final(const DexsimState* st, const DexsimParams* p, const Dexsim
                       const uint16_t* group_of_env, const DexsimStepIO* io,
                       float* final_obs /* device [45, ld] */, void* stream);
 
+/* dexsim_step with NEXT-STEP auto-reset (Gymnasium's AutoresetMode.NEXT_STEP): the step that ends an episode returns that
+ * episode's terminal observation and does not reset; the env's next call resets it instead of stepping it.  Same
+ * arguments as dexsim_step, one launch, no state beyond DexsimState.
+ *   - An env has a pending reset when its stored state is what a step that ended an episode left behind:
+ *       step_count > 0 && (popcount(cmask) >= success_threshold || step_count > max_episode_steps
+ *                          || (loop_max_steps > 0 && step_count >= loop_max_steps)).
+ *     Every reset leaves step_count == 0, so a freshly reset env is never pending.
+ *   - A pending env ignores its action (no dynamics noise is drawn for it) and is reset as the same-step auto-reset
+ *     resets a finished env: episode += 1, Philox draws of its group, respawn per p->respawn, ep_return / ep_stats
+ *     zeroed; episode, size, mass, friction, thr and damp are written.  Its outputs: reward 0 (reward components and
+ *     reward64 0 where present), terminated = truncated = finished = 0, num_contacts = the contact count of the reset
+ *     state, and the observation of the reset state (noisy_obs keyed by the new episode and step 0).
+ *   - Every other env is stepped exactly as with auto_reset = 0.  If its episode ends, finished[i] = 1 and the episode is
+ *     counted in io->counters / io->ret_sums (and classified with full tracking) as the same-step auto-reset counts it;
+ *     the env is not reset.  finished is the only output that shows an episode ended at the loop bound.
+ *   - A caller must not change max_episode_steps, loop_max_steps or success_threshold between the call that ends an
+ *     episode and the one that resets it: the pending test reads them.
+ *   - Returns, before anything touches the device: DEXSIM_E_PARAM when p->auto_reset == 0, io->host_static_rows is set
+ *     or io->flags has DEXSIM_STEP_HOST_ALL_ROWS; DEXSIM_E_NULL when io->finished is NULL.
+ * Available since ABI 5 without a version bump (no struct or signature changed): look the symbol up to detect it. */
+int dexsim_step_next_reset(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                           const uint16_t* group_of_env, const DexsimStepIO* io, void* stream);
+
 /* ---- fused rollout: replaces the caller loops training/episode_utils.py:42-53,
  *      evaluation/evaluator.py:135-158, evaluation/robustness_tests.py:292-304 with the policy
  *      (policies/random_policy.py:40 / policies/heuristic_policy.py:55-62) generated in-kernel.
