@@ -552,7 +552,7 @@ reset_philox_kernel(const DexsimState st, const DexsimParams p, const DexsimGrou
 // load_env -> finish_and_reset -> store_env_full, and the reset observation's noise.  Before the reset, the column the
 // step returned (noisy_obs when observation noise is on, obs otherwise) is copied into `final_obs`; columns of envs
 // that did not finish are not written.  One thread per env of a grid-stride loop: a warp without a finished lane moves
-// on after one ballot.  `pdl`: launched as a programmatic dependent of the step (see launch_finish_reset).
+// on after one ballot.  `pdl`: launched as a programmatic dependent of the step (see step_then_finish_reset).
 //
 // HOST (dexsim_step_host_final): the outputs of `hf` instead of `final_obs`, all of them device aliases of the caller's
 // mapped page-locked buffers, offset to the chunk.
@@ -1011,15 +1011,13 @@ static void launch_step_variant(bool extras, bool next, int grid, cudaStream_t s
     else             step_kernel<DENSE, AOS, false, false><<<grid, STEP_THREADS, 0, s>>>(st, p, groups, goe, io);
 }
 
-template <bool DENSE, bool AOS, int TRACK, bool EXTRA, int STAGES, int TILE_, bool NEXT>
-static int launch_tma_variant(int sm_count, cudaStream_t s, const DexsimState& st, const DexsimParams& p,
-                              const DexsimGroup* groups, const uint16_t* goe, const DexsimStepIO& io,
-                              const StepMaps& maps, int num_tiles) {
-    auto kern = step_tma_kernel<DENSE, AOS, TRACK, EXTRA, STAGES, TILE_, NEXT>;
-    constexpr int TMA_THREADS = TILE_ + 32;            // one compute thread per env of a tile + the producer warp
-    const size_t smem = (size_t)STAGES * StageLayout<TILE_>::stage_bytes(TRACK) + 2 * STAGES * (sizeof(uint64_t) + sizeof(int)) +
-                        (TRACK ? TMA_GROUPS_MAX * (DEXSIM_NCOUNTERS * sizeof(unsigned long long) + 2 * sizeof(double)) : 0);
-    // per template instantiation and per device: the shared-memory opt-in is a per-device function attribute
+// Launches KERNEL with programmatic dependent launch, eagerly and inside captured graphs: its grid may start while the
+// previous grid on `s` drains and blocks in griddepcontrol.wait until that grid has completed -- stream order is
+// preserved for every access.  `grid_of(CTAs per SM)` must stay within one resident wave (SMs x CTAs per SM), so that
+// all CTAs of a launch are resident at once and a waiting grid can never keep its predecessor's CTAs off the SMs.
+template <auto KERNEL, typename GridOf, typename... Args>
+static int launch_pdl(int threads, size_t smem, GridOf grid_of, cudaStream_t s, const Args&... args) {
+    // per kernel and per device: the shared-memory opt-in is a per-device function attribute
     static thread_local int occupancy[64] = {0};
     int dev = 0;
     cudaError_t err = cudaGetDevice(&dev);
@@ -1027,29 +1025,39 @@ static int launch_tma_variant(int sm_count, cudaStream_t s, const DexsimState& s
     int uncached = 0;
     int& ctas_per_sm = (dev >= 0 && dev < 64) ? occupancy[dev] : uncached;
     if (ctas_per_sm == 0) {
-        err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (err != cudaSuccess) return -(int)err;
-        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kern, TMA_THREADS, smem);
+        if (smem) {
+            err = cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            if (err != cudaSuccess) return -(int)err;
+        }
+        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, KERNEL, threads, smem);
         if (err != cudaSuccess) return -(int)err;
         if (ctas_per_sm < 1) ctas_per_sm = 1;
     }
-    int grid = sm_count * ctas_per_sm;
-    if (grid > num_tiles) grid = num_tiles;
-    // Programmatic dependent launch, eagerly and inside captured graphs: this grid may start (barrier init, counter
-    // staging) while the previous step's grid drains and blocks in griddepcontrol.wait until that grid has completed --
-    // stream order is preserved for every access.  All CTAs of a launch are resident at once (grid <= SMs x CTAs per SM),
-    // so a waiting grid can never keep its predecessor's CTAs off the SMs.  Measured on B200, us per step with / without:
-    // eager (tools/time_small.py) 131,072 envs 12.1 / 14.3, 1 Mi 67.7 / 70.0; replayed from capture_step(steps=8)
-    // (tools/time_graph.py) 65,536 envs 9.4 / 10.6, 131,072 12.6 / 13.6, 1 Mi 69.2 / 70.0.  Eager stepping with PDL
-    // (9.3 / 12.1 / 67.1) is as fast as a graph replay once the GPU, not the host, is the bound (>= 65,536 envs); at
-    // 4,096 envs the replay wins (6.5 vs 7.5, the eager loop runs at the host's issue rate).
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3(TMA_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = s;
+    cfg.gridDim = dim3((unsigned)grid_of(ctas_per_sm)); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = smem; cfg.stream = s;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    return cuda_rc(cudaLaunchKernelEx(&cfg, kern, st, p, groups, goe, io, maps, num_tiles, /*pdl=*/1));
+    return cuda_rc(cudaLaunchKernelEx(&cfg, KERNEL, args...));
+}
+
+template <bool DENSE, bool AOS, int TRACK, bool EXTRA, int STAGES, int TILE_, bool NEXT>
+static int launch_tma_variant(int sm_count, cudaStream_t s, const DexsimState& st, const DexsimParams& p,
+                              const DexsimGroup* groups, const uint16_t* goe, const DexsimStepIO& io,
+                              const StepMaps& maps, int num_tiles) {
+    constexpr int TMA_THREADS = TILE_ + 32;            // one compute thread per env of a tile + the producer warp
+    const size_t smem = (size_t)STAGES * StageLayout<TILE_>::stage_bytes(TRACK) + 2 * STAGES * (sizeof(uint64_t) + sizeof(int)) +
+                        (TRACK ? TMA_GROUPS_MAX * (DEXSIM_NCOUNTERS * sizeof(unsigned long long) + 2 * sizeof(double)) : 0);
+    // Programmatic dependent launch lets this grid start (barrier init, counter staging) while the previous step's grid
+    // drains.  Measured on B200, us per step with / without:
+    // eager (tools/time_small.py) 131,072 envs 12.1 / 14.3, 1 Mi 67.7 / 70.0; replayed from capture_step(steps=8)
+    // (tools/time_graph.py) 65,536 envs 9.4 / 10.6, 131,072 12.6 / 13.6, 1 Mi 69.2 / 70.0.  Eager stepping with PDL
+    // (9.3 / 12.1 / 67.1) is as fast as a graph replay once the GPU, not the host, is the bound (>= 65,536 envs); at
+    // 4,096 envs the replay wins (6.5 vs 7.5, the eager loop runs at the host's issue rate).
+    return launch_pdl<step_tma_kernel<DENSE, AOS, TRACK, EXTRA, STAGES, TILE_, NEXT>>(
+        TMA_THREADS, smem, [&](int ctas_per_sm) { return sm_count * ctas_per_sm < num_tiles ? sm_count * ctas_per_sm : num_tiles; }, s,
+        st, p, groups, goe, io, maps, num_tiles, /*pdl=*/1);
 }
 
 // Step kernel (dexsim_set_step_impl): 0 = auto (TMA pipeline when eligible), 1 = register-resident kernel only,
@@ -1218,37 +1226,47 @@ static int launch_step(const DexsimState* st, const DexsimParams* p, const Dexsi
     return cuda_rc(cudaGetLastError());
 }
 
-// The pass of dexsim_step_final (HOST: of dexsim_step_host_final): one resident wave of CTAs, launched as a programmatic
-// dependent of the step, so that its launch and counter staging overlap the step's tail (griddepcontrol.wait orders every
-// global access behind the step).
+// dexsim_step_final (HOST: one chunk of dexsim_step_host_final, outputs in `hf`): the step without the reset, which leaves
+// the observation of the step that ended an episode in obs / noisy_obs and writes neither `finished` nor the counters,
+// then the finish-and-reset pass, which resets, counts and writes them.  The pass is one resident wave of CTAs, launched
+// as a programmatic dependent of the step, so that its launch and counter staging overlap the step's tail.
 template <bool HOST>
-static int launch_finish_reset(const DexsimState& st, const DexsimParams& p, const DexsimGroup* groups, const uint16_t* goe,
-                               const DexsimStepIO& io, float* final_obs, const FinishHost& hf, cudaStream_t s, int sm_count) {
-    auto kern = finish_reset_kernel<HOST>;
-    const int smem = HOST ? FINISH_HOST_SMEM : 0;
-    static thread_local int occupancy[64] = {0};
-    int dev = 0;
-    cudaError_t err = cudaGetDevice(&dev);
-    if (err != cudaSuccess) return -(int)err;
-    int uncached = 0;
-    int& ctas_per_sm = (dev >= 0 && dev < 64) ? occupancy[dev] : uncached;
-    if (ctas_per_sm == 0) {
-        if (HOST) {                 // the record blocks and the static counter arrays together exceed the default 48 KB
-            err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-            if (err != cudaSuccess) return -(int)err;
-        }
-        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, kern, STEP_THREADS, smem);
-        if (err != cudaSuccess) return -(int)err;
-        if (ctas_per_sm < 1) ctas_per_sm = 1;
-    }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid_for(st.n, STEP_THREADS, ctas_per_sm, sm_count));
-    cfg.blockDim = dim3(STEP_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    return cuda_rc(cudaLaunchKernelEx(&cfg, kern, st, p, groups, goe, io, final_obs, /*pdl=*/1, hf));
+static int step_then_finish_reset(const DexsimState& st, const DexsimParams& p, const DexsimGroup* groups, const uint16_t* goe,
+                                  const DexsimStepIO& io, float* final_obs, const FinishHost& hf, cudaStream_t s) {
+    DexsimParams sp = p;
+    sp.auto_reset = 0;
+    DexsimStepIO sio = io;
+    sio.finished = nullptr; sio.counters = nullptr; sio.ret_sums = nullptr;
+    int rc = launch_step(&st, &sp, groups, goe, &sio, s);
+    if (rc || st.n == 0) return rc;
+    DeviceInfo di;
+    rc = device_info_cached(di);
+    if (rc) return rc;
+    // HOST: the record blocks and the static counter arrays together exceed the default 48 KB of shared memory
+    return launch_pdl<finish_reset_kernel<HOST>>(
+        STEP_THREADS, HOST ? FINISH_HOST_SMEM : 0,
+        [&](int ctas_per_sm) { return grid_for(st.n, STEP_THREADS, ctas_per_sm, di.sm_count); }, s,
+        st, p, groups, goe, io, final_obs, /*pdl=*/1, hf);
+}
+
+// The arguments every auto-reset entry point checks first, in this order: p and io, auto-reset on, then its outputs
+// (`outputs`: whether the entry point's own outputs are present; io->finished is one of every such entry point).
+static int check_auto_reset(const DexsimParams* p, const DexsimStepIO* io, bool outputs) {
+    if (!p || !io) return DEXSIM_E_NULL;
+    if (!p->auto_reset) return DEXSIM_E_PARAM;
+    if (!outputs || !io->finished) return DEXSIM_E_NULL;
+    return 0;
+}
+
+// ... and, of the entry points that run the step without the reset (step_then_finish_reset), the state and the limits of
+// an auto-reset call, which that step does not check.
+static int check_finish_reset(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups, const DexsimStepIO* io,
+                              bool outputs) {
+    int rc = check_auto_reset(p, io, outputs);
+    if (rc) return rc;
+    rc = check_state(st);
+    if (rc) return rc;
+    return check_params(p, true, groups, st->ep_return != nullptr);
 }
 
 }  // namespace dexsim
@@ -1259,6 +1277,17 @@ void expand_contact_rows_range(float* h_obs, const uint8_t* mask, int64_t lo, in
 }  // namespace dexsim
 
 using namespace dexsim;
+
+template <bool TAGGED>
+static int pack_env(const DexsimState* st, const DexsimStepIO* io, int64_t index, int32_t after_reset, double* out64,
+                    double tag, void* stream) {
+    int rc = check_state(st);
+    if (rc) return rc;
+    if (!io || !out64 || !io->reward || !io->terminated || !io->truncated) return DEXSIM_E_NULL;
+    if (index < 0 || index >= st->n) return DEXSIM_E_SIZE;
+    pack_env_kernel<TAGGED><<<1, 64, 0, (cudaStream_t)stream>>>(*st, *io, index, after_reset ? 1 : 0, out64, tag);
+    return cuda_rc(cudaGetLastError());
+}
 
 static std::atomic<int64_t> g_zero_copy_steps{0};    // dexsim_step_host calls served by the single-launch transport
 
@@ -1361,33 +1390,19 @@ int dexsim_step_single(const DexsimState* st, const DexsimParams* p, const Dexsi
 
 int dexsim_step_final(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
                       const uint16_t* group_of_env, const DexsimStepIO* io, float* final_obs, void* stream) {
-    if (!p || !io) return DEXSIM_E_NULL;
-    if (!p->auto_reset || io->host_static_rows || (io->flags & DEXSIM_STEP_HOST_ALL_ROWS)) return DEXSIM_E_PARAM;
-    if (!final_obs || !io->finished) return DEXSIM_E_NULL;
-    int rc = check_state(st);
+    // the host mirrors are dexsim_step_host's (a NULL p or io is check_auto_reset's error)
+    if (p && io && (io->host_static_rows || (io->flags & DEXSIM_STEP_HOST_ALL_ROWS))) return DEXSIM_E_PARAM;
+    const int rc = check_finish_reset(st, p, groups, io, final_obs != nullptr);
     if (rc) return rc;
-    // the limits of an auto-reset call (the step below runs without auto-reset and would not check them)
-    rc = check_params(p, true, groups, st->ep_return != nullptr);
-    if (rc) return rc;
-    // the step without the reset: it leaves the observation of the step that ended an episode in obs / noisy_obs
-    DexsimParams sp = *p;
-    sp.auto_reset = 0;
-    DexsimStepIO sio = *io;
-    sio.finished = nullptr; sio.counters = nullptr; sio.ret_sums = nullptr;
-    const cudaStream_t s = (cudaStream_t)stream;
-    rc = launch_step(st, &sp, groups, group_of_env, &sio, s);
-    if (rc || st->n == 0) return rc;
-    DeviceInfo di;
-    rc = device_info_cached(di);
-    if (rc) return rc;
-    return launch_finish_reset<false>(*st, *p, groups, group_of_env, *io, final_obs, FinishHost{}, s, di.sm_count);
+    return step_then_finish_reset<false>(*st, *p, groups, group_of_env, *io, final_obs, FinishHost{}, (cudaStream_t)stream);
 }
 
 int dexsim_step_next_reset(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
                            const uint16_t* group_of_env, const DexsimStepIO* io, void* stream) {
-    if (!p || !io) return DEXSIM_E_NULL;
-    if (!p->auto_reset || io->host_static_rows || (io->flags & DEXSIM_STEP_HOST_ALL_ROWS)) return DEXSIM_E_PARAM;
-    if (!io->finished) return DEXSIM_E_NULL;
+    // the host mirrors are dexsim_step_host's (a NULL p or io is check_auto_reset's error)
+    if (p && io && (io->host_static_rows || (io->flags & DEXSIM_STEP_HOST_ALL_ROWS))) return DEXSIM_E_PARAM;
+    const int rc = check_auto_reset(p, io, true);
+    if (rc) return rc;
     return launch_step(st, p, groups, group_of_env, io, (cudaStream_t)stream, nullptr, 0.0, /*next=*/true);
 }
 
@@ -1450,22 +1465,12 @@ int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGro
 
 int dexsim_pack_env(const DexsimState* st, const DexsimStepIO* io, int64_t index, int32_t after_reset, double* out64,
                     void* stream) {
-    int rc = check_state(st);
-    if (rc) return rc;
-    if (!io || !out64 || !io->reward || !io->terminated || !io->truncated) return DEXSIM_E_NULL;
-    if (index < 0 || index >= st->n) return DEXSIM_E_SIZE;
-    pack_env_kernel<false><<<1, 64, 0, (cudaStream_t)stream>>>(*st, *io, index, after_reset ? 1 : 0, out64, 0.0);
-    return cuda_rc(cudaGetLastError());
+    return pack_env<false>(st, io, index, after_reset, out64, 0.0, stream);
 }
 
 int dexsim_pack_env_tagged(const DexsimState* st, const DexsimStepIO* io, int64_t index, int32_t after_reset, double* out64,
                            double tag, void* stream) {
-    int rc = check_state(st);
-    if (rc) return rc;
-    if (!io || !out64 || !io->reward || !io->terminated || !io->truncated) return DEXSIM_E_NULL;
-    if (index < 0 || index >= st->n) return DEXSIM_E_SIZE;
-    pack_env_kernel<true><<<1, 64, 0, (cudaStream_t)stream>>>(*st, *io, index, after_reset ? 1 : 0, out64, tag);
-    return cuda_rc(cudaGetLastError());
+    return pack_env<true>(st, io, index, after_reset, out64, tag, stream);
 }
 
 int dexsim_fill_policy_actions(const DexsimState* st, const DexsimParams* p, int32_t policy_kind, float* actions,
@@ -1623,13 +1628,6 @@ static int step_host_impl(const DexsimState* st, const DexsimParams* p, const De
     cudaStream_t user = (cudaStream_t)stream;
     const int64_t n = st->n, ld = st->ld;
     if (n == 0) return 0;
-    int sm_count = 0;
-    if (final) {
-        DeviceInfo di;
-        rc = device_info_cached(di);
-        if (rc) return rc;
-        sm_count = di.sm_count;
-    }
     const bool aos = io->action_layout == 1;
     // Zero-copy transport (DEXSIM_HOST_ZERO_COPY): the pipelined kernel itself writes every result into the caller's mapped
     // page-locked buffers -- the joint rows as a second bulk tensor store per tile, object z, its velocity and the contact
@@ -1704,14 +1702,7 @@ static int step_host_impl(const DexsimState* st, const DexsimParams* p, const De
     // Rows 30, 31, 37, 38 (object x, y and their velocities) only change when an episode is reset.  When h_obs is mapped
     // page-locked memory the step kernel mirrors every such change straight into it (DexsimStepIO.host_static_rows), and a
     // caller whose buffer is already current (DEXSIM_HOST_STATIC_ROWS) does not download those rows at all.
-    float* mirror = nullptr;
-    if (h_obs && !io->host_static_rows) {
-        cudaPointerAttributes attr;
-        if (cudaPointerGetAttributes(&attr, h_obs) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer)
-            mirror = static_cast<float*>(attr.devicePointer);
-        else
-            (void)cudaGetLastError();                 // pageable memory: not an error, just no mirror
-    }
+    float* mirror = io->host_static_rows ? nullptr : static_cast<float*>(mapped_alias(h_obs));
     const bool skip_static = (flags & DEXSIM_HOST_STATIC_ROWS) && mirror != nullptr && (flags & DEXSIM_HOST_SKIP_QUAT);
     // Whatever happens while enqueueing, the caller's stream is joined with the internal ones before returning,
     // so that no copy is still in flight on a stream the caller cannot see.
@@ -1766,13 +1757,6 @@ static int step_host_impl(const DexsimState* st, const DexsimParams* p, const De
         if (!final) {
             rc = launch_step(&sub, &sp, groups, goe, &sio, s);
         } else {
-            // as dexsim_step_final: the step without the reset, then the pass, which resets, counts and writes the records
-            DexsimParams np = sp;
-            np.auto_reset = 0;
-            DexsimStepIO nio = sio;
-            nio.finished = nullptr; nio.counters = nullptr; nio.ret_sums = nullptr;
-            rc = launch_step(&sub, &np, groups, goe, &nio, s);
-            if (rc) break;
             FinishHost hf = {};
             hf.final_obs = d_final + lo * NOBS;
             hf.obs = sio.host_static_rows;
@@ -1782,7 +1766,7 @@ static int step_host_impl(const DexsimState* st, const DexsimParams* p, const De
                 hf.terminated = zflags.terminated + lo; hf.truncated = zflags.truncated + lo; hf.finished = zflags.finished + lo;
                 hf.num_contacts = zflags.num_contacts ? zflags.num_contacts + lo : nullptr;
             }
-            rc = launch_finish_reset<true>(sub, sp, groups, goe, sio, nullptr, hf, s, sm_count);
+            rc = step_then_finish_reset<true>(sub, sp, groups, goe, sio, nullptr, hf, s);
         }
         if (rc) break;
         if (tracing) cudaEventRecord(g_trace.k[c], s);
@@ -1889,13 +1873,7 @@ int dexsim_step_host_final(const DexsimState* st, const DexsimParams* p, const D
                            float* h_reward, uint8_t* h_terminated, uint8_t* h_truncated, uint8_t* h_num_contacts,
                            uint8_t* h_contact_mask, uint8_t* h_finished, float* h_final_obs, int32_t chunks, int32_t flags,
                            void* stream) {
-    if (!p || !io) return DEXSIM_E_NULL;
-    if (!p->auto_reset) return DEXSIM_E_PARAM;
-    if (!h_finished || !h_final_obs || !io->finished) return DEXSIM_E_NULL;
-    int rc = check_state(st);
-    if (rc) return rc;
-    // the limits of an auto-reset call (the step runs without auto-reset and would not check them)
-    rc = check_params(p, true, groups, st->ep_return != nullptr);
+    const int rc = check_finish_reset(st, p, groups, io, h_finished && h_final_obs);
     if (rc) return rc;
     return step_host_impl(st, p, groups, group_of_env, io, h_action, h_obs, h_reward, h_terminated, h_truncated,
                           h_num_contacts, h_contact_mask, h_finished, h_final_obs, chunks, flags, stream);

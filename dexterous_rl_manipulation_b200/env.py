@@ -227,11 +227,9 @@ class BatchedManipulationEnv:
         self._noisy_obs = None
         self._obs_noise = None
         self._dyn_noise = None
-        self._goe = None
+        self._goe = self._goe_ptr = None
         if group_of_env is not None:
-            goe = torch.as_tensor(group_of_env).to(torch.int16).to(dev)
-            self._goe = torch.zeros(ld, dtype=torch.int16, device=dev)
-            self._goe[:n] = goe
+            self._set_group_of_env(group_of_env)
         self._groups_dev = None
         self.counters = None
         self.ret_sums = None
@@ -259,11 +257,14 @@ class BatchedManipulationEnv:
         self.host_zero_copy = "auto"
         self._h_primed_slot = None                       # result slot whose pinned observation is current (see step_host)
         self._state_ref, self._params_ref, self._io_ref = C.byref(self._state), C.byref(self._params), C.byref(self._io)
-        self._goe_ptr = self._ptr(self._goe)
-        self._final_obs_ptr = self._ptr(self._final_obs)
-        # the one-launch step entry of this env (dexsim_step_final is called where _final_obs is set)
-        self._step_entry = self._lib.dexsim_step_next_reset if self._next_step else self._lib.dexsim_step
-        self._step_entry_name = "dexsim_step_next_reset" if self._next_step else "dexsim_step"
+        # the step entry of this env, chosen once; dexsim_step_final takes the final-observation buffer before the stream
+        self._step_entry_name = ("dexsim_step_final" if self.final_observation else
+                                 "dexsim_step_next_reset" if self._next_step else "dexsim_step")
+        self._step_entry = getattr(self._lib, self._step_entry_name)
+        self._step_final_obs = self._ptr(self._final_obs)
+        # filled on first use: pinned host buffers (a batched env pins none it does not use), the rollout's optional outputs
+        self._action_pin = self._pack_host = self._ep_log = self._ep_log_count = self._hist = self._learner_mean = None
+        self._h_slots, self._host_keepalive = {}, {}
         self._step_out = None
         if not self.single:
             self._step_out = (self._obs_view, self._reward[:n], self._terminated[:n].view(torch.bool),
@@ -342,10 +343,13 @@ class BatchedManipulationEnv:
         self._group_cfgs = list(configs)
         self._group_sigma = (sigma_obs, sigma_dyn)
         if group_of_env is not None:
-            self._goe = torch.zeros(self.ld, dtype=torch.int16, device=self.device)
-            self._goe[:self.num_envs] = torch.as_tensor(group_of_env).to(torch.int16).to(self.device)
-            self._goe_ptr = self._goe.data_ptr()
+            self._set_group_of_env(group_of_env)
         self._groups_dirty = True
+
+    def _set_group_of_env(self, group_of_env):
+        self._goe = torch.zeros(self.ld, dtype=torch.int16, device=self.device)
+        self._goe[:self.num_envs] = torch.as_tensor(group_of_env).to(torch.int16).to(self.device)
+        self._goe_ptr = self._goe.data_ptr()
 
     @property
     def num_groups(self):
@@ -460,34 +464,27 @@ class BatchedManipulationEnv:
                 m = torch.as_tensor(options["mask"]).to(self.device).to(torch.uint8)
                 mask = torch.zeros(self.ld, dtype=torch.uint8, device=self.device)
                 mask[:self.num_envs] = m
-            n, ld = self.num_envs, self.ld
+            n = self.num_envs
             respawn = self._respawn_now()
             if self.rng_mode == "numpy":
                 rngs = self._host_rngs(seed)
-                jp0 = np.zeros((15, ld), np.float32)
-                size = np.zeros(ld); mass = np.zeros(ld); fric = np.zeros(ld)
-                pos = np.zeros((3, ld), np.float32) if (respawn or (not self._spawned and self._object_position_arg is not None)) else None
+                jp0 = np.zeros((n, 15), np.float32)
+                size = np.zeros(n); mass = np.zeros(n); fric = np.zeros(n)
+                pos = np.zeros((n, 3), np.float32) if (respawn or (not self._spawned and self._object_position_arg is not None)) else None
                 mask_host = None if mask is None else mask.cpu().numpy()
                 for i in range(n):
                     if mask_host is not None and not mask_host[i]:
                         continue
                     r, cfg = rngs[i], self._config_of_env(i)
-                    jp0[:, i] = r.uniform(low=-0.1, high=0.1, size=(15,)).astype(np.float32)       # :143-145
+                    jp0[i] = r.uniform(low=-0.1, high=0.1, size=(15,)).astype(np.float32)          # :143-145
                     size[i] = cfg.get_object_size(r); mass[i] = cfg.get_object_mass(r)            # :151-153
                     fric[i] = cfg.get_friction_coefficient(r)
                     if respawn:
-                        pos[:, i] = np.array(cfg.get_spawn_position(r), dtype=np.float32)         # :156-159
+                        pos[i] = np.array(cfg.get_spawn_position(r), dtype=np.float32)            # :156-159
                     elif pos is not None:
                         a = self._object_position_arg
-                        pos[:, i] = a if a.ndim == 1 else a[i]                                     # :160-161
-                dev = self.device
-                t = lambda a: torch.from_numpy(a).to(dev)
-                jp0_d, size_d, mass_d, fric_d = t(jp0), t(size), t(mass), t(fric)
-                pos_d = None if pos is None else t(pos)
-                _lib.check(self._lib.dexsim_reset_predrawn(
-                    C.byref(self._state), C.byref(self._params), self._ptr(mask), self._ptr(jp0_d), self._ptr(size_d),
-                    self._ptr(mass_d), self._ptr(fric_d), self._ptr(pos_d), self._stream()), "dexsim_reset_predrawn")
-                torch.cuda.current_stream(self.device).synchronize()     # host arrays go out of scope
+                        pos[i] = a if a.ndim == 1 else a[i]                                        # :160-161
+                self._reset_predrawn(jp0, size, mass, fric, pos, mask)
             else:
                 if seed is not None:
                     self.seed = int(seed)
@@ -511,7 +508,7 @@ class BatchedManipulationEnv:
                 self._custom_reward.reset()                  # envs/manipulation_env.py:177
             if mask is None:
                 self._rollout_steps = 0
-                if getattr(self, "_ep_log_count", None) is not None:
+                if self._ep_log_count is not None:
                     self._ep_log_count.zero_()
                 if self.rng_mode == "numpy":
                     self._episode.zero_()
@@ -525,31 +522,26 @@ class BatchedManipulationEnv:
         self._h_primed_slot = None
         with torch.cuda.device(dev):
             self._sync_groups()
-
-            def soa(x, rows, dtype):
-                t = torch.as_tensor(np.asarray(x), dtype=dtype).reshape(n, rows) if rows else \
-                    torch.as_tensor(np.broadcast_to(np.asarray(x, np.float64), (n,)).copy(), dtype=dtype)
-                out = torch.zeros((rows, ld) if rows else (ld,), dtype=dtype, device=dev)
-                if rows:
-                    out[:, :n] = t.t().to(dev)
-                else:
-                    out[:n] = t.to(dev)
-                return out
-
-            jp0_d = soa(jp0, 15, torch.float32)
-            size_d, mass_d, fric_d = soa(size, 0, torch.float64), soa(mass, 0, torch.float64), soa(friction, 0, torch.float64)
-            pos_d = None if pos is None else soa(pos, 3, torch.float32)
             mask_d = None
             if mask is not None:
                 mask_d = torch.zeros(ld, dtype=torch.uint8, device=dev)
                 mask_d[:n] = torch.as_tensor(np.asarray(mask)).to(torch.uint8).to(dev)
-            _lib.check(self._lib.dexsim_reset_predrawn(
-                C.byref(self._state), C.byref(self._params), self._ptr(mask_d), self._ptr(jp0_d), self._ptr(size_d),
-                self._ptr(mass_d), self._ptr(fric_d), self._ptr(pos_d), self._stream()), "dexsim_reset_predrawn")
-            torch.cuda.current_stream(dev).synchronize()
+            self._reset_predrawn(jp0, size, mass, friction, pos, mask_d)
             self._spawned = True
             self._did_reset = True
             return self._reset_outputs()
+
+    def _reset_predrawn(self, jp0, size, mass, friction, pos, mask):
+        """dexsim_reset_predrawn of the envs in ``mask`` (device uint8 [ld], None = all) from host draws, batch first as
+        reset_from_draws() takes them; returns once the kernel has read them."""
+        per_env = lambda x: self._soa(np.broadcast_to(np.asarray(x, np.float64), (self.num_envs,)).copy(), 1,
+                                       torch.float64)
+        jp0_d, size_d, mass_d, fric_d = self._soa(jp0, 15), per_env(size), per_env(mass), per_env(friction)
+        pos_d = None if pos is None else self._soa(pos, 3)
+        _lib.check(self._lib.dexsim_reset_predrawn(
+            self._state_ref, self._params_ref, self._ptr(mask), self._ptr(jp0_d), self._ptr(size_d),
+            self._ptr(mass_d), self._ptr(fric_d), self._ptr(pos_d), self._stream()), "dexsim_reset_predrawn")
+        torch.cuda.current_stream(self.device).synchronize()
 
     # ------------------------------------------------------------------ step
     def _ingest_action(self, action):
@@ -573,13 +565,17 @@ class BatchedManipulationEnv:
         if self.single:
             # 60 bytes: the kernel reads them from mapped page-locked host memory, no copy call.  Safe to
             # overwrite: every single-env step ends by waiting for its result, so no kernel is still reading.
-            if getattr(self, "_action_pin", None) is None:
-                self._action_pin = torch.zeros(16, dtype=torch.float32).pin_memory()
-                self._action_pin_np = self._action_pin.numpy()
-            self._action_pin_np[:15] = a.reshape(15)
+            self._pin_action()[:15] = a.reshape(15)
             return self._action_pin
         self._action_dev.copy_(torch.from_numpy(np.ascontiguousarray(a.reshape(n, 15))), non_blocking=False)
         return self._action_dev
+
+    def _pin_action(self):
+        """NumPy view of the single env's page-locked action buffer, allocated on first use."""
+        if self._action_pin is None:
+            self._action_pin = torch.zeros(16, dtype=torch.float32).pin_memory()
+            self._action_pin_np = self._action_pin.numpy()
+        return self._action_pin_np
 
     def _noise_buffers(self):
         if self._noisy_obs is None:
@@ -587,12 +583,19 @@ class BatchedManipulationEnv:
             self._obs_noise = torch.zeros(45, self.ld, dtype=torch.float32, device=self.device)
             self._dyn_noise = torch.zeros(15, self.ld, dtype=torch.float32, device=self.device)
 
-    def _soa(self, x, rows):
-        """[n, rows] batch-first (or [rows] for a single env) -> SoA [rows, ld] device tensor."""
-        t = torch.as_tensor(x, dtype=torch.float32, device=self.device).reshape(self.num_envs, rows)
-        out = torch.zeros(rows, self.ld, dtype=torch.float32, device=self.device)
-        out[:, :self.num_envs] = t.t()
+    def _soa(self, x, rows, dtype=torch.float32, steps=None):
+        """Batch-first [n, rows] (or [rows] for a single env; [steps, n, rows] with ``steps``) -> SoA [rows, ld]
+        ([steps, rows, ld]) device tensor, zero past n."""
+        lead = () if steps is None else (steps,)
+        t = torch.as_tensor(x, dtype=dtype, device=self.device).reshape(*lead, self.num_envs, rows)
+        out = torch.zeros(*lead, rows, self.ld, dtype=dtype, device=self.device)
+        out[..., :self.num_envs] = t.transpose(-1, -2)
         return out
+
+    @staticmethod
+    def _clear_noise(io):
+        io.dyn_noise = io.obs_noise = io.noisy_obs = None
+        io.sigma_dyn = io.sigma_obs = 0.0
 
     def step(self, action, dyn_noise=None, obs_noise=None):
         """envs/manipulation_env.py:184-252 for every env.  ``dyn_noise`` [n,15] / ``obs_noise`` [n,45]
@@ -612,17 +615,18 @@ class BatchedManipulationEnv:
             io.action, io.action_layout = action.data_ptr(), 1
             io.flags ^= self._alternate_tiles          # walk the batch back and forth: a step starts on what is still in L2
             if self._io_has_noise:
-                io.dyn_noise = io.obs_noise = io.noisy_obs = None
-                io.sigma_dyn = io.sigma_obs = 0.0
+                self._clear_noise(io)
                 self._io_has_noise = False
-            if self._final_obs is None:
-                rc = self._step_entry(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
-                                      self._io_ref, _raw_stream(self.device.index))
+            # two spelled-out calls: a starred one costs ~0.1 us, which shows at the host-bound batch sizes
+            fo = self._step_final_obs
+            if fo is None:
+                rc = self._step_entry(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr, self._io_ref,
+                                      _raw_stream(self.device.index))
             else:
-                rc = self._lib.dexsim_step_final(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
-                                                 self._io_ref, self._final_obs_ptr, _raw_stream(self.device.index))
+                rc = self._step_entry(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr, self._io_ref,
+                                      fo, _raw_stream(self.device.index))
             if rc:
-                raise _lib.DexsimError(rc, "dexsim_step_final" if self._final_obs is not None else self._step_entry_name)
+                raise _lib.DexsimError(rc, self._step_entry_name)
             return self._step_out
         if (self.single and dyn_noise is None and obs_noise is None and not self._noisy_env
                 and not (isinstance(action, torch.Tensor) and action.is_cuda)
@@ -636,15 +640,12 @@ class BatchedManipulationEnv:
         (dexsim_step_single), persistent argument structs, result decoded from mapped host memory."""
         io = self._io_single
         if io is None:
-            if getattr(self, "_action_pin", None) is None:
-                self._action_pin = torch.zeros(16, dtype=torch.float32).pin_memory()
-                self._action_pin_np = self._action_pin.numpy()
-            if getattr(self, "_pack_host", None) is None:
+            self._pin_action()
+            if self._pack_host is None:
                 self._next_pack_tag()                   # allocates the mapped result record
             io = self._io_single = _lib.DexsimStepIO.from_buffer_copy(self._io)
             io.action, io.action_layout = self._action_pin.data_ptr(), 1
-            io.dyn_noise = io.obs_noise = io.noisy_obs = None
-            io.sigma_dyn = io.sigma_obs = 0.0
+            self._clear_noise(io)
             self._io_single_ref = C.byref(io)
             self._pack_ptr = self._pack_host.data_ptr()
         # float64 / list actions are cast exactly like the general path's astype(np.float32)
@@ -665,8 +666,7 @@ class BatchedManipulationEnv:
         group_obs, group_dyn = self._group_noise
         want_dyn = dyn_noise is not None or self.dynamics_noise_std > 0.0 or group_dyn
         want_obs = obs_noise is not None or self.observation_noise_std > 0.0 or group_obs
-        io.dyn_noise = io.obs_noise = io.noisy_obs = None
-        io.sigma_dyn = io.sigma_obs = 0.0
+        self._clear_noise(io)
         self._io_has_noise = want_dyn or want_obs
         if want_dyn or want_obs:
             self._noise_buffers()
@@ -764,20 +764,14 @@ class BatchedManipulationEnv:
         io = self._io
         self._h_primed_slot = None
         io.action, io.action_layout = action_soa.data_ptr(), 0
-        io.dyn_noise = io.obs_noise = io.noisy_obs = None
-        io.sigma_dyn = io.sigma_obs = 0.0
+        self._clear_noise(io)
         self._launch_step()
         return self._step_out
 
     def _launch_step(self):
-        """dexsim_step (dexsim_step_next_reset in next-step mode), or dexsim_step_final when the env returns final
-        observations."""
-        if self._final_obs is None:
-            _lib.check(self._step_entry(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
-                                        self._io_ref, self._stream()), self._step_entry_name)
-        else:
-            _lib.check(self._lib.dexsim_step_final(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr,
-                                                   self._io_ref, self._final_obs_ptr, self._stream()), "dexsim_step_final")
+        extra = () if self._step_final_obs is None else (self._step_final_obs,)
+        _lib.check(self._step_entry(self._state_ref, self._params_ref, self._groups_ptr, self._goe_ptr, self._io_ref,
+                                    *extra, self._stream()), self._step_entry_name)
 
     def _reset_outputs(self):
         obs = self._emit_obs(reset=True)          # also draws the reset observation's noise when enabled
@@ -800,7 +794,7 @@ class BatchedManipulationEnv:
         return self._single_wait_decode(tag, after_reset)
 
     def _next_pack_tag(self):
-        if getattr(self, "_pack_host", None) is None:
+        if self._pack_host is None:
             # page-locked and (unified addressing) mapped into the device: the pack code writes straight into it
             self._pack_host = torch.zeros(64, dtype=torch.float64).pin_memory()
             self._pack_np = self._pack_host.numpy()
@@ -889,9 +883,7 @@ class BatchedManipulationEnv:
 
     # ------------------------------------------------------------------ host-buffer step (end to end)
     def _host_buffers(self, slot):
-        bufs = getattr(self, "_h_slots", None)
-        if bufs is None:
-            bufs = self._h_slots = {}
+        bufs = self._h_slots
         if slot not in bufs:
             n, ld = self.num_envs, self.ld
             pin = lambda *shape, dtype: torch.zeros(*shape, dtype=dtype).pin_memory()
@@ -964,8 +956,7 @@ class BatchedManipulationEnv:
             self._sync_groups()
             io = self._io
             io.action, io.action_layout = self._action_dev.data_ptr(), 1
-            io.dyn_noise = io.obs_noise = io.noisy_obs = None
-            io.sigma_dyn = io.sigma_obs = 0.0
+            self._clear_noise(io)
             args = (C.byref(self._state), C.byref(self._params), self._ptr(self._groups_dev), self._ptr(self._goe),
                     C.byref(io), a.data_ptr(), b["obs"].data_ptr(), b["reward"].data_ptr(), b["term"].data_ptr(),
                     b["trunc"].data_ptr(), b["nc"].data_ptr(), b["cmask"].data_ptr())
@@ -979,8 +970,6 @@ class BatchedManipulationEnv:
         self._h_primed_slot = slot if sync else None
         if not sync:
             # the upload may still be reading the action buffer: keep it alive until this slot is used again
-            if getattr(self, "_host_keepalive", None) is None:
-                self._host_keepalive = {}
             self._host_keepalive[slot] = a
         return b["out"]
 
@@ -1028,7 +1017,7 @@ class BatchedManipulationEnv:
     def read_episode_log(self, sort=True):
         """Finished episodes as a NumPy structured array (fields of DexsimEpisodeRecord), ordered by
         (t_end, env_gid) -- the order a sequential caller would have seen them in."""
-        if getattr(self, "_ep_log", None) is None:
+        if self._ep_log is None:
             raise RuntimeError("enable_episode_log() first")
         produced = int(self._ep_log_count.item())
         kept = min(produced, self._ep_log_capacity)
@@ -1059,7 +1048,7 @@ class BatchedManipulationEnv:
             raise RuntimeError("rollout() needs track_episodes=True (per-env history summaries)")
         kind = {"external": _L.POLICY_EXTERNAL, "random": _L.POLICY_RANDOM, "heuristic": _L.POLICY_HEURISTIC,
                 "learner": _L.POLICY_LEARNER}[policy]
-        if kind == _L.POLICY_LEARNER and getattr(self, "_learner_mean", None) is None:
+        if kind == _L.POLICY_LEARNER and self._learner_mean is None:
             self.enable_learner()
         with torch.cuda.device(self.device):
             self._sync_groups()
@@ -1072,14 +1061,10 @@ class BatchedManipulationEnv:
             keep = []
             rio = _lib.DexsimRolloutIO()
             if kind == _L.POLICY_EXTERNAL:
-                a = torch.as_tensor(actions, dtype=torch.float32, device=self.device).reshape(k_steps, self.num_envs, 15)
-                buf = torch.zeros(k_steps, 15, self.ld, dtype=torch.float32, device=self.device)
-                buf[:, :, :self.num_envs] = a.permute(0, 2, 1)
+                buf = self._soa(actions, 15, steps=k_steps)
                 rio.actions = buf.data_ptr(); keep.append(buf)
             if dyn_noise is not None:
-                d = torch.as_tensor(dyn_noise, dtype=torch.float32, device=self.device).reshape(k_steps, self.num_envs, 15)
-                nbuf = torch.zeros(k_steps, 15, self.ld, dtype=torch.float32, device=self.device)
-                nbuf[:, :, :self.num_envs] = d.permute(0, 2, 1)
+                nbuf = self._soa(dyn_noise, 15, steps=k_steps)
                 rio.dyn_noise = nbuf.data_ptr(); keep.append(nbuf)
             rio.counters, rio.ret_sums = self._ptr(self.counters), self._ptr(self.ret_sums)
             if kind == _L.POLICY_LEARNER:
@@ -1088,14 +1073,12 @@ class BatchedManipulationEnv:
                 for name, src, dt in (("learner_act_noise", learner_act_noise, torch.float32),
                                       ("learner_upd_noise", learner_upd_noise, torch.float64)):
                     if src is not None:         # pre-drawn [k, n, 15] (parity runs)
-                        d = torch.as_tensor(src, dtype=dt, device=self.device).reshape(k_steps, self.num_envs, 15)
-                        b = torch.zeros(k_steps, 15, self.ld, dtype=dt, device=self.device)
-                        b[:, :, :self.num_envs] = d.permute(0, 2, 1)
+                        b = self._soa(src, 15, dt, steps=k_steps)
                         setattr(rio, name, b.data_ptr()); keep.append(b)
-            if getattr(self, "_ep_log", None) is not None:
+            if self._ep_log is not None:
                 rio.ep_log, rio.ep_log_count = self._ep_log.data_ptr(), self._ep_log_count.data_ptr()
                 rio.ep_log_capacity = self._ep_log_capacity
-            if getattr(self, "_hist", None) is not None:
+            if self._hist is not None:
                 rio.hist, rio.hist_steps = self._hist.data_ptr(), self._hist_steps
             rio.step_base = self._rollout_steps
             rio.one_episode = int(bool(one_episode))
