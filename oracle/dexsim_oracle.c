@@ -465,16 +465,16 @@ typedef struct {
     dexo_env* e; int64_t lo, hi, n; const dexo_params* p; const dexo_group* groups;
     const uint16_t* group_of_env; const dexo_rollout_cfg* cfg; const float* actions;
     const float* dyn_noise; int64_t* counters; double* ret_sums; const dexo_learner* learner;
+    int32_t err;
 } rollout_job;
 
 static void finish_episode(dexo_env* e, const dexo_params* p, const dexo_rollout_cfg* cfg,
                            int terminated, int64_t* cnt, double* rs) {
     const int success = cfg->success_is_terminated ? terminated : 0;
-    const int64_t len = e->ep_steps < DEXO_HIST_MAX ? e->ep_steps : DEXO_HIST_MAX;
     const int la = dexo_classify_metrics(success, e->ep_steps, e->num_contacts, e->num_contacts,
-                                         e->hist, len, cfg->loop_max_steps, p->success_threshold);
+                                         e->hist, e->ep_steps, cfg->loop_max_steps, p->success_threshold);
     const int lb = dexo_classify_taxonomy(success, e->ep_steps, e->num_contacts, e->num_contacts,
-                                          e->hist, len, cfg->loop_max_steps, p->success_threshold, NULL);
+                                          e->hist, e->ep_steps, cfg->loop_max_steps, p->success_threshold, NULL);
     cnt[DEXO_CNT_EPISODES] += 1;
     cnt[DEXO_CNT_SUCCESSES] += success;
     cnt[DEXO_CNT_SUM_STEPS] += e->ep_steps;
@@ -516,7 +516,8 @@ static void* rollout_worker(void* arg) {
                 L->best[i] = r.total;
             }
             e->ep_return += r.total;                                 /* evaluator.py:144 */
-            if (e->ep_steps < DEXO_HIST_MAX) e->hist[e->ep_steps] = (uint8_t)e->num_contacts;
+            if (e->ep_steps >= DEXO_HIST_MAX) { j->err = DEXO_E_HIST; return NULL; }   /* labels need every count */
+            e->hist[e->ep_steps] = (uint8_t)e->num_contacts;
             e->ep_steps += 1;                                        /* evaluator.py:145 */
             if (te || tr || e->ep_steps >= cfg->loop_max_steps) {    /* evaluator.py:156, :135 */
                 finish_episode(e, j->p, cfg, te, cnt, rs);
@@ -531,9 +532,9 @@ static void* rollout_worker(void* arg) {
     return NULL;
 }
 
-static void rollout_impl(dexo_env* e, int64_t n, const dexo_params* p, const dexo_group* groups,
-                         const uint16_t* group_of_env, const dexo_rollout_cfg* cfg, const float* actions,
-                         const float* dyn_noise, const dexo_learner* learner, int64_t* counters, double* ret_sums) {
+static int32_t rollout_impl(dexo_env* e, int64_t n, const dexo_params* p, const dexo_group* groups,
+                            const uint16_t* group_of_env, const dexo_rollout_cfg* cfg, const float* actions,
+                            const float* dyn_noise, const dexo_learner* learner, int64_t* counters, double* ret_sums) {
     int threads = cfg->threads < 1 ? 1 : cfg->threads;
     if (threads > 256) threads = 256;
     if ((int64_t)threads > n) threads = (int)(n > 0 ? n : 1);
@@ -545,7 +546,7 @@ static void rollout_impl(dexo_env* e, int64_t n, const dexo_params* p, const dex
     rollout_job jobs[256]; pthread_t tid[256];
     for (int t = 0; t < threads; ++t) {
         rollout_job j = {e, n * t / threads, n * (t + 1) / threads, n, p, groups, group_of_env, cfg,
-                         actions, dyn_noise, tc + (size_t)t * G * DEXO_NCOUNTERS, tr + (size_t)t * G * 2, learner};
+                         actions, dyn_noise, tc + (size_t)t * G * DEXO_NCOUNTERS, tr + (size_t)t * G * 2, learner, 0};
         jobs[t] = j;
     }
     if (threads == 1) rollout_worker(&jobs[0]);
@@ -553,23 +554,26 @@ static void rollout_impl(dexo_env* e, int64_t n, const dexo_params* p, const dex
         for (int t = 0; t < threads; ++t) pthread_create(&tid[t], NULL, rollout_worker, &jobs[t]);
         for (int t = 0; t < threads; ++t) pthread_join(tid[t], NULL);
     }
+    int32_t err = 0;
     for (int t = 0; t < threads; ++t) {
         for (int k = 0; k < G * DEXO_NCOUNTERS; ++k) counters[k] += tc[(size_t)t * G * DEXO_NCOUNTERS + k];
         for (int k = 0; k < G * 2; ++k) ret_sums[k] += tr[(size_t)t * G * 2 + k];
+        if (jobs[t].err) err = jobs[t].err;
     }
     free(tc); free(tr);
+    return err;
 }
 
-void dexo_rollout(dexo_env* e, int64_t n, const dexo_params* p, const dexo_group* groups,
-                  const uint16_t* group_of_env, const dexo_rollout_cfg* cfg, const float* actions,
-                  const float* dyn_noise, int64_t* counters, double* ret_sums) {
-    rollout_impl(e, n, p, groups, group_of_env, cfg, actions, dyn_noise, NULL, counters, ret_sums);
+int32_t dexo_rollout(dexo_env* e, int64_t n, const dexo_params* p, const dexo_group* groups,
+                     const uint16_t* group_of_env, const dexo_rollout_cfg* cfg, const float* actions,
+                     const float* dyn_noise, int64_t* counters, double* ret_sums) {
+    return rollout_impl(e, n, p, groups, group_of_env, cfg, actions, dyn_noise, NULL, counters, ret_sums);
 }
 
-void dexo_rollout_learner(dexo_env* e, int64_t n, const dexo_params* p, const dexo_group* groups,
-                          const uint16_t* group_of_env, const dexo_rollout_cfg* cfg, const dexo_learner* L,
-                          int64_t* counters, double* ret_sums) {
-    rollout_impl(e, n, p, groups, group_of_env, cfg, NULL, NULL, L, counters, ret_sums);
+int32_t dexo_rollout_learner(dexo_env* e, int64_t n, const dexo_params* p, const dexo_group* groups,
+                             const uint16_t* group_of_env, const dexo_rollout_cfg* cfg, const dexo_learner* L,
+                             int64_t* counters, double* ret_sums) {
+    return rollout_impl(e, n, p, groups, group_of_env, cfg, NULL, NULL, L, counters, ret_sums);
 }
 
 int32_t dexo_sizeof_env(void) { return (int32_t)sizeof(dexo_env); }

@@ -27,7 +27,10 @@ extern "C" {
 #define DEXO_NF 5         /* num_fingers                        envs/manipulation_env.py:50  */
 #define DEXO_JPF 3        /* joints_per_finger                  envs/manipulation_env.py:51  */
 #define DEXO_OBS 45       /* 2*15 + 10 + 5                      envs/manipulation_env.py:96-106 */
-#define DEXO_HIST_MAX 1024
+/* per-step contact counts kept per env: the longest tracked episode the library accepts (5,242 steps, EPSTATS_MAX_STEPS
+ * in dexterous_rl_manipulation_b200/csrc/dexsim_core.cuh) rounded up to a multiple of 8.  A longer episode is an error
+ * of dexo_rollout, never a cut history. */
+#define DEXO_HIST_MAX 5248
 
 /* label codes: enum declaration order of FailureType (evaluation/metrics.py:15-22) and
  * FailureMode (evaluation/failure_taxonomy.py:14-26); -1 = success (classifier returns None) */
@@ -138,13 +141,16 @@ typedef struct {
     int32_t  pad_;
 } dexo_rollout_cfg;
 
-void dexo_rollout(dexo_env* e, int64_t n, const dexo_params* p, const dexo_group* groups,
-                  const uint16_t* group_of_env /* [n] or NULL: gid % num_groups */,
-                  const dexo_rollout_cfg* cfg,
-                  const float* actions /* [k,n,15] for policy 0 */,
-                  const float* dyn_noise /* [k,n,15] or NULL */,
-                  int64_t* counters /* [num_groups, DEXO_NCOUNTERS] accumulated */,
-                  double* ret_sums /* [num_groups, 2]: sum, sum of squares of episode returns */);
+/* Returns 0, or DEXO_E_HIST when an episode outgrew the history (DEXO_HIST_MAX steps); the envs are then left
+ * mid-step and the call's outputs are meaningless. */
+enum { DEXO_E_HIST = 1 };
+int32_t dexo_rollout(dexo_env* e, int64_t n, const dexo_params* p, const dexo_group* groups,
+                     const uint16_t* group_of_env /* [n] or NULL: gid % num_groups */,
+                     const dexo_rollout_cfg* cfg,
+                     const float* actions /* [k,n,15] for policy 0 */,
+                     const float* dyn_noise /* [k,n,15] or NULL */,
+                     int64_t* counters /* [num_groups, DEXO_NCOUNTERS] accumulated */,
+                     double* ret_sums /* [num_groups, 2]: sum, sum of squares of episode returns */);
 
 /* SimpleLearner (policies/simple_learner.py:13-95) as a per-env policy inside the rollout:
  * mean[n,15] float32 and best[n] float64 persist across calls; the normal draws of select_action
@@ -159,9 +165,9 @@ typedef struct {
     int32_t pad_;
 } dexo_learner;
 
-void dexo_rollout_learner(dexo_env* e, int64_t n, const dexo_params* p, const dexo_group* groups,
-                          const uint16_t* group_of_env, const dexo_rollout_cfg* cfg, const dexo_learner* L,
-                          int64_t* counters, double* ret_sums);
+int32_t dexo_rollout_learner(dexo_env* e, int64_t n, const dexo_params* p, const dexo_group* groups,
+                             const uint16_t* group_of_env, const dexo_rollout_cfg* cfg, const dexo_learner* L,
+                             int64_t* counters, double* ret_sums);
 
 int32_t dexo_sizeof_env(void);
 int32_t dexo_sizeof_group(void);

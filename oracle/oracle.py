@@ -13,7 +13,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _SO = os.path.join(_HERE, "_build", "libdexsim_oracle.so")
 
-NJ, NF, OBS, HIST_MAX, NCOUNTERS = 15, 5, 45, 1024, 18
+NJ, NF, OBS, HIST_MAX, NCOUNTERS = 15, 5, 45, 5248, 18     # HIST_MAX == DEXO_HIST_MAX (dexsim_oracle.h)
 LABELS_METRICS = ["slippage", "unstable_contacts", "misaligned_grasp", "timeout", "object_dropped",
                   "insufficient_contacts"]           # evaluation/metrics.py:15-22
 LABELS_TAXONOMY = ["slippage", "unstable_grasp", "misalignment", "timeout", "object_dropped",
@@ -55,9 +55,9 @@ _lib = None
 
 
 def build(force=False):
-    if force or not os.path.exists(_SO) or (
-            os.path.exists(os.path.join(_HERE, "dexsim_oracle.c"))
-            and os.path.getmtime(os.path.join(_HERE, "dexsim_oracle.c")) > os.path.getmtime(_SO)):
+    srcs = [os.path.join(_HERE, f) for f in ("dexsim_oracle.c", "dexsim_oracle.h")]   # the Makefile's prerequisites
+    if force or not os.path.exists(_SO) or any(
+            os.path.exists(f) and os.path.getmtime(f) > os.path.getmtime(_SO) for f in srcs):
         subprocess.run(["make", "-C", _HERE, "--no-print-directory"], check=True,
                        stdout=subprocess.DEVNULL)
     return _SO
@@ -73,6 +73,8 @@ def lib():
         _lib.dexo_classify_taxonomy.restype = C.c_int32
         _lib.dexo_sizeof_env.restype = C.c_int32
         _lib.dexo_sizeof_group.restype = C.c_int32
+        _lib.dexo_rollout.restype = C.c_int32
+        _lib.dexo_rollout_learner.restype = C.c_int32
         assert _lib.dexo_sizeof_env() == ENV_DTYPE.itemsize, (_lib.dexo_sizeof_env(), ENV_DTYPE.itemsize)
         assert _lib.dexo_sizeof_group() == GROUP_DTYPE.itemsize, (_lib.dexo_sizeof_group(), GROUP_DTYPE.itemsize)
     return _lib
@@ -80,6 +82,12 @@ def lib():
 
 def _p(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+def _check_rollout(rc):
+    if rc != 0:
+        raise RuntimeError(f"oracle rollout: an episode ran past the {HIST_MAX}-step contact history (code {rc}); "
+                           "its labels would need counts the oracle does not keep")
 
 
 def make_params(dense=True, max_episode_steps=200, weights=(1.0, 0.5, 0.3, 0.2)):
@@ -179,8 +187,8 @@ class OracleBatch:
             dyn_noise = np.ascontiguousarray(dyn_noise, np.float32).reshape(k_steps, self.n, NJ)
         if group_of_env is not None:
             group_of_env = np.ascontiguousarray(group_of_env, np.uint16)
-        self.lib.dexo_rollout(_p(self.env), C.c_int64(self.n), _p(self.params), _p(groups), _p(group_of_env),
-                              _p(cfg), _p(actions), _p(dyn_noise), _p(counters), _p(ret_sums))
+        _check_rollout(self.lib.dexo_rollout(_p(self.env), C.c_int64(self.n), _p(self.params), _p(groups), _p(group_of_env),
+                                             _p(cfg), _p(actions), _p(dyn_noise), _p(counters), _p(ret_sums)))
         return counters, ret_sums
 
 
@@ -203,8 +211,8 @@ def rollout_learner(batch, groups, k_steps, seed, mean, best, act_noise, upd_noi
     L = np.zeros(1, LEARNER_DTYPE)
     L["mean"], L["best"] = mean.ctypes.data, best.ctypes.data
     L["act_noise"], L["upd_noise"], L["clip_range"] = act_noise.ctypes.data, upd_noise.ctypes.data, clip_range
-    batch.lib.dexo_rollout_learner(_p(batch.env), C.c_int64(batch.n), _p(batch.params), _p(groups), None, _p(cfg), _p(L),
-                                   _p(counters), _p(ret_sums))
+    _check_rollout(batch.lib.dexo_rollout_learner(_p(batch.env), C.c_int64(batch.n), _p(batch.params), _p(groups), None,
+                                                  _p(cfg), _p(L), _p(counters), _p(ret_sums)))
     return counters, ret_sums
 
 
