@@ -89,6 +89,11 @@ class DexsimRolloutIO(C.Structure):
                 ("learner_clip", C.c_float), ("pad2_", C.c_int32)]
 
 
+class DexsimTrajectory(C.Structure):
+    _fields_ = [("obs", C.c_void_p), ("action", C.c_void_p), ("reward", C.c_void_p), ("terminated", C.c_void_p),
+                ("truncated", C.c_void_p), ("finished", C.c_void_p), ("capacity", C.c_int64)]
+
+
 class DexsimEpisodeSummary(C.Structure):
     _fields_ = [("success", C.c_int32), ("episode_steps", C.c_int32), ("num_contacts", C.c_int32),
                 ("final_contacts", C.c_int32), ("hist_len", C.c_int32), ("max_count", C.c_int32),
@@ -100,7 +105,8 @@ EXPORTS = (
     "dexsim_version", "dexsim_error_string", "dexsim_sizeof_state", "dexsim_sizeof_params",
     "dexsim_sizeof_group", "dexsim_sizeof_step_io", "dexsim_sizeof_rollout_io", "dexsim_sizeof_episode_record",
     "dexsim_device_info", "dexsim_set_step_impl", "dexsim_set_step_tile", "dexsim_set_rollout_impl", "dexsim_reset_predrawn",
-    "dexsim_reset_philox", "dexsim_step", "dexsim_rollout", "dexsim_fill_policy_actions",
+    "dexsim_reset_philox", "dexsim_step", "dexsim_rollout", "dexsim_rollout_record", "dexsim_sizeof_trajectory",
+    "dexsim_fill_policy_actions",
     "dexsim_fill_normal", "dexsim_classify_summary", "dexsim_step_host", "dexsim_pack_env", "dexsim_pack_env_tagged", "dexsim_step_single",
     "dexsim_step_final", "dexsim_step_host_final", "dexsim_step_next_reset",
     "dexsim_expand_contact_rows",
@@ -132,7 +138,7 @@ def lib():
     L.dexsim_error_string.restype = C.c_char_p
     L.dexsim_error_string.argtypes = [C.c_int]
     for name in ("dexsim_sizeof_state", "dexsim_sizeof_params", "dexsim_sizeof_group", "dexsim_sizeof_step_io",
-                 "dexsim_sizeof_rollout_io", "dexsim_sizeof_episode_record"):
+                 "dexsim_sizeof_rollout_io", "dexsim_sizeof_episode_record", "dexsim_sizeof_trajectory"):
         getattr(L, name).restype = C.c_int
     L.dexsim_device_info.argtypes = [C.POINTER(C.c_int)] * 3
     L.dexsim_set_step_impl.argtypes = [C.c_int]
@@ -145,6 +151,8 @@ def lib():
     L.dexsim_step_next_reset.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, C.POINTER(DexsimStepIO), vp]
     L.dexsim_rollout.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, i32, i32,
                                  C.POINTER(DexsimRolloutIO), vp]
+    L.dexsim_rollout_record.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, i32, i32,
+                                        C.POINTER(DexsimRolloutIO), C.POINTER(DexsimTrajectory), vp]
     L.dexsim_fill_policy_actions.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, vp, vp]
     L.dexsim_fill_normal.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, i32, C.c_float, vp, vp]
     L.dexsim_pack_env.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimStepIO), i64, i32, vp, vp]
@@ -172,6 +180,7 @@ def lib():
     assert L.dexsim_sizeof_step_io() == C.sizeof(DexsimStepIO)
     assert L.dexsim_sizeof_rollout_io() == C.sizeof(DexsimRolloutIO)
     assert L.dexsim_sizeof_episode_record() == C.sizeof(DexsimEpisodeRecord) == 32
+    assert L.dexsim_sizeof_trajectory() == C.sizeof(DexsimTrajectory)
     _ = i64
     _lib = L
     return L

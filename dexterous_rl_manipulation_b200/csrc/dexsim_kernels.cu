@@ -707,13 +707,42 @@ finish_reset_kernel(const DexsimState st, const DexsimParams p, const DexsimGrou
 }
 
 // ---- fused rollout ------------------------------------------------------------------------------------
+// Row t of a recorded rollout (DexsimTrajectory), stored from registers in three parts so that nothing of it stays live
+// across the step: the action as the policy produced it, the step's outcome, and the observation once the step and a
+// possible reset are done.  Every store of a warp is one 128-byte line of one row.
+__device__ __forceinline__ void record_action(const DexsimTrajectory& tr, int64_t ld, int t, int64_t i, const float* a) {
+    if (!tr.action) return;
+    float* out = tr.action + (int64_t)t * NJ * ld + i;
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) out[j * ld] = a[j];
+}
+
+__device__ __forceinline__ void record_outcome(const DexsimTrajectory& tr, int64_t ld, int t, int64_t i, const StepResult& r,
+                                               bool done) {
+    const int64_t at = (int64_t)t * ld + i;
+    tr.reward[at] = (float)r.total;
+    tr.terminated[at] = r.terminated ? 1 : 0;
+    tr.truncated[at] = r.truncated ? 1 : 0;
+    tr.finished[at] = done ? 1 : 0;
+}
+
+__device__ __forceinline__ void record_obs(const DexsimTrajectory& tr, int64_t ld, int t, int64_t i, const EnvRegs& e) {
+    float* out = tr.obs + (int64_t)t * DEXSIM_OBS * ld + i;
+#pragma unroll
+    for (int row = 0; row < DEXSIM_OBS; ++row) out[row * ld] = obs_entry(e, row);
+}
+
 constexpr int ROLLOUT_MIN_BLOCKS = 2;
 constexpr int ROLLOUT_THREADS = 256;      // CTA shape of the fused rollout for large batches (x MIN_BLOCKS resident CTAs per SM)
-template <bool DENSE, bool LEARNER>
+// REC: record every step into the trajectory (dexsim_rollout_record), passed as the one element of `traj`.  The REC =
+// false instantiations take no trajectory at all, so their parameter list -- and their code -- is what it was before
+// recording existed.
+template <bool DENSE, bool LEARNER, bool REC, typename... Traj>
 __global__ void __launch_bounds__(ROLLOUT_THREADS, ROLLOUT_MIN_BLOCKS)
 rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
                const uint16_t* __restrict__ group_of_env, const int k_steps, const int policy_kind,
-               const DexsimRolloutIO rio) {
+               const DexsimRolloutIO rio, const Traj... traj) {
+    static_assert(sizeof...(Traj) == (REC ? 1 : 0), "a recording rollout takes one DexsimTrajectory");
     const float* __restrict__ actions = rio.actions;
     const float* __restrict__ dyn_noise = rio.dyn_noise;
     int64_t* __restrict__ counters = rio.counters;
@@ -783,6 +812,7 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
             } else {
                 policy_action(p.seed, gid, episode, (uint32_t)e.sc, policy_kind, a);
             }
+            if constexpr (REC) record_action(traj..., ld, t, i, a);     // the policy's action, before dynamics noise
             if (dyn_noise) {                               // pre-drawn, already scaled by sigma
 #pragma unroll
                 for (int j = 0; j < NJ; ++j)
@@ -822,6 +852,7 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
             epstats_push(es, e.sc - 1, r.n_c);
             if (rio.hist && rio.step_base + t < rio.hist_steps) rio.hist[(rio.step_base + t) * ld + i] = (uint8_t)r.n_c;
             const bool done = r.terminated || r.truncated || (p.loop_max_steps > 0 && e.sc >= p.loop_max_steps);
+            if constexpr (REC) record_outcome(traj..., ld, t, i, r, done);
             if (done) {
                 if (LEARNER) lbest = -INFINITY;              // policy.reset() before the next episode
                 EpisodeLog log;
@@ -829,12 +860,14 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
                 log.capacity = rio.ep_log_capacity; log.t_end = (uint32_t)(rio.step_base + t);
                 if (rio.one_episode) {          // run_episode semantics: stop here, the caller resets
                     finish_episode(e, p, gid, episode, ep_return, es, r.terminated, r.n_c, cnt, rs, &log);
+                    if constexpr (REC) record_obs(traj..., ld, t, i, e);   // the terminal observation
                     break;
                 }
                 finish_and_reset(e, p, grp, gid, episode, ep_return, es, r.terminated, r.n_c, cnt, rs,
                                  size, mass, friction, &log);
                 params_dirty = true;
             }
+            if constexpr (REC) record_obs(traj..., ld, t, i, e);       // after the auto-reset, as step() returns it
         }
         store_env_full(st, i, e);
         st.episode[i] = episode;
@@ -943,7 +976,7 @@ static int query_device(DeviceInfo& d) {
     if (err != cudaSuccess) return -(int)err;
     err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&d.step_ctas, step_kernel<true, false, false, false>, STEP_THREADS, 0);
     if (err != cudaSuccess) return -(int)err;
-    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&d.rollout_ctas, rollout_kernel<true, false>, ROLLOUT_THREADS, 0);
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&d.rollout_ctas, rollout_kernel<true, false, false>, ROLLOUT_THREADS, 0);
     if (err != cudaSuccess) return -(int)err;
     d.valid = true;
     return 0;
@@ -1334,6 +1367,7 @@ int dexsim_sizeof_group(void) { return (int)sizeof(DexsimGroup); }
 int dexsim_sizeof_step_io(void) { return (int)sizeof(DexsimStepIO); }
 int dexsim_sizeof_rollout_io(void) { return (int)sizeof(DexsimRolloutIO); }
 int dexsim_sizeof_episode_record(void) { return (int)sizeof(DexsimEpisodeRecord); }
+int dexsim_sizeof_trajectory(void) { return (int)sizeof(DexsimTrajectory); }
 
 int dexsim_device_info(int* sm_count, int* step_ctas_per_sm, int* rollout_ctas_per_sm) {
     DeviceInfo di;
@@ -1406,9 +1440,10 @@ int dexsim_step_next_reset(const DexsimState* st, const DexsimParams* p, const D
     return launch_step(st, p, groups, group_of_env, io, (cudaStream_t)stream, nullptr, 0.0, /*next=*/true);
 }
 
-int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
-                   const uint16_t* group_of_env, int32_t k_steps, int32_t policy_kind, const DexsimRolloutIO* rio,
-                   void* stream) {
+// dexsim_rollout (traj == NULL) and dexsim_rollout_record
+static int rollout_launch(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups, const uint16_t* group_of_env,
+                          int32_t k_steps, int32_t policy_kind, const DexsimRolloutIO* rio, const DexsimTrajectory* traj,
+                          void* stream) {
     int rc = check_state(st);
     if (rc) return rc;
     rc = check_params(p, true, groups, st->ep_return != nullptr);
@@ -1422,6 +1457,21 @@ int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGro
     if ((rio->counters || rio->ep_log) && !st->ep_return) return DEXSIM_E_NULL;   // labels need the per-env history summary
     if (rio->ep_log && (!rio->ep_log_count || rio->ep_log_capacity < 0)) return DEXSIM_E_NULL;
     if (rio->hist && rio->hist_steps < 0) return DEXSIM_E_SIZE;
+    // small batches with an in-kernel policy: 5 lanes per env (dexsim_rollout_split.cuh); the crossover with the
+    // one-thread-per-env kernel was measured between 4k and 16k envs on B200 (DESIGN.md 5.2).  Only the one-thread-per-env
+    // kernel records a trajectory.
+    const bool split_ok = (rio->flags & DEXSIM_ROLLOUT_NO_DYN_NOISE) && !rio->dyn_noise && st->ep_return != nullptr &&
+                          (policy_kind == DEXSIM_POLICY_RANDOM || policy_kind == DEXSIM_POLICY_HEURISTIC);
+    if (traj) {
+        if (!traj->obs || !traj->reward || !traj->terminated || !traj->truncated || !traj->finished ||
+            (!traj->action && policy_kind != DEXSIM_POLICY_EXTERNAL))
+            return DEXSIM_E_NULL;
+        if (k_steps > traj->capacity) return DEXSIM_E_SIZE;
+        if (!aligned16(traj->obs) || !aligned16(traj->action) || !aligned16(traj->reward) || !aligned16(traj->terminated) ||
+            !aligned16(traj->truncated) || !aligned16(traj->finished))
+            return DEXSIM_E_ALIGN;
+        if (split_ok && g_rollout_impl == 2) return DEXSIM_E_PARAM;
+    }
     if (st->n == 0) return 0;
     DeviceInfo di;
     rc = device_info_cached(di);
@@ -1438,20 +1488,25 @@ int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGro
         ? (size_t)G * (sizeof(DexsimGroup) + DEXSIM_NCOUNTERS * sizeof(unsigned long long) + 2 * sizeof(double)) : 0;
     cudaStream_t s = (cudaStream_t)stream;
     const bool dense = p->reward_type == 1, learner = policy_kind == DEXSIM_POLICY_LEARNER;
-    // small batches with an in-kernel policy: 5 lanes per env (dexsim_rollout_split.cuh); the crossover with the
-    // one-thread-per-env kernel was measured between 4k and 16k envs on B200 (DESIGN.md 5.2)
-    const bool split_ok = (rio->flags & DEXSIM_ROLLOUT_NO_DYN_NOISE) && !rio->dyn_noise && st->ep_return != nullptr &&
-                          (policy_kind == DEXSIM_POLICY_RANDOM || policy_kind == DEXSIM_POLICY_HEURISTIC);
-    if (split_ok && g_rollout_impl != 1 && (g_rollout_impl == 2 || st->n <= 8192)) {
+    // the one-thread-per-env kernel, recording (one trailing DexsimTrajectory) or not (none)
+    auto launch_thread_kernel = [&](const auto&... tr) {
+        constexpr bool REC = sizeof...(tr) == 1;
+        if (dense && learner) rollout_kernel<true, true, REC><<<(int)blocks, threads, smem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio, tr...);
+        else if (dense) rollout_kernel<true, false, REC><<<(int)blocks, threads, smem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio, tr...);
+        else if (learner) rollout_kernel<false, true, REC><<<(int)blocks, threads, smem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio, tr...);
+        else rollout_kernel<false, false, REC><<<(int)blocks, threads, smem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio, tr...);
+    };
+    if (split_ok && !traj && g_rollout_impl != 1 && (g_rollout_impl == 2 || st->n <= 8192)) {
         const int64_t warps_needed = (st->n + SPLIT_ENVS_PER_WARP - 1) / SPLIT_ENVS_PER_WARP;
         const int64_t sblocks = (warps_needed * 32 + SPLIT_THREADS - 1) / SPLIT_THREADS;
         if (sblocks > 0x7FFFFFFFll) return DEXSIM_E_SIZE;
         if (dense) rollout_split_kernel<true><<<(int)sblocks, SPLIT_THREADS, 0, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio);
         else rollout_split_kernel<false><<<(int)sblocks, SPLIT_THREADS, 0, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio);
-    } else if (dense && learner) rollout_kernel<true, true><<<(int)blocks, threads, smem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio);
-    else if (dense) rollout_kernel<true, false><<<(int)blocks, threads, smem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio);
-    else if (learner) rollout_kernel<false, true><<<(int)blocks, threads, smem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio);
-    else rollout_kernel<false, false><<<(int)blocks, threads, smem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio);
+    } else if (traj) {
+        launch_thread_kernel(*traj);
+    } else {
+        launch_thread_kernel();
+    }
     rc = cuda_rc(cudaGetLastError());
     if (rc) return rc;
     if (rio->ep_log && rio->hist && rio->ep_log_capacity > 0) {
@@ -1461,6 +1516,19 @@ int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGro
         rc = cuda_rc(cudaGetLastError());
     }
     return rc;
+}
+
+int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                   const uint16_t* group_of_env, int32_t k_steps, int32_t policy_kind, const DexsimRolloutIO* rio,
+                   void* stream) {
+    return rollout_launch(st, p, groups, group_of_env, k_steps, policy_kind, rio, nullptr, stream);
+}
+
+int dexsim_rollout_record(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                          const uint16_t* group_of_env, int32_t k_steps, int32_t policy_kind, const DexsimRolloutIO* rio,
+                          const DexsimTrajectory* traj, void* stream) {
+    if (!traj) return DEXSIM_E_NULL;
+    return rollout_launch(st, p, groups, group_of_env, k_steps, policy_kind, rio, traj, stream);
 }
 
 int dexsim_pack_env(const DexsimState* st, const DexsimStepIO* io, int64_t index, int32_t after_reset, double* out64,

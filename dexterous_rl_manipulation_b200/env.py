@@ -264,6 +264,7 @@ class BatchedManipulationEnv:
         self._step_final_obs = self._ptr(self._final_obs)
         # filled on first use: pinned host buffers (a batched env pins none it does not use), the rollout's optional outputs
         self._action_pin = self._pack_host = self._ep_log = self._ep_log_count = self._hist = self._learner_mean = None
+        self._traj, self._traj_rows, self._traj_has_action = None, 0, False
         self._h_slots, self._host_keepalive = {}, {}
         self._step_out = None
         if not self.single:
@@ -999,6 +1000,37 @@ class BatchedManipulationEnv:
         self._hist = torch.zeros(int(steps), self.ld, dtype=torch.uint8, device=self.device)
         self._hist_steps = int(steps)
 
+    def enable_trajectory(self, steps):
+        """Allocate device buffers for ``steps`` rows of per-step trajectory that every later ``rollout()`` of at most
+        that many steps fills as it steps (``dexsim_rollout_record``); ``trajectory`` returns them.  Row t of a call
+        holds what the (t+1)-th step would return from ``step()`` on a same-step auto-reset env: the observation after
+        the step and a possible reset, the float32 reward, ``terminated`` / ``truncated``, ``finished`` (the loop bound
+        included) and the policy's action before dynamics noise.  The buffers take ``steps x num_envs x 247`` bytes:
+        about 13 GB for 1 Mi envs x 50 steps.  A recording rollout always runs the one-thread-per-env kernel."""
+        k, ld, dev = int(steps), self.ld, self.device
+        if k < 1:
+            raise ValueError("steps must be >= 1")
+        z = lambda *shape, dtype=torch.float32: torch.zeros(*shape, dtype=dtype, device=dev)
+        self._traj = {"obs": z(k, 45, ld), "action": z(k, 15, ld), "reward": z(k, ld), "terminated": z(k, ld, dtype=torch.uint8),
+                      "truncated": z(k, ld, dtype=torch.uint8), "finished": z(k, ld, dtype=torch.uint8)}
+        self._traj_rows, self._traj_has_action = 0, False
+
+    @property
+    def trajectory(self):
+        """The rows the last ``rollout()`` recorded, as batch-first views of the device buffers: ``obs`` [k, n, 45],
+        ``action`` [k, n, 15] (absent after ``policy="external"``: the caller holds the actions), ``reward`` [k, n]
+        float32 and ``terminated`` / ``truncated`` / ``finished`` [k, n] bool.  With ``one_episode=True`` an env's rows
+        after the step that ended its episode are not written.  The next ``rollout()`` overwrites them."""
+        if self._traj is None:
+            raise RuntimeError("enable_trajectory() first")
+        k, n, tr = self._traj_rows, self.num_envs, self._traj
+        out = {"obs": tr["obs"][:k, :, :n].transpose(1, 2), "reward": tr["reward"][:k, :n]}
+        if self._traj_has_action:
+            out["action"] = tr["action"][:k, :, :n].transpose(1, 2)
+        for name in ("terminated", "truncated", "finished"):
+            out[name] = tr[name][:k, :n].view(torch.bool)
+        return out
+
     def enable_learner(self, learning_rate=0.01, exploration_noise=0.3, action_clip_range=0.5):
         """One independent SimpleLearner per env (policies/simple_learner.py:27-47): ``learner_mean``
         [num_envs, 15] starts at zero, ``learner_best`` at -inf; ``rollout(policy="learner")`` trains them."""
@@ -1037,7 +1069,9 @@ class BatchedManipulationEnv:
         ``one_episode=True``: every env stops at the end of its first episode and is left un-reset
         (run_episode / evaluate_episode semantics); otherwise finished episodes auto-reset.
         Not available in ``autoreset_mode="next_step"``: the fused rollout resets in the same step, and an episode a
-        step() left pending would be counted twice."""
+        step() left pending would be counted twice.
+        After ``enable_trajectory(steps)`` the call also records every step (``trajectory``); ``k_steps`` must not exceed
+        ``steps``."""
         if self._next_step:
             raise NotImplementedError("rollout() resets finished episodes in the same step; it does not support "
                                       "autoreset_mode='next_step'")
@@ -1085,9 +1119,17 @@ class BatchedManipulationEnv:
             so, sd = self._group_sigma if self._group_cfgs is not None else (0.0, self.dynamics_noise_std)
             no_noise = not np.any(np.asarray(sd, dtype=np.float64) > 0.0)
             rio.flags = _L.ROLLOUT_NO_DYN_NOISE if no_noise else 0
-            _lib.check(self._lib.dexsim_rollout(
-                C.byref(self._state), C.byref(p), self._ptr(self._groups_dev), self._ptr(self._goe), int(k_steps), kind,
-                C.byref(rio), self._stream()), "dexsim_rollout")
+            args = (C.byref(self._state), C.byref(p), self._ptr(self._groups_dev), self._ptr(self._goe), int(k_steps), kind,
+                    C.byref(rio))
+            if self._traj is None:
+                _lib.check(self._lib.dexsim_rollout(*args, self._stream()), "dexsim_rollout")
+            else:
+                tr = self._traj
+                traj = _lib.DexsimTrajectory(tr["obs"].data_ptr(), None if kind == _L.POLICY_EXTERNAL else tr["action"].data_ptr(),
+                                             tr["reward"].data_ptr(), tr["terminated"].data_ptr(), tr["truncated"].data_ptr(),
+                                             tr["finished"].data_ptr(), tr["obs"].shape[0])
+                _lib.check(self._lib.dexsim_rollout_record(*args, C.byref(traj), self._stream()), "dexsim_rollout_record")
+                self._traj_rows, self._traj_has_action = int(k_steps), kind != _L.POLICY_EXTERNAL
             self._rollout_steps += int(k_steps)
             self._spawned = True
         return self.counters, self.ret_sums

@@ -221,7 +221,8 @@ int         dexsim_set_step_impl(int impl);
 int         dexsim_set_step_tile(int tile);
 /* Which fused-rollout kernel dexsim_rollout uses: 0 = auto (the 5-lanes-per-env kernel for small batches with an
  * in-kernel policy and no dynamics noise, else one thread per env), 1 = one thread per env, 2 = 5 lanes per env
- * whenever eligible.  Identical results; for tests and profiling.  Process-wide. */
+ * whenever eligible (dexsim_rollout_record then refuses an eligible call: it records with one thread per env only).
+ * Identical results; for tests and profiling.  Process-wide. */
 int         dexsim_set_rollout_impl(int impl);
 
 /* ---- reset: replaces DexterousManipulationEnv.reset, envs/manipulation_env.py:124-182 ------ */
@@ -333,6 +334,41 @@ typedef struct DexsimRolloutIO {
 int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
                    const uint16_t* group_of_env, int32_t k_steps, int32_t policy_kind,
                    const DexsimRolloutIO* rio, void* stream);
+
+/* Per-step trajectory of a rollout (dexsim_rollout_record): device arrays of `capacity` rows, row t holding step t of
+ * the call for every env, laid out [row, field, ld] like the state (247 bytes per env and row). */
+typedef struct DexsimTrajectory {
+    float*   obs;          /* [capacity, 45, ld] */
+    float*   action;       /* [capacity, 15, ld], or NULL = not recorded (allowed with DEXSIM_POLICY_EXTERNAL only) */
+    float*   reward;       /* [capacity, ld] */
+    uint8_t* terminated;   /* [capacity, ld] 0/1 */
+    uint8_t* truncated;    /* [capacity, ld] 0/1 */
+    uint8_t* finished;     /* [capacity, ld] 0/1 */
+    int64_t  capacity;     /* rows */
+} DexsimTrajectory;
+int dexsim_sizeof_trajectory(void);
+
+/* dexsim_rollout that also records every env-step into `traj` -- the transitions behind behaviour-cloning or offline-RL
+ * datasets and per-step analysis, without giving up the in-kernel policy.  Same arguments as dexsim_rollout plus `traj`;
+ * every other output equals what dexsim_rollout produces.  Row t (0 <= t < k_steps) of the call holds what the (t+1)-th
+ * step would return from dexsim_step with same-step auto-reset:
+ *   - obs: all 45 entries after the step and after a possible auto-reset (the observation dexsim_step leaves in st->obs);
+ *   - reward: float32 of the float64 total, as DexsimStepIO.reward; terminated, truncated;
+ *   - finished: the episode ended at this step, the loop bound (p->loop_max_steps) included (DexsimStepIO.finished);
+ *   - action: the policy's action before dynamics noise (for DEXSIM_POLICY_LEARNER after its exploration noise and
+ *     clip) -- what a dexsim_step caller passes as io->action, the noise passed separately.
+ * With rio->one_episode, the row of the step that ends an env's episode holds the terminal observation (the env is not
+ * reset) and its later rows are not written.  Every call writes rows 0 .. k_steps-1 (whatever rio->step_base is) and
+ * overwrites the previous call's; columns n .. ld-1 are not written.  A recording call always runs the one-thread-per-env
+ * kernel.
+ * Returns, before anything touches the device: DEXSIM_E_NULL when traj or one of its arrays is NULL (action only when
+ * policy_kind != DEXSIM_POLICY_EXTERNAL); DEXSIM_E_SIZE when k_steps > traj->capacity; DEXSIM_E_ALIGN when an array is
+ * not 16-byte aligned; DEXSIM_E_PARAM when dexsim_set_rollout_impl(2) would force the 5-lanes-per-env kernel; and every
+ * error of dexsim_rollout.
+ * Available since ABI 5 without a version bump (no struct or signature changed): look the symbol up to detect it. */
+int dexsim_rollout_record(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                          const uint16_t* group_of_env, int32_t k_steps, int32_t policy_kind,
+                          const DexsimRolloutIO* rio, const DexsimTrajectory* traj, void* stream);
 
 /* ---- single-env read-back: everything the reference's step()/reset() return for env `index`, packed into
  *      64 float64 on the device (one launch + one small D2H instead of a dozen scalar reads):

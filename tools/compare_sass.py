@@ -6,8 +6,9 @@ Runs ``cuobjdump -sass`` on both files, splits the listing per kernel and demang
 encoding words, comments and line information are dropped, so two kernels compare equal when their instruction text
 is the same.  A kernel template that gained a trailing template argument keeps its old instantiations' names only once
 that argument is removed: ``--strip-last-arg`` names such templates (default: step_tma_kernel and step_kernel), and a
-trailing ``false`` argument of them is stripped from NEW's names -- NEW's ``true`` instantiations stay distinct and are
-reported as new.  Prints one line per kernel (identical / changed / new / removed) and a summary; exits 1 when a kernel
+trailing ``false`` argument of them is stripped from a NEW name that OLD lacks when OLD has the stripped name (so a
+template that already had the argument in OLD is compared as it is) -- NEW's ``true`` instantiations stay distinct and
+are reported as new.  Prints one line per kernel (identical / changed / new / removed) and a summary; exits 1 when a kernel
 of OLD is changed or missing in NEW.
 """
 import argparse
@@ -71,7 +72,8 @@ def main():
     old = kernels(args.old)
     new = {}
     for name, body in kernels(args.new).items():
-        new[strip_last_arg(name, args.strip_last_arg)] = body
+        stripped = strip_last_arg(name, args.strip_last_arg)
+        new[stripped if name not in old and stripped in old else name] = body
     status = {}
     for name in sorted(set(old) | set(new)):
         if name not in new:
