@@ -105,7 +105,8 @@ EXPORTS = (
     "dexsim_version", "dexsim_error_string", "dexsim_sizeof_state", "dexsim_sizeof_params",
     "dexsim_sizeof_group", "dexsim_sizeof_step_io", "dexsim_sizeof_rollout_io", "dexsim_sizeof_episode_record",
     "dexsim_device_info", "dexsim_set_step_impl", "dexsim_set_step_tile", "dexsim_set_rollout_impl", "dexsim_reset_predrawn",
-    "dexsim_reset_philox", "dexsim_step", "dexsim_rollout", "dexsim_rollout_record", "dexsim_sizeof_trajectory",
+    "dexsim_reset_philox", "dexsim_step", "dexsim_rollout", "dexsim_rollout_record", "dexsim_rollout_record_final",
+    "dexsim_sizeof_trajectory",
     "dexsim_fill_policy_actions",
     "dexsim_fill_normal", "dexsim_classify_summary", "dexsim_step_host", "dexsim_pack_env", "dexsim_pack_env_tagged", "dexsim_step_single",
     "dexsim_step_final", "dexsim_step_host_final", "dexsim_step_next_reset",
@@ -153,6 +154,8 @@ def lib():
                                  C.POINTER(DexsimRolloutIO), vp]
     L.dexsim_rollout_record.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, i32, i32,
                                         C.POINTER(DexsimRolloutIO), C.POINTER(DexsimTrajectory), vp]
+    L.dexsim_rollout_record_final.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, i32, i32,
+                                              C.POINTER(DexsimRolloutIO), C.POINTER(DexsimTrajectory), vp, vp]
     L.dexsim_fill_policy_actions.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, vp, vp]
     L.dexsim_fill_normal.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, i32, C.c_float, vp, vp]
     L.dexsim_pack_env.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimStepIO), i64, i32, vp, vp]

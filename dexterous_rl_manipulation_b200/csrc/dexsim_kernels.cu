@@ -732,9 +732,41 @@ __device__ __forceinline__ void record_obs(const DexsimTrajectory& tr, int64_t l
     for (int row = 0; row < DEXSIM_OBS; ++row) out[row * ld] = obs_entry(e, row);
 }
 
+// A recording that also keeps the terminal observation of every episode it ends (dexsim_rollout_record_final):
+// `final_obs` [capacity, 45, ld] like tr.obs.  A distinct type, so that it instantiates rollout_kernel anew and the
+// DexsimTrajectory instantiations keep their code: for them record_final_obs is empty.
+struct TrajectoryFinal {
+    DexsimTrajectory tr;
+    float* final_obs;
+};
+
+__device__ __forceinline__ void record_action(const TrajectoryFinal& f, int64_t ld, int t, int64_t i, const float* a) {
+    record_action(f.tr, ld, t, i, a);
+}
+
+__device__ __forceinline__ void record_outcome(const TrajectoryFinal& f, int64_t ld, int t, int64_t i, const StepResult& r,
+                                               bool done) {
+    record_outcome(f.tr, ld, t, i, r, done);
+}
+
+__device__ __forceinline__ void record_obs(const TrajectoryFinal& f, int64_t ld, int t, int64_t i, const EnvRegs& e) {
+    record_obs(f.tr, ld, t, i, e);
+}
+
+__device__ __forceinline__ void record_final_obs(const DexsimTrajectory&, int64_t, int, int64_t, const EnvRegs&) {}
+
+// Called where the episode has ended and `e` still holds the state after the step, before any reset: the observation
+// dexsim_step_final returns in final_obs.  Only finished lanes store, so a warp's store covers its finished lanes.
+__device__ __forceinline__ void record_final_obs(const TrajectoryFinal& f, int64_t ld, int t, int64_t i, const EnvRegs& e) {
+    float* out = f.final_obs + (int64_t)t * DEXSIM_OBS * ld + i;
+#pragma unroll
+    for (int row = 0; row < DEXSIM_OBS; ++row) out[row * ld] = obs_entry(e, row);
+}
+
 constexpr int ROLLOUT_MIN_BLOCKS = 2;
 constexpr int ROLLOUT_THREADS = 256;      // CTA shape of the fused rollout for large batches (x MIN_BLOCKS resident CTAs per SM)
-// REC: record every step into the trajectory (dexsim_rollout_record), passed as the one element of `traj`.  The REC =
+// REC: record every step into the trajectory (dexsim_rollout_record), passed as the one element of `traj`: a
+// DexsimTrajectory, or a TrajectoryFinal that also records terminal observations (dexsim_rollout_record_final).  The REC =
 // false instantiations take no trajectory at all, so their parameter list -- and their code -- is what it was before
 // recording existed.
 template <bool DENSE, bool LEARNER, bool REC, typename... Traj>
@@ -742,7 +774,7 @@ __global__ void __launch_bounds__(ROLLOUT_THREADS, ROLLOUT_MIN_BLOCKS)
 rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
                const uint16_t* __restrict__ group_of_env, const int k_steps, const int policy_kind,
                const DexsimRolloutIO rio, const Traj... traj) {
-    static_assert(sizeof...(Traj) == (REC ? 1 : 0), "a recording rollout takes one DexsimTrajectory");
+    static_assert(sizeof...(Traj) == (REC ? 1 : 0), "a recording rollout takes one trajectory");
     const float* __restrict__ actions = rio.actions;
     const float* __restrict__ dyn_noise = rio.dyn_noise;
     int64_t* __restrict__ counters = rio.counters;
@@ -861,8 +893,10 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
                 if (rio.one_episode) {          // run_episode semantics: stop here, the caller resets
                     finish_episode(e, p, gid, episode, ep_return, es, r.terminated, r.n_c, cnt, rs, &log);
                     if constexpr (REC) record_obs(traj..., ld, t, i, e);   // the terminal observation
+                    if constexpr (REC) record_final_obs(traj..., ld, t, i, e);
                     break;
                 }
+                if constexpr (REC) record_final_obs(traj..., ld, t, i, e); // the terminal observation, before the reset
                 finish_and_reset(e, p, grp, gid, episode, ep_return, es, r.terminated, r.n_c, cnt, rs,
                                  size, mass, friction, &log);
                 params_dirty = true;
@@ -1440,10 +1474,10 @@ int dexsim_step_next_reset(const DexsimState* st, const DexsimParams* p, const D
     return launch_step(st, p, groups, group_of_env, io, (cudaStream_t)stream, nullptr, 0.0, /*next=*/true);
 }
 
-// dexsim_rollout (traj == NULL) and dexsim_rollout_record
+// dexsim_rollout (traj == NULL), dexsim_rollout_record (final_obs == NULL) and dexsim_rollout_record_final
 static int rollout_launch(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups, const uint16_t* group_of_env,
                           int32_t k_steps, int32_t policy_kind, const DexsimRolloutIO* rio, const DexsimTrajectory* traj,
-                          void* stream) {
+                          float* final_obs, void* stream) {
     int rc = check_state(st);
     if (rc) return rc;
     rc = check_params(p, true, groups, st->ep_return != nullptr);
@@ -1468,7 +1502,7 @@ static int rollout_launch(const DexsimState* st, const DexsimParams* p, const De
             return DEXSIM_E_NULL;
         if (k_steps > traj->capacity) return DEXSIM_E_SIZE;
         if (!aligned16(traj->obs) || !aligned16(traj->action) || !aligned16(traj->reward) || !aligned16(traj->terminated) ||
-            !aligned16(traj->truncated) || !aligned16(traj->finished))
+            !aligned16(traj->truncated) || !aligned16(traj->finished) || !aligned16(final_obs))
             return DEXSIM_E_ALIGN;
         if (split_ok && g_rollout_impl == 2) return DEXSIM_E_PARAM;
     }
@@ -1488,7 +1522,7 @@ static int rollout_launch(const DexsimState* st, const DexsimParams* p, const De
         ? (size_t)G * (sizeof(DexsimGroup) + DEXSIM_NCOUNTERS * sizeof(unsigned long long) + 2 * sizeof(double)) : 0;
     cudaStream_t s = (cudaStream_t)stream;
     const bool dense = p->reward_type == 1, learner = policy_kind == DEXSIM_POLICY_LEARNER;
-    // the one-thread-per-env kernel, recording (one trailing DexsimTrajectory) or not (none)
+    // the one-thread-per-env kernel, recording (one trailing DexsimTrajectory or TrajectoryFinal) or not (none)
     auto launch_thread_kernel = [&](const auto&... tr) {
         constexpr bool REC = sizeof...(tr) == 1;
         if (dense && learner) rollout_kernel<true, true, REC><<<(int)blocks, threads, smem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio, tr...);
@@ -1502,6 +1536,8 @@ static int rollout_launch(const DexsimState* st, const DexsimParams* p, const De
         if (sblocks > 0x7FFFFFFFll) return DEXSIM_E_SIZE;
         if (dense) rollout_split_kernel<true><<<(int)sblocks, SPLIT_THREADS, 0, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio);
         else rollout_split_kernel<false><<<(int)sblocks, SPLIT_THREADS, 0, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio);
+    } else if (traj && final_obs) {
+        launch_thread_kernel(TrajectoryFinal{*traj, final_obs});
     } else if (traj) {
         launch_thread_kernel(*traj);
     } else {
@@ -1521,14 +1557,21 @@ static int rollout_launch(const DexsimState* st, const DexsimParams* p, const De
 int dexsim_rollout(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
                    const uint16_t* group_of_env, int32_t k_steps, int32_t policy_kind, const DexsimRolloutIO* rio,
                    void* stream) {
-    return rollout_launch(st, p, groups, group_of_env, k_steps, policy_kind, rio, nullptr, stream);
+    return rollout_launch(st, p, groups, group_of_env, k_steps, policy_kind, rio, nullptr, nullptr, stream);
 }
 
 int dexsim_rollout_record(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
                           const uint16_t* group_of_env, int32_t k_steps, int32_t policy_kind, const DexsimRolloutIO* rio,
                           const DexsimTrajectory* traj, void* stream) {
     if (!traj) return DEXSIM_E_NULL;
-    return rollout_launch(st, p, groups, group_of_env, k_steps, policy_kind, rio, traj, stream);
+    return rollout_launch(st, p, groups, group_of_env, k_steps, policy_kind, rio, traj, nullptr, stream);
+}
+
+int dexsim_rollout_record_final(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                                const uint16_t* group_of_env, int32_t k_steps, int32_t policy_kind, const DexsimRolloutIO* rio,
+                                const DexsimTrajectory* traj, float* final_obs, void* stream) {
+    if (!traj || !final_obs) return DEXSIM_E_NULL;
+    return rollout_launch(st, p, groups, group_of_env, k_steps, policy_kind, rio, traj, final_obs, stream);
 }
 
 int dexsim_pack_env(const DexsimState* st, const DexsimStepIO* io, int64_t index, int32_t after_reset, double* out64,

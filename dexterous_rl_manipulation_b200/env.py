@@ -1000,31 +1000,41 @@ class BatchedManipulationEnv:
         self._hist = torch.zeros(int(steps), self.ld, dtype=torch.uint8, device=self.device)
         self._hist_steps = int(steps)
 
-    def enable_trajectory(self, steps):
+    def enable_trajectory(self, steps, final_observation=False):
         """Allocate device buffers for ``steps`` rows of per-step trajectory that every later ``rollout()`` of at most
         that many steps fills as it steps (``dexsim_rollout_record``); ``trajectory`` returns them.  Row t of a call
         holds what the (t+1)-th step would return from ``step()`` on a same-step auto-reset env: the observation after
         the step and a possible reset, the float32 reward, ``terminated`` / ``truncated``, ``finished`` (the loop bound
         included) and the policy's action before dynamics noise.  The buffers take ``steps x num_envs x 247`` bytes:
-        about 13 GB for 1 Mi envs x 50 steps.  A recording rollout always runs the one-thread-per-env kernel."""
+        about 13 GB for 1 Mi envs x 50 steps.  A recording rollout always runs the one-thread-per-env kernel.
+        ``final_observation=True`` also records, on every row where ``finished`` is set, the observation that ended the
+        episode, before its reset (``dexsim_rollout_record_final``): what ``info["final_observation"]`` of a
+        ``final_observation=True`` env's ``step()`` holds, and the ``next_obs`` of that transition.  Its buffer adds
+        ``steps x num_envs x 180`` bytes: 9.4 GB more for 1 Mi envs x 50 steps."""
         k, ld, dev = int(steps), self.ld, self.device
         if k < 1:
             raise ValueError("steps must be >= 1")
         z = lambda *shape, dtype=torch.float32: torch.zeros(*shape, dtype=dtype, device=dev)
         self._traj = {"obs": z(k, 45, ld), "action": z(k, 15, ld), "reward": z(k, ld), "terminated": z(k, ld, dtype=torch.uint8),
                       "truncated": z(k, ld, dtype=torch.uint8), "finished": z(k, ld, dtype=torch.uint8)}
+        if final_observation:
+            self._traj["final_observation"] = z(k, 45, ld)
         self._traj_rows, self._traj_has_action = 0, False
 
     @property
     def trajectory(self):
         """The rows the last ``rollout()`` recorded, as batch-first views of the device buffers: ``obs`` [k, n, 45],
         ``action`` [k, n, 15] (absent after ``policy="external"``: the caller holds the actions), ``reward`` [k, n]
-        float32 and ``terminated`` / ``truncated`` / ``finished`` [k, n] bool.  With ``one_episode=True`` an env's rows
-        after the step that ended its episode are not written.  The next ``rollout()`` overwrites them."""
+        float32 and ``terminated`` / ``truncated`` / ``finished`` [k, n] bool.  After
+        ``enable_trajectory(steps, final_observation=True)`` also ``final_observation`` [k, n, 45]: the observation that
+        ended the episode, valid where ``finished`` is True (other entries are not written).  With ``one_episode=True``
+        an env's rows after the step that ended its episode are not written.  The next ``rollout()`` overwrites them."""
         if self._traj is None:
             raise RuntimeError("enable_trajectory() first")
         k, n, tr = self._traj_rows, self.num_envs, self._traj
         out = {"obs": tr["obs"][:k, :, :n].transpose(1, 2), "reward": tr["reward"][:k, :n]}
+        if "final_observation" in tr:
+            out["final_observation"] = tr["final_observation"][:k, :, :n].transpose(1, 2)
         if self._traj_has_action:
             out["action"] = tr["action"][:k, :, :n].transpose(1, 2)
         for name in ("terminated", "truncated", "finished"):
@@ -1070,7 +1080,8 @@ class BatchedManipulationEnv:
         (run_episode / evaluate_episode semantics); otherwise finished episodes auto-reset.
         Not available in ``autoreset_mode="next_step"``: the fused rollout resets in the same step, and an episode a
         step() left pending would be counted twice.
-        After ``enable_trajectory(steps)`` the call also records every step (``trajectory``); ``k_steps`` must not exceed
+        After ``enable_trajectory(steps)`` the call also records every step (``trajectory``), with
+        ``final_observation=True`` the terminal observation of every episode it ends too; ``k_steps`` must not exceed
         ``steps``."""
         if self._next_step:
             raise NotImplementedError("rollout() resets finished episodes in the same step; it does not support "
@@ -1128,7 +1139,11 @@ class BatchedManipulationEnv:
                 traj = _lib.DexsimTrajectory(tr["obs"].data_ptr(), None if kind == _L.POLICY_EXTERNAL else tr["action"].data_ptr(),
                                              tr["reward"].data_ptr(), tr["terminated"].data_ptr(), tr["truncated"].data_ptr(),
                                              tr["finished"].data_ptr(), tr["obs"].shape[0])
-                _lib.check(self._lib.dexsim_rollout_record(*args, C.byref(traj), self._stream()), "dexsim_rollout_record")
+                if "final_observation" in tr:
+                    _lib.check(self._lib.dexsim_rollout_record_final(*args, C.byref(traj), tr["final_observation"].data_ptr(),
+                                                                     self._stream()), "dexsim_rollout_record_final")
+                else:
+                    _lib.check(self._lib.dexsim_rollout_record(*args, C.byref(traj), self._stream()), "dexsim_rollout_record")
                 self._traj_rows, self._traj_has_action = int(k_steps), kind != _L.POLICY_EXTERNAL
             self._rollout_steps += int(k_steps)
             self._spawned = True

@@ -221,7 +221,8 @@ int         dexsim_set_step_impl(int impl);
 int         dexsim_set_step_tile(int tile);
 /* Which fused-rollout kernel dexsim_rollout uses: 0 = auto (the 5-lanes-per-env kernel for small batches with an
  * in-kernel policy and no dynamics noise, else one thread per env), 1 = one thread per env, 2 = 5 lanes per env
- * whenever eligible (dexsim_rollout_record then refuses an eligible call: it records with one thread per env only).
+ * whenever eligible (dexsim_rollout_record and dexsim_rollout_record_final then refuse an eligible call: they record with
+ * one thread per env only).
  * Identical results; for tests and profiling.  Process-wide. */
 int         dexsim_set_rollout_impl(int impl);
 
@@ -369,6 +370,22 @@ int dexsim_sizeof_trajectory(void);
 int dexsim_rollout_record(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
                           const uint16_t* group_of_env, int32_t k_steps, int32_t policy_kind,
                           const DexsimRolloutIO* rio, const DexsimTrajectory* traj, void* stream);
+
+/* dexsim_rollout_record that also records the terminal observation of every episode the call ends -- the `next_obs` an
+ * offline-RL learner bootstraps from at truncation, which traj->obs does not hold on those rows (it holds the first
+ * observation of the next episode).  `final_obs` is a device float32 array [traj->capacity, 45, ld], laid out like
+ * traj->obs.  For every (t, i) with traj->finished[t][i] == 1 (the loop bound included), column i of row t holds all 45
+ * observation entries of env i after step t and before its auto-reset: bit for bit what dexsim_step_final returns in
+ * final_obs for the same step (Gymnasium's info["final_observation"]).  With rio->one_episode the ending row's final_obs
+ * equals its traj->obs row.  Nothing else of final_obs is written: not the entries of unfinished (t, i), not columns
+ * n .. ld-1, not rows k_steps .., not an env's rows after a one_episode stop.  Rows are indexed by the call's step t, as
+ * in traj.  Every other output equals what dexsim_rollout_record produces with the same arguments.
+ * Returns, before anything touches the device: DEXSIM_E_NULL when final_obs is NULL; DEXSIM_E_ALIGN when it is not
+ * 16-byte aligned; and every error of dexsim_rollout_record (DEXSIM_E_PARAM under dexsim_set_rollout_impl(2) included).
+ * Available since ABI 5 without a version bump: look the symbol up to detect it. */
+int dexsim_rollout_record_final(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                                const uint16_t* group_of_env, int32_t k_steps, int32_t policy_kind,
+                                const DexsimRolloutIO* rio, const DexsimTrajectory* traj, float* final_obs, void* stream);
 
 /* ---- single-env read-back: everything the reference's step()/reset() return for env `index`, packed into
  *      64 float64 on the device (one launch + one small D2H instead of a dozen scalar reads):
