@@ -75,7 +75,10 @@ DEXSIM_D double clip_f64(double x, double lo, double hi) {
 //   sq > thr^2 (1 + 2^-50)  =>  sqrt(sq) > thr                           =>  no contact
 // (thr^2 itself carries one rounding, 2^-53, absorbed by the 2^-50 margins).  Only inside that band --
 // relative width 2^-49, the "contact branch" -- is the square root evaluated; the decision is
-// bit-identical to the reference's everywhere.  Likewise min_i RN(sqrt(sq_i)) == RN(sqrt(min_i sq_i)),
+// bit-identical to the reference's for every threshold (0, negative, thr^2 underflowing or overflowing, inf, NaN) on the
+// domain stepping produces: fingertips and object positions lie on the float32 grid (multiples of 2^-149), so sq is 0
+// or >= 2^-298 (or inf / NaN from such inputs).  tests/test_contact_boundary.py puts fingers in the band and on
+// d == thr exactly, through this function and split_contact (dexsim_rollout_split.cuh).  Likewise min_i RN(sqrt(sq_i)) == RN(sqrt(min_i sq_i)),
 // so the dense reward needs one square root, not five.
 // One finger of the test below (shared by update_contacts and the warp-cooperative reset): returns the contact bit,
 // sq = squared fingertip-object distance.
