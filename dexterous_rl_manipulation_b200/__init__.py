@@ -21,6 +21,7 @@ if not ("-m" in _argv and __name__ + ".build" in _argv):
     _lib.lib()
 
 from .env import BatchedManipulationEnv, Box  # noqa: E402
+from .policy import MlpPolicy  # noqa: E402
 from . import distributed  # noqa: E402
 from .curriculum import BatchedCurriculumDriver, CurriculumScheduler  # noqa: E402
 from . import evaluation  # noqa: E402
@@ -30,7 +31,7 @@ from .training import run_episodes_batched  # noqa: E402
 DexterousManipulationEnv = BatchedManipulationEnv   # the reference's class name, for drop-in imports
 
 __all__ = [
-    "BatchedManipulationEnv", "DexterousManipulationEnv", "Box", "CurriculumConfig", "group_from_config",
+    "BatchedManipulationEnv", "DexterousManipulationEnv", "Box", "MlpPolicy", "CurriculumConfig", "group_from_config",
     "group_table", "classify_summary", "classify_counts", "run_episodes_batched", "evaluation", "training", "BatchedCurriculumDriver", "CurriculumScheduler", "DexsimError", "distributed", "LABELS_METRICS", "LABELS_TAXONOMY",
     "LABEL_NONE", "NCOUNTERS", "CNT_EPISODES", "CNT_SUCCESSES", "CNT_SUM_STEPS", "CNT_SUM_FINAL_CONTACTS",
     "CNT_LABEL_METRICS", "CNT_LABEL_TAXONOMY", "CNT_VAR_TIES", "CNT_SUM_STEPS_SQ",

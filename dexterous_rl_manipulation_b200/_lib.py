@@ -30,6 +30,8 @@ SCHED_WORDS = 64
 STEP_REVERSE_TILES = 1
 STEP_HOST_ALL_ROWS = 2
 ROLLOUT_NO_DYN_NOISE = 1
+ACT_RELU, ACT_TANH = 0, 1
+MLP_MAX_WIDTH = 64
 
 # value strings of FailureType (evaluation/metrics.py:15-22) / FailureMode
 # (evaluation/failure_taxonomy.py:14-26) in enum declaration order = device label codes
@@ -94,6 +96,11 @@ class DexsimTrajectory(C.Structure):
                 ("truncated", C.c_void_p), ("finished", C.c_void_p), ("capacity", C.c_int64)]
 
 
+class DexsimMlpPolicy(C.Structure):
+    _fields_ = [("params", C.c_void_p), ("num_hidden", C.c_int32), ("hidden", C.c_int32 * 2), ("activation", C.c_int32),
+                ("action_std", C.c_void_p)]
+
+
 class DexsimEpisodeSummary(C.Structure):
     _fields_ = [("success", C.c_int32), ("episode_steps", C.c_int32), ("num_contacts", C.c_int32),
                 ("final_contacts", C.c_int32), ("hist_len", C.c_int32), ("max_count", C.c_int32),
@@ -106,7 +113,7 @@ EXPORTS = (
     "dexsim_sizeof_group", "dexsim_sizeof_step_io", "dexsim_sizeof_rollout_io", "dexsim_sizeof_episode_record",
     "dexsim_device_info", "dexsim_set_step_impl", "dexsim_set_step_tile", "dexsim_set_rollout_impl", "dexsim_reset_predrawn",
     "dexsim_reset_philox", "dexsim_step", "dexsim_rollout", "dexsim_rollout_record", "dexsim_rollout_record_final",
-    "dexsim_sizeof_trajectory",
+    "dexsim_sizeof_trajectory", "dexsim_sizeof_mlp_policy", "dexsim_rollout_mlp", "dexsim_mlp_policy_mean",
     "dexsim_fill_policy_actions",
     "dexsim_fill_normal", "dexsim_classify_summary", "dexsim_step_host", "dexsim_pack_env", "dexsim_pack_env_tagged", "dexsim_step_single",
     "dexsim_step_final", "dexsim_step_host_final", "dexsim_step_next_reset",
@@ -139,7 +146,8 @@ def lib():
     L.dexsim_error_string.restype = C.c_char_p
     L.dexsim_error_string.argtypes = [C.c_int]
     for name in ("dexsim_sizeof_state", "dexsim_sizeof_params", "dexsim_sizeof_group", "dexsim_sizeof_step_io",
-                 "dexsim_sizeof_rollout_io", "dexsim_sizeof_episode_record", "dexsim_sizeof_trajectory"):
+                 "dexsim_sizeof_rollout_io", "dexsim_sizeof_episode_record", "dexsim_sizeof_trajectory",
+                 "dexsim_sizeof_mlp_policy"):
         getattr(L, name).restype = C.c_int
     L.dexsim_device_info.argtypes = [C.POINTER(C.c_int)] * 3
     L.dexsim_set_step_impl.argtypes = [C.c_int]
@@ -156,6 +164,9 @@ def lib():
                                         C.POINTER(DexsimRolloutIO), C.POINTER(DexsimTrajectory), vp]
     L.dexsim_rollout_record_final.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, i32, i32,
                                               C.POINTER(DexsimRolloutIO), C.POINTER(DexsimTrajectory), vp, vp]
+    L.dexsim_rollout_mlp.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, i32, C.POINTER(DexsimRolloutIO),
+                                     C.POINTER(DexsimMlpPolicy), C.POINTER(DexsimTrajectory), vp, vp]
+    L.dexsim_mlp_policy_mean.argtypes = [C.POINTER(DexsimMlpPolicy), vp, i64, i64, vp, vp]
     L.dexsim_fill_policy_actions.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, vp, vp]
     L.dexsim_fill_normal.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, i32, C.c_float, vp, vp]
     L.dexsim_pack_env.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimStepIO), i64, i32, vp, vp]
@@ -184,6 +195,7 @@ def lib():
     assert L.dexsim_sizeof_rollout_io() == C.sizeof(DexsimRolloutIO)
     assert L.dexsim_sizeof_episode_record() == C.sizeof(DexsimEpisodeRecord) == 32
     assert L.dexsim_sizeof_trajectory() == C.sizeof(DexsimTrajectory)
+    assert L.dexsim_sizeof_mlp_policy() == C.sizeof(DexsimMlpPolicy)
     _ = i64
     _lib = L
     return L

@@ -763,18 +763,205 @@ __device__ __forceinline__ void record_final_obs(const TrajectoryFinal& f, int64
     for (int row = 0; row < DEXSIM_OBS; ++row) out[row * ld] = obs_entry(e, row);
 }
 
+// ---- MLP policy (dexsim_rollout_mlp, dexsim_mlp_policy_mean) -------------------------------------------------------
+// The packed torch-layout parameters are staged once per CTA into shared memory, transposed and zero-padded so that the
+// weights of 16 consecutive neurons for one input are four warp-uniform (broadcast) 128-bit loads:
+//   W1T [45][h1p]  b1 [h1p]  (W2T [h1][h2p]  b2 [h2p])  W3T [h_last][16]  b3 [16]  std [16]      (hNp = hN rounded up to 16)
+// A thread keeps 16 accumulators and walks the inputs in ascending order, so every neuron's FMA chain is the one
+// include/dexsim.h specifies.  The first layer reads its inputs from registers (the env state, plus regenerated noise);
+// the last hidden layer feeds each finished block of 16 straight into the 15 output accumulators.  Only a second hidden
+// layer needs per-thread scratch for the first layer's outputs: h1 floats per thread, in shared memory, thread-major.
+constexpr int MLP_BLOCK = 16;
+constexpr int DEXSIM_POLICY_MLP_KIND = 4;        // policy_kind the MLP instantiations receive (dexsim_rollout rejects it)
+
+struct MlpArgs {             // validated DexsimMlpPolicy + the shared-memory layout (offsets in floats)
+    const float* params;
+    const float* action_std;
+    int32_t nh, h1, h2, act;
+    int32_t h1p, h2p, o_b1, o_w2, o_b2, o_w3, o_b3, o_std, words;
+    int32_t scratch_off;     // float offset of the per-thread scratch (second hidden layer only)
+};
+
+__device__ __forceinline__ float mlp_act(float y, int act) {
+    if (act == DEXSIM_ACT_TANH) return tanhf(y);
+    return (y > 0.0f || y != y) ? y : 0.0f;
+}
+
+// Cooperative copy of the packed parameters into the padded transposed layout; every thread of the CTA calls it.
+__device__ __forceinline__ void mlp_stage(const MlpArgs& m, float* sw) {
+    const int hl = m.nh == 2 ? m.h2 : m.h1;
+    // packed offsets (torch layout)
+    const int p_b1 = m.h1 * NOBS, p_w2 = p_b1 + m.h1;
+    const int p_b2 = p_w2 + (m.nh == 2 ? m.h2 * m.h1 : 0), p_w3 = p_b2 + (m.nh == 2 ? m.h2 : 0);
+    const int p_b3 = p_w3 + NJ * hl;
+    for (int w = threadIdx.x; w < m.words; w += blockDim.x) {
+        float v = 0.0f;
+        if (w < m.o_b1) {                                  // W1T[i][j] = W1[j][i]
+            const int i = w / m.h1p, j = w % m.h1p;
+            if (j < m.h1) v = m.params[j * NOBS + i];
+        } else if (w < m.o_w2) {
+            const int j = w - m.o_b1;
+            if (j < m.h1) v = m.params[p_b1 + j];
+        } else if (w < m.o_b2) {                           // W2T[i][j] = W2[j][i]
+            const int i = (w - m.o_w2) / m.h2p, j = (w - m.o_w2) % m.h2p;
+            if (j < m.h2) v = m.params[p_w2 + j * m.h1 + i];
+        } else if (w < m.o_w3) {
+            const int j = w - m.o_b2;
+            if (j < m.h2) v = m.params[p_b2 + j];
+        } else if (w < m.o_b3) {                           // W3T[i][j] = W3[j][i]
+            const int i = (w - m.o_w3) / MLP_BLOCK, j = (w - m.o_w3) % MLP_BLOCK;
+            if (j < NJ) v = m.params[p_w3 + j * hl + i];
+        } else if (w < m.o_std) {
+            const int j = w - m.o_b3;
+            if (j < NJ) v = m.params[p_b3 + j];
+        } else {
+            const int j = w - m.o_std;
+            if (j < NJ && m.action_std) v = m.action_std[j];
+        }
+        sw[w] = v;
+    }
+}
+
+// acc[k] = fmaf(w[k], x, acc[k]) for the 16 weights at `w` (16-byte aligned shared memory, the same for the whole warp)
+__device__ __forceinline__ void mlp_fma16(const float* w, const float x, float* acc) {
+#pragma unroll
+    for (int q = 0; q < MLP_BLOCK / 4; ++q) {
+        const float4 v = reinterpret_cast<const float4*>(w)[q];
+        acc[4 * q + 0] = __fmaf_rn(v.x, x, acc[4 * q + 0]);
+        acc[4 * q + 1] = __fmaf_rn(v.y, x, acc[4 * q + 1]);
+        acc[4 * q + 2] = __fmaf_rn(v.z, x, acc[4 * q + 2]);
+        acc[4 * q + 3] = __fmaf_rn(v.w, x, acc[4 * q + 3]);
+    }
+}
+
+// A finished block of the last hidden layer, acc[k] = pre-activation of neuron jb + k, into the output accumulators.
+__device__ __forceinline__ void mlp_block_out(const MlpArgs& m, const float* sw, const float* b, int jb, int h, float* acc,
+                                              float* o) {
+#pragma unroll
+    for (int k = 0; k < MLP_BLOCK; ++k) {
+        if (jb + k < h) mlp_fma16(sw + m.o_w3 + (jb + k) * MLP_BLOCK, mlp_act(__fadd_rn(acc[k], b[jb + k]), m.act), o);
+    }
+}
+
+// The network's mean for one env.  `X` provides the 45 inputs in chunks of four: X::chunk(b, x) fills x[0..3] with
+// inputs 4b .. 4b+3 (b = 0..11; the last chunk has one).  `scr`: this thread's scratch, stride `ss` floats.
+template <typename X>
+__device__ __forceinline__ void mlp_mean(const MlpArgs& m, const float* sw, float* scr, int ss, const X& xin, float* mean) {
+    float o[MLP_BLOCK];
+#pragma unroll
+    for (int j = 0; j < MLP_BLOCK; ++j) o[j] = 0.0f;
+    for (int jb = 0; jb < m.h1p; jb += MLP_BLOCK) {
+        float acc[MLP_BLOCK];
+#pragma unroll
+        for (int k = 0; k < MLP_BLOCK; ++k) acc[k] = 0.0f;
+#pragma unroll
+        for (int b = 0; b < (NOBS + 3) / 4; ++b) {
+            float x[4];
+            xin.chunk(b, x);
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+                if (4 * b + k < NOBS) mlp_fma16(sw + (4 * b + k) * m.h1p + jb, x[k], acc);
+        }
+        if (m.nh == 1) {
+            mlp_block_out(m, sw, sw + m.o_b1, jb, m.h1, acc, o);
+        } else {
+#pragma unroll
+            for (int k = 0; k < MLP_BLOCK; ++k)
+                if (jb + k < m.h1) scr[(jb + k) * ss] = mlp_act(__fadd_rn(acc[k], sw[m.o_b1 + jb + k]), m.act);
+        }
+    }
+    if (m.nh == 2) {
+        for (int jb = 0; jb < m.h2p; jb += MLP_BLOCK) {
+            float acc[MLP_BLOCK];
+#pragma unroll
+            for (int k = 0; k < MLP_BLOCK; ++k) acc[k] = 0.0f;
+#pragma unroll 4
+            for (int i = 0; i < m.h1; ++i) mlp_fma16(sw + m.o_w2 + i * m.h2p + jb, scr[i * ss], acc);
+            mlp_block_out(m, sw, sw + m.o_b2, jb, m.h2, acc, o);
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) mean[j] = __fadd_rn(o[j], sw[m.o_b3 + j]);
+}
+
+// Inputs of the rollout: the observation of the env's registers, plus the stream-3 noise of its current state where
+// sigma > 0 -- what the step kernel writes to noisy_obs (one Philox block = four observation rows).
+struct MlpEnvInput {
+    const EnvRegs& e;
+    uint64_t seed;
+    uint32_t gid, episode;
+    float sigma;
+    __device__ __forceinline__ void chunk(const int b, float* x) const {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) x[k] = 4 * b + k < NOBS ? obs_entry(e, 4 * b + k) : 0.0f;
+        if (sigma > 0.0f) {
+            const U4 o = rng_block(seed, gid, episode, (uint32_t)e.sc, STREAM_OBS, (uint32_t)b);
+            float z[4];
+            normal_pair(o.x, o.y, z[0], z[1]);
+            normal_pair(o.z, o.w, z[2], z[3]);
+#pragma unroll
+            for (int k = 0; k < 4; ++k) x[k] = __fadd_rn(x[k], __fmul_rn(sigma, z[k]));
+        }
+    }
+};
+
+// Inputs of dexsim_mlp_policy_mean: column i of an [45, ld] array
+struct MlpColumnInput {
+    const float* obs;
+    int64_t ld, i;
+    __device__ __forceinline__ void chunk(const int b, float* x) const {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) x[k] = 4 * b + k < NOBS ? obs[(4 * b + k) * ld + i] : 0.0f;
+    }
+};
+
+__global__ void __launch_bounds__(256)
+mlp_mean_kernel(const MlpArgs m, const float* __restrict__ obs, const int64_t n, const int64_t ld, float* __restrict__ out) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float* sw = reinterpret_cast<float*>(smem_raw);
+    mlp_stage(m, sw);
+    __syncthreads();
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    float mean[NJ];
+    mlp_mean(m, sw, sw + m.scratch_off + threadIdx.x, (int)blockDim.x, MlpColumnInput{obs, ld, i}, mean);
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) out[j * ld + i] = mean[j];
+}
+
+// The rollout kernel receives the policy as the first element of its trailing pack: (MlpArgs) or (MlpArgs, trajectory).
+// The record_* calls forward past it.
+template <typename Tr> __device__ __forceinline__ void record_action(const MlpArgs&, const Tr& tr, int64_t ld, int t, int64_t i,
+                                                                     const float* a) { record_action(tr, ld, t, i, a); }
+template <typename Tr> __device__ __forceinline__ void record_outcome(const MlpArgs&, const Tr& tr, int64_t ld, int t, int64_t i,
+                                                                      const StepResult& r, bool done) {
+    record_outcome(tr, ld, t, i, r, done);
+}
+template <typename Tr> __device__ __forceinline__ void record_obs(const MlpArgs&, const Tr& tr, int64_t ld, int t, int64_t i,
+                                                                  const EnvRegs& e) { record_obs(tr, ld, t, i, e); }
+template <typename Tr> __device__ __forceinline__ void record_final_obs(const MlpArgs&, const Tr& tr, int64_t ld, int t,
+                                                                        int64_t i, const EnvRegs& e) {
+    record_final_obs(tr, ld, t, i, e);
+}
+
+template <typename... T> struct first_is_mlp : std::false_type {};
+template <typename... T> struct first_is_mlp<MlpArgs, T...> : std::true_type {};
+template <typename... T> __device__ __forceinline__ const MlpArgs& mlp_of(const MlpArgs& m, const T&...) { return m; }
+
 constexpr int ROLLOUT_MIN_BLOCKS = 2;
 constexpr int ROLLOUT_THREADS = 256;      // CTA shape of the fused rollout for large batches (x MIN_BLOCKS resident CTAs per SM)
 // REC: record every step into the trajectory (dexsim_rollout_record), passed as the one element of `traj`: a
 // DexsimTrajectory, or a TrajectoryFinal that also records terminal observations (dexsim_rollout_record_final).  The REC =
 // false instantiations take no trajectory at all, so their parameter list -- and their code -- is what it was before
-// recording existed.
+// recording existed.  The MLP policy (dexsim_rollout_mlp) comes first in the pack when present: (MlpArgs[, trajectory]).
 template <bool DENSE, bool LEARNER, bool REC, typename... Traj>
 __global__ void __launch_bounds__(ROLLOUT_THREADS, ROLLOUT_MIN_BLOCKS)
 rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
                const uint16_t* __restrict__ group_of_env, const int k_steps, const int policy_kind,
                const DexsimRolloutIO rio, const Traj... traj) {
-    static_assert(sizeof...(Traj) == (REC ? 1 : 0), "a recording rollout takes one trajectory");
+    constexpr bool MLP = first_is_mlp<Traj...>::value;
+    static_assert(sizeof...(Traj) == (REC ? 1 : 0) + (MLP ? 1 : 0), "a recording rollout takes one trajectory");
+    static_assert(!(MLP && LEARNER), "the MLP and the learner never share a launch");
     const float* __restrict__ actions = rio.actions;
     const float* __restrict__ dyn_noise = rio.dyn_noise;
     int64_t* __restrict__ counters = rio.counters;
@@ -792,6 +979,13 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
             reinterpret_cast<uint32_t*>(sh_groups)[w] = reinterpret_cast<const uint32_t*>(groups)[w];
         for (int w = threadIdx.x; w < G * DEXSIM_NCOUNTERS; w += blockDim.x) sh_cnt[w] = 0ull;
         for (int w = threadIdx.x; w < G * 2; w += blockDim.x) sh_rs[w] = 0.0;
+        __syncthreads();
+    }
+    float* sh_mlp = nullptr;                      // the MLP's weights, after the group table (16-byte aligned)
+    if constexpr (MLP) {
+        const size_t groups_bytes = staged ? (size_t)G * (sizeof(DexsimGroup) + DEXSIM_NCOUNTERS * 8 + 16) : 0;
+        sh_mlp = reinterpret_cast<float*>(smem_raw + ((groups_bytes + 15) & ~(size_t)15));
+        mlp_stage(mlp_of(traj...), sh_mlp);
         __syncthreads();
     }
     const DexsimGroup* gtab = staged ? sh_groups : groups;
@@ -828,7 +1022,19 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
 
         for (int t = 0; t < k_steps; ++t) {
             float a[NJ];
-            if (LEARNER) {                                 // SimpleLearner.select_action, policies/simple_learner.py:60-69
+            if constexpr (MLP) {                           // dexsim_rollout_mlp: the observation this state returns from step()
+                const MlpArgs& m = mlp_of(traj...);
+                mlp_mean(m, sh_mlp, sh_mlp + m.scratch_off + threadIdx.x, (int)blockDim.x,
+                         MlpEnvInput{e, p.seed, gid, episode, grp.sigma_obs}, a);
+                if (m.action_std) {
+                    float z[NJ];
+                    normal_rows<NJ>(p.seed, gid, episode, (uint32_t)e.sc, STREAM_LEARNER_ACT, 1.0f, z);
+#pragma unroll
+                    for (int j = 0; j < NJ; ++j) a[j] = __fadd_rn(a[j], __fmul_rn(sh_mlp[m.o_std + j], z[j]));
+                }
+#pragma unroll
+                for (int j = 0; j < NJ; ++j) a[j] = clip_f32(a[j], -1.0f, 1.0f);
+            } else if (LEARNER) {                          // SimpleLearner.select_action, policies/simple_learner.py:60-69
                 float nz[NJ];
                 if (rio.learner_act_noise) {
 #pragma unroll
@@ -1474,17 +1680,48 @@ int dexsim_step_next_reset(const DexsimState* st, const DexsimParams* p, const D
     return launch_step(st, p, groups, group_of_env, io, (cudaStream_t)stream, nullptr, 0.0, /*next=*/true);
 }
 
-// dexsim_rollout (traj == NULL), dexsim_rollout_record (final_obs == NULL) and dexsim_rollout_record_final
+// DexsimMlpPolicy -> MlpArgs (shape checks and the shared-memory layout of mlp_stage); no device call
+static int mlp_args(const DexsimMlpPolicy* pol, MlpArgs& m) {
+    if (!pol || !pol->params) return DEXSIM_E_NULL;
+    if (pol->num_hidden != 1 && pol->num_hidden != 2) return DEXSIM_E_PARAM;
+    for (int l = 0; l < pol->num_hidden; ++l)
+        if (pol->hidden[l] < 1 || pol->hidden[l] > DEXSIM_MLP_MAX_WIDTH) return DEXSIM_E_PARAM;
+    if (pol->activation != DEXSIM_ACT_RELU && pol->activation != DEXSIM_ACT_TANH) return DEXSIM_E_PARAM;
+    if (!aligned16(pol->params) || !aligned16(pol->action_std)) return DEXSIM_E_ALIGN;
+    const auto pad = [](int h) { return (h + MLP_BLOCK - 1) / MLP_BLOCK * MLP_BLOCK; };
+    m.params = pol->params; m.action_std = pol->action_std;
+    m.nh = pol->num_hidden; m.h1 = pol->hidden[0]; m.h2 = m.nh == 2 ? pol->hidden[1] : 0; m.act = pol->activation;
+    m.h1p = pad(m.h1); m.h2p = m.nh == 2 ? pad(m.h2) : 0;
+    m.o_b1 = NOBS * m.h1p;
+    m.o_w2 = m.o_b1 + m.h1p;
+    m.o_b2 = m.o_w2 + m.h1 * m.h2p;
+    m.o_w3 = m.o_b2 + m.h2p;
+    m.o_b3 = m.o_w3 + (m.nh == 2 ? m.h2 : m.h1) * MLP_BLOCK;
+    m.o_std = m.o_b3 + MLP_BLOCK;
+    m.words = m.o_std + MLP_BLOCK;
+    m.scratch_off = m.words;
+    return 0;
+}
+
+// bytes of shared memory the MLP needs behind `base` bytes: weights + one scratch float per first-layer unit and thread
+static size_t mlp_smem(const MlpArgs& m, size_t base, int threads) {
+    return ((base + 15) & ~(size_t)15) + (size_t)m.words * 4 + (m.nh == 2 ? (size_t)m.h1 * threads * 4 : 0);
+}
+
+// dexsim_rollout (traj == NULL), dexsim_rollout_record (final_obs == NULL) and dexsim_rollout_record_final; with `mlp`
+// dexsim_rollout_mlp (policy_kind == DEXSIM_POLICY_MLP_KIND)
 static int rollout_launch(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups, const uint16_t* group_of_env,
                           int32_t k_steps, int32_t policy_kind, const DexsimRolloutIO* rio, const DexsimTrajectory* traj,
-                          float* final_obs, void* stream) {
+                          float* final_obs, void* stream, const MlpArgs* mlp = nullptr) {
     int rc = check_state(st);
     if (rc) return rc;
     rc = check_params(p, true, groups, st->ep_return != nullptr);
     if (rc) return rc;
     if (!rio) return DEXSIM_E_NULL;
     if (k_steps < 1) return DEXSIM_E_SIZE;
-    if (policy_kind < DEXSIM_POLICY_EXTERNAL || policy_kind > DEXSIM_POLICY_LEARNER) return DEXSIM_E_PARAM;
+    if ((policy_kind < DEXSIM_POLICY_EXTERNAL || policy_kind > DEXSIM_POLICY_LEARNER) &&
+        !(mlp && policy_kind == DEXSIM_POLICY_MLP_KIND))
+        return DEXSIM_E_PARAM;
     if (policy_kind == DEXSIM_POLICY_EXTERNAL && !rio->actions) return DEXSIM_E_NULL;
     if (policy_kind == DEXSIM_POLICY_LEARNER && (!rio->learner_mean || !rio->learner_best)) return DEXSIM_E_NULL;
     if (rio->ret_sums && !rio->counters) return DEXSIM_E_NULL;
@@ -1530,7 +1767,23 @@ static int rollout_launch(const DexsimState* st, const DexsimParams* p, const De
         else if (learner) rollout_kernel<false, true, REC><<<(int)blocks, threads, smem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio, tr...);
         else rollout_kernel<false, false, REC><<<(int)blocks, threads, smem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio, tr...);
     };
-    if (split_ok && !traj && g_rollout_impl != 1 && (g_rollout_impl == 2 || st->n <= 8192)) {
+    // the MLP policy: the one-thread-per-env kernel with the weights (and the second layer's scratch) in shared memory
+    auto launch_mlp_kernel = [&](const auto&... tr) {
+        constexpr bool REC = sizeof...(tr) == 1;
+        const auto kernel = dense ? rollout_kernel<true, false, REC, MlpArgs, std::decay_t<decltype(tr)>...>
+                                  : rollout_kernel<false, false, REC, MlpArgs, std::decay_t<decltype(tr)>...>;
+        const size_t msmem = mlp_smem(*mlp, smem, threads);
+        const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msmem);
+        if (e != cudaSuccess) return cuda_rc(e);
+        kernel<<<(int)blocks, threads, msmem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio, *mlp, tr...);
+        return 0;
+    };
+    if (mlp) {
+        rc = traj && final_obs ? launch_mlp_kernel(TrajectoryFinal{*traj, final_obs})
+           : traj              ? launch_mlp_kernel(*traj)
+                               : launch_mlp_kernel();
+        if (rc) return rc;
+    } else if (split_ok && !traj && g_rollout_impl != 1 && (g_rollout_impl == 2 || st->n <= 8192)) {
         const int64_t warps_needed = (st->n + SPLIT_ENVS_PER_WARP - 1) / SPLIT_ENVS_PER_WARP;
         const int64_t sblocks = (warps_needed * 32 + SPLIT_THREADS - 1) / SPLIT_THREADS;
         if (sblocks > 0x7FFFFFFFll) return DEXSIM_E_SIZE;
@@ -1572,6 +1825,36 @@ int dexsim_rollout_record_final(const DexsimState* st, const DexsimParams* p, co
                                 const DexsimTrajectory* traj, float* final_obs, void* stream) {
     if (!traj || !final_obs) return DEXSIM_E_NULL;
     return rollout_launch(st, p, groups, group_of_env, k_steps, policy_kind, rio, traj, final_obs, stream);
+}
+
+int dexsim_sizeof_mlp_policy(void) { return (int)sizeof(DexsimMlpPolicy); }
+
+int dexsim_rollout_mlp(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                       const uint16_t* group_of_env, int32_t k_steps, const DexsimRolloutIO* rio,
+                       const DexsimMlpPolicy* policy, const DexsimTrajectory* traj, float* final_obs, void* stream) {
+    MlpArgs m;
+    const int rc = mlp_args(policy, m);
+    if (rc) return rc;
+    if (final_obs && !traj) return DEXSIM_E_NULL;
+    if (rio && (rio->actions || rio->learner_mean || rio->learner_best || rio->learner_act_noise || rio->learner_upd_noise))
+        return DEXSIM_E_PARAM;
+    return rollout_launch(st, p, groups, group_of_env, k_steps, DEXSIM_POLICY_MLP_KIND, rio, traj, final_obs, stream, &m);
+}
+
+int dexsim_mlp_policy_mean(const DexsimMlpPolicy* policy, const float* obs, int64_t n, int64_t ld, float* out, void* stream) {
+    MlpArgs m;
+    const int rc = mlp_args(policy, m);
+    if (rc) return rc;
+    if (n < 0 || ld < n || ld % 32 != 0) return DEXSIM_E_SIZE;
+    if (n == 0) return 0;
+    if (!obs || !out) return DEXSIM_E_NULL;
+    const int64_t blocks = (n + 255) / 256;
+    if (blocks > 0x7FFFFFFFll) return DEXSIM_E_SIZE;
+    const size_t smem = mlp_smem(m, 0, 256);
+    cudaError_t e = cudaFuncSetAttribute(mlp_mean_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return cuda_rc(e);
+    mlp_mean_kernel<<<(int)blocks, 256, smem, (cudaStream_t)stream>>>(m, obs, n, ld, out);
+    return cuda_rc(cudaGetLastError());
 }
 
 int dexsim_pack_env(const DexsimState* st, const DexsimStepIO* io, int64_t index, int32_t after_reset, double* out64,

@@ -20,6 +20,7 @@ import torch
 
 from . import _lib
 from .config import CurriculumConfig, group_table
+from .policy import MlpPolicy
 
 _L = _lib
 
@@ -1082,7 +1083,10 @@ class BatchedManipulationEnv:
         step() left pending would be counted twice.
         After ``enable_trajectory(steps)`` the call also records every step (``trajectory``), with
         ``final_observation=True`` the terminal observation of every episode it ends too; ``k_steps`` must not exceed
-        ``steps``."""
+        ``steps``.
+        ``policy`` may also be an ``MlpPolicy``: every env acts on the observation ``step()`` would return for its
+        current state (with the env's observation noise where its ``sigma_obs`` > 0), through the network, in the same
+        launch (``dexsim_rollout_mlp``); recorded actions are the policy's, before dynamics noise."""
         if self._next_step:
             raise NotImplementedError("rollout() resets finished episodes in the same step; it does not support "
                                       "autoreset_mode='next_step'")
@@ -1091,8 +1095,16 @@ class BatchedManipulationEnv:
         self._h_primed_slot = None
         if self._ep_return is None:
             raise RuntimeError("rollout() needs track_episodes=True (per-env history summaries)")
-        kind = {"external": _L.POLICY_EXTERNAL, "random": _L.POLICY_RANDOM, "heuristic": _L.POLICY_HEURISTIC,
-                "learner": _L.POLICY_LEARNER}[policy]
+        mlp = policy if isinstance(policy, MlpPolicy) else None
+        if mlp is not None:
+            if actions is not None or learner_act_noise is not None or learner_upd_noise is not None:
+                raise ValueError("an MlpPolicy rollout takes no actions and no learner noise")
+            if mlp.device != self.device:
+                raise ValueError(f"the policy lives on {mlp.device}, the env on {self.device}")
+            kind = None
+        else:
+            kind = {"external": _L.POLICY_EXTERNAL, "random": _L.POLICY_RANDOM, "heuristic": _L.POLICY_HEURISTIC,
+                    "learner": _L.POLICY_LEARNER}[policy]
         if kind == _L.POLICY_LEARNER and self._learner_mean is None:
             self.enable_learner()
         with torch.cuda.device(self.device):
@@ -1132,7 +1144,21 @@ class BatchedManipulationEnv:
             rio.flags = _L.ROLLOUT_NO_DYN_NOISE if no_noise else 0
             args = (C.byref(self._state), C.byref(p), self._ptr(self._groups_dev), self._ptr(self._goe), int(k_steps), kind,
                     C.byref(rio))
-            if self._traj is None:
+            if mlp is not None:
+                traj, fo = None, None
+                if self._traj is not None:
+                    tr = self._traj
+                    traj = _lib.DexsimTrajectory(tr["obs"].data_ptr(), tr["action"].data_ptr(), tr["reward"].data_ptr(),
+                                                 tr["terminated"].data_ptr(), tr["truncated"].data_ptr(),
+                                                 tr["finished"].data_ptr(), tr["obs"].shape[0])
+                    fo = tr["final_observation"].data_ptr() if "final_observation" in tr else None
+                _lib.check(self._lib.dexsim_rollout_mlp(
+                    C.byref(self._state), C.byref(p), self._ptr(self._groups_dev), self._ptr(self._goe), int(k_steps),
+                    C.byref(rio), C.byref(mlp._struct), None if traj is None else C.byref(traj), fo, self._stream()),
+                    "dexsim_rollout_mlp")
+                if traj is not None:
+                    self._traj_rows, self._traj_has_action = int(k_steps), True
+            elif self._traj is None:
                 _lib.check(self._lib.dexsim_rollout(*args, self._stream()), "dexsim_rollout")
             else:
                 tr = self._traj

@@ -387,6 +387,52 @@ int dexsim_rollout_record_final(const DexsimState* st, const DexsimParams* p, co
                                 const uint16_t* group_of_env, int32_t k_steps, int32_t policy_kind,
                                 const DexsimRolloutIO* rio, const DexsimTrajectory* traj, float* final_obs, void* stream);
 
+/* ---- observation-conditioned MLP policy inside the fused rollout --------------------------------------------------
+ * An MLP 45 -> h1 [-> h2] -> 15, one or two hidden layers of 1..64 units, every hidden layer with the same activation,
+ * a linear output layer.  `params`: device float32, 16-byte aligned, packed in torch's nn.Linear layout, contiguous:
+ * W1 [h1, 45], b1 [h1], (W2 [h2, h1], b2 [h2],) W3 [15, h_last], b3 [15].  The arithmetic is fixed so that a C
+ * reference reproduces it bit for bit (ReLU) or within tanhf's ulp error (tanh):
+ *   - neuron j of a layer: acc = 0; for every input i in ascending order acc = fmaf(W[j, i], x[i], acc);
+ *     y = acc + b[j] (one float32 addition);
+ *   - ReLU: y > 0 || y != y ? y : 0 (NaN propagates as in torch.relu);  tanh: the device tanhf (2 ulp);
+ *   - action a_j = clip(mean_j + std_j * z_j, -1, 1) (product and sum rounded separately), z the float32 N(0, 1) of
+ *     Philox stream 4 keyed by the step count BEFORE the step (dexsim_fill_normal(4, 15, 1.0) exposes it);
+ *     `action_std` NULL = deterministic policy, a = clip(mean).
+ * The input of a step is the observation dexsim_step would have returned for the env's current state: the 45
+ * observation entries, plus, where the env's group has sigma_obs > 0, the observation noise of stream 3 keyed by the
+ * current step count (bit for bit io->noisy_obs of that dexsim_step). */
+#define DEXSIM_ACT_RELU 0
+#define DEXSIM_ACT_TANH 1
+#define DEXSIM_MLP_MAX_WIDTH 64
+typedef struct DexsimMlpPolicy {
+    const float* params;       /* device, 16-byte aligned, packed as above */
+    int32_t      num_hidden;   /* 1 or 2 */
+    int32_t      hidden[2];    /* widths 1..64; hidden[1] ignored when num_hidden == 1 */
+    int32_t      activation;   /* DEXSIM_ACT_RELU or DEXSIM_ACT_TANH */
+    const float* action_std;   /* device float32 [15], 16-byte aligned, or NULL = deterministic */
+} DexsimMlpPolicy;
+int dexsim_sizeof_mlp_policy(void);
+
+/* dexsim_rollout / _record / _record_final with the actions produced by `policy` in the kernel.  Same arguments and
+ * outputs as those (traj NULL = no recording; final_obs needs traj); recorded actions are the policy's action before
+ * dynamics noise.  The weights are staged in shared memory per CTA; the call always runs the one-thread-per-env kernel.
+ * Returns, before anything touches the device: DEXSIM_E_NULL when policy, policy->params or (with final_obs) traj is
+ * NULL; DEXSIM_E_PARAM when num_hidden is not 1 or 2, a width is outside 1..64, the activation is unknown, or
+ * rio->actions / any learner field of rio is set; DEXSIM_E_ALIGN when params or action_std is not 16-byte aligned; and
+ * every error of dexsim_rollout / dexsim_rollout_record / dexsim_rollout_record_final.
+ * Available since ABI 5 without a version bump: look the symbol up to detect it. */
+int dexsim_rollout_mlp(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                       const uint16_t* group_of_env, int32_t k_steps, const DexsimRolloutIO* rio,
+                       const DexsimMlpPolicy* policy, const DexsimTrajectory* traj /* or NULL */,
+                       float* final_obs /* or NULL */, void* stream);
+
+/* The policy's mean (the network's output, no exploration, no clip) for n observation columns: obs device float32
+ * [45, ld] -> out [15, ld], the arithmetic of dexsim_rollout_mlp.  For log-probabilities of recorded actions and for
+ * checking the fused rollout.  Returns DEXSIM_E_NULL / E_PARAM / E_ALIGN for the policy as dexsim_rollout_mlp,
+ * DEXSIM_E_NULL for a NULL obs or out (n > 0), DEXSIM_E_SIZE when n < 0, ld < n or ld % 32 != 0. */
+int dexsim_mlp_policy_mean(const DexsimMlpPolicy* policy, const float* obs, int64_t n, int64_t ld, float* out,
+                           void* stream);
+
 /* ---- single-env read-back: everything the reference's step()/reset() return for env `index`, packed into
  *      64 float64 on the device (one launch + one small D2H instead of a dozen scalar reads):
  *      [0..44] obs (noisy_obs if given), 45 reward, 46 terminated, 47 truncated, 48 num_contacts, 49 step_count,
