@@ -101,6 +101,10 @@ class DexsimMlpPolicy(C.Structure):
                 ("action_std", C.c_void_p)]
 
 
+class DexsimPolicyRecord(C.Structure):
+    _fields_ = [("obs", C.c_void_p), ("raw_action", C.c_void_p), ("log_prob", C.c_void_p)]
+
+
 class DexsimEpisodeSummary(C.Structure):
     _fields_ = [("success", C.c_int32), ("episode_steps", C.c_int32), ("num_contacts", C.c_int32),
                 ("final_contacts", C.c_int32), ("hist_len", C.c_int32), ("max_count", C.c_int32),
@@ -114,6 +118,7 @@ EXPORTS = (
     "dexsim_device_info", "dexsim_set_step_impl", "dexsim_set_step_tile", "dexsim_set_rollout_impl", "dexsim_reset_predrawn",
     "dexsim_reset_philox", "dexsim_step", "dexsim_rollout", "dexsim_rollout_record", "dexsim_rollout_record_final",
     "dexsim_sizeof_trajectory", "dexsim_sizeof_mlp_policy", "dexsim_rollout_mlp", "dexsim_mlp_policy_mean",
+    "dexsim_sizeof_policy_record", "dexsim_rollout_mlp_record", "dexsim_gae",
     "dexsim_fill_policy_actions",
     "dexsim_fill_normal", "dexsim_classify_summary", "dexsim_step_host", "dexsim_pack_env", "dexsim_pack_env_tagged", "dexsim_step_single",
     "dexsim_step_final", "dexsim_step_host_final", "dexsim_step_next_reset",
@@ -147,7 +152,7 @@ def lib():
     L.dexsim_error_string.argtypes = [C.c_int]
     for name in ("dexsim_sizeof_state", "dexsim_sizeof_params", "dexsim_sizeof_group", "dexsim_sizeof_step_io",
                  "dexsim_sizeof_rollout_io", "dexsim_sizeof_episode_record", "dexsim_sizeof_trajectory",
-                 "dexsim_sizeof_mlp_policy"):
+                 "dexsim_sizeof_mlp_policy", "dexsim_sizeof_policy_record"):
         getattr(L, name).restype = C.c_int
     L.dexsim_device_info.argtypes = [C.POINTER(C.c_int)] * 3
     L.dexsim_set_step_impl.argtypes = [C.c_int]
@@ -166,6 +171,10 @@ def lib():
                                               C.POINTER(DexsimRolloutIO), C.POINTER(DexsimTrajectory), vp, vp]
     L.dexsim_rollout_mlp.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, i32, C.POINTER(DexsimRolloutIO),
                                      C.POINTER(DexsimMlpPolicy), C.POINTER(DexsimTrajectory), vp, vp]
+    L.dexsim_rollout_mlp_record.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp, i32,
+                                            C.POINTER(DexsimRolloutIO), C.POINTER(DexsimMlpPolicy),
+                                            C.POINTER(DexsimTrajectory), vp, C.POINTER(DexsimPolicyRecord), vp]
+    L.dexsim_gae.argtypes = [C.POINTER(DexsimTrajectory), i64, i64, i32, vp, vp, C.c_float, C.c_float, vp, vp, vp]
     L.dexsim_mlp_policy_mean.argtypes = [C.POINTER(DexsimMlpPolicy), vp, i64, i64, vp, vp]
     L.dexsim_fill_policy_actions.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, vp, vp]
     L.dexsim_fill_normal.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, i32, C.c_float, vp, vp]
@@ -196,6 +205,7 @@ def lib():
     assert L.dexsim_sizeof_episode_record() == C.sizeof(DexsimEpisodeRecord) == 32
     assert L.dexsim_sizeof_trajectory() == C.sizeof(DexsimTrajectory)
     assert L.dexsim_sizeof_mlp_policy() == C.sizeof(DexsimMlpPolicy)
+    assert L.dexsim_sizeof_policy_record() == C.sizeof(DexsimPolicyRecord)
     _ = i64
     _lib = L
     return L

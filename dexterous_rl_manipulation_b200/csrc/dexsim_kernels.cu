@@ -948,12 +948,90 @@ template <typename... T> struct first_is_mlp : std::false_type {};
 template <typename... T> struct first_is_mlp<MlpArgs, T...> : std::true_type {};
 template <typename... T> __device__ __forceinline__ const MlpArgs& mlp_of(const MlpArgs& m, const T&...) { return m; }
 
+// ---- behaviour-policy record (dexsim_rollout_mlp_record) --------------------------------------------------------------
+// A recording (DexsimTrajectory or TrajectoryFinal) plus what an on-policy learner needs of the policy that acted: the
+// network's input, the action before the clip and its log-density.  A distinct type, so that it instantiates
+// rollout_kernel anew and the existing MLP instantiations keep their code: for them the three hooks below are empty.
+// The log-density's constant c = float32(-sum_j log(double std_j) - 7.5 log(2 pi)) is computed once per CTA into the
+// padding slot std[15] of the staged weights (the mean never reads it).
+template <typename Tr> struct TrajectoryPolicy {
+    Tr tr;
+    DexsimPolicyRecord pr;
+};
+constexpr double LOG_2PI = 1.8378770664093453;   // double(log(2 pi)), the constant of include/dexsim.h
+
+template <typename Tr> __device__ __forceinline__ void record_action(const TrajectoryPolicy<Tr>& f, int64_t ld, int t, int64_t i,
+                                                                     const float* a) { record_action(f.tr, ld, t, i, a); }
+template <typename Tr> __device__ __forceinline__ void record_outcome(const TrajectoryPolicy<Tr>& f, int64_t ld, int t,
+                                                                      int64_t i, const StepResult& r, bool done) {
+    record_outcome(f.tr, ld, t, i, r, done);
+}
+template <typename Tr> __device__ __forceinline__ void record_obs(const TrajectoryPolicy<Tr>& f, int64_t ld, int t, int64_t i,
+                                                                  const EnvRegs& e) { record_obs(f.tr, ld, t, i, e); }
+template <typename Tr> __device__ __forceinline__ void record_final_obs(const TrajectoryPolicy<Tr>& f, int64_t ld, int t,
+                                                                        int64_t i, const EnvRegs& e) {
+    record_final_obs(f.tr, ld, t, i, e);
+}
+
+// The hooks take the rollout kernel's whole trailing pack, (MlpArgs) or (MlpArgs, recording), and do nothing unless the
+// recording is a TrajectoryPolicy.
+__device__ __forceinline__ void stage_log_prob_const(const MlpArgs&, float*) {}
+template <typename Tr> __device__ __forceinline__ void stage_log_prob_const(const MlpArgs&, const Tr&, float*) {}
+template <typename Tr> __device__ __forceinline__ void stage_log_prob_const(const MlpArgs& m, const TrajectoryPolicy<Tr>& f,
+                                                                            float* sw) {
+    if (!f.pr.log_prob) return;                  // uniform over the CTA: every thread returns or every thread syncs
+    if (threadIdx.x == 0) {
+        double s = 0.0;
+        for (int j = 0; j < NJ; ++j) s = __dadd_rn(s, log((double)sw[m.o_std + j]));
+        sw[m.o_std + NJ] = (float)__dsub_rn(-s, __dmul_rn(7.5, LOG_2PI));
+    }
+    __syncthreads();
+}
+
+// Row t of the record: the 45 inputs of the network (regenerated from the registers and stream 3, as the mean read them)
+// and the action before the clip.
+template <typename Tr> __device__ __forceinline__ void record_policy(const MlpArgs&, const Tr&, int64_t, int, int64_t,
+                                                                     const MlpEnvInput&, const float*) {}
+template <typename Tr> __device__ __forceinline__ void record_policy(const MlpArgs&, const TrajectoryPolicy<Tr>& f, int64_t ld,
+                                                                     int t, int64_t i, const MlpEnvInput& xin,
+                                                                     const float* raw) {
+    if (f.pr.obs) {
+        float* out = f.pr.obs + (int64_t)t * NOBS * ld + i;
+#pragma unroll
+        for (int b = 0; b < (NOBS + 3) / 4; ++b) {
+            float x[4];
+            xin.chunk(b, x);
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+                if (4 * b + k < NOBS) out[(4 * b + k) * ld] = x[k];
+        }
+    }
+    if (f.pr.raw_action) {
+        float* out = f.pr.raw_action + (int64_t)t * NJ * ld + i;
+#pragma unroll
+        for (int j = 0; j < NJ; ++j) out[j * ld] = raw[j];
+    }
+}
+
+// log N(raw; mean, diag(std^2)) = c - 0.5 sum_j z_j^2, the sum an ascending fmaf chain from 0
+template <typename Tr> __device__ __forceinline__ void record_log_prob(const MlpArgs&, const Tr&, int64_t, int, int64_t,
+                                                                       const float*, const float*) {}
+template <typename Tr> __device__ __forceinline__ void record_log_prob(const MlpArgs&, const TrajectoryPolicy<Tr>& f, int64_t ld,
+                                                                       int t, int64_t i, const float* z, const float* std16) {
+    if (!f.pr.log_prob) return;
+    float s = 0.0f;
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) s = __fmaf_rn(z[j], z[j], s);
+    f.pr.log_prob[(int64_t)t * ld + i] = __fmaf_rn(-0.5f, s, std16[NJ]);
+}
+
 constexpr int ROLLOUT_MIN_BLOCKS = 2;
 constexpr int ROLLOUT_THREADS = 256;      // CTA shape of the fused rollout for large batches (x MIN_BLOCKS resident CTAs per SM)
 // REC: record every step into the trajectory (dexsim_rollout_record), passed as the one element of `traj`: a
 // DexsimTrajectory, or a TrajectoryFinal that also records terminal observations (dexsim_rollout_record_final).  The REC =
 // false instantiations take no trajectory at all, so their parameter list -- and their code -- is what it was before
-// recording existed.  The MLP policy (dexsim_rollout_mlp) comes first in the pack when present: (MlpArgs[, trajectory]).
+// recording existed.  The MLP policy (dexsim_rollout_mlp) comes first in the pack when present: (MlpArgs[, trajectory]);
+// with dexsim_rollout_mlp_record the trajectory is a TrajectoryPolicy.
 template <bool DENSE, bool LEARNER, bool REC, typename... Traj>
 __global__ void __launch_bounds__(ROLLOUT_THREADS, ROLLOUT_MIN_BLOCKS)
 rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
@@ -987,6 +1065,7 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
         sh_mlp = reinterpret_cast<float*>(smem_raw + ((groups_bytes + 15) & ~(size_t)15));
         mlp_stage(mlp_of(traj...), sh_mlp);
         __syncthreads();
+        stage_log_prob_const(traj..., sh_mlp);
     }
     const DexsimGroup* gtab = staged ? sh_groups : groups;
     unsigned long long* cnt_base = staged ? sh_cnt : reinterpret_cast<unsigned long long*>(counters);
@@ -1031,7 +1110,9 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
                     normal_rows<NJ>(p.seed, gid, episode, (uint32_t)e.sc, STREAM_LEARNER_ACT, 1.0f, z);
 #pragma unroll
                     for (int j = 0; j < NJ; ++j) a[j] = __fadd_rn(a[j], __fmul_rn(sh_mlp[m.o_std + j], z[j]));
+                    if constexpr (REC) record_log_prob(traj..., ld, t, i, z, sh_mlp + m.o_std);
                 }
+                if constexpr (REC) record_policy(traj..., ld, t, i, MlpEnvInput{e, p.seed, gid, episode, grp.sigma_obs}, a);
 #pragma unroll
                 for (int j = 0; j < NJ; ++j) a[j] = clip_f32(a[j], -1.0f, 1.0f);
             } else if (LEARNER) {                          // SimpleLearner.select_action, policies/simple_learner.py:60-69
@@ -1130,6 +1211,31 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
         if (ret_sums)
             for (int w = threadIdx.x; w < G * 2; w += blockDim.x)
                 if (sh_rs[w] != 0.0) atomicAdd(&ret_sums[w], sh_rs[w]);
+    }
+}
+
+// ---- generalized advantage estimation over a recorded rollout (dexsim_gae) ------------------------------------------
+// One thread per env walks its rows backwards; every row read is coalesced across the warp.  The float32 arithmetic is
+// the one include/dexsim.h fixes, each operation rounded on its own, so that a NumPy float32 restatement matches it bit
+// for bit.  The advantage is a select at `finished`, not a product with 0, so a non-finite A_next stays in its episode.
+__global__ void __launch_bounds__(256)
+gae_kernel(const DexsimTrajectory tr, const int64_t n, const int64_t ld, const int k_steps, const float* __restrict__ values,
+           const float* __restrict__ final_values, const float gamma, const float lam, float* __restrict__ adv,
+           float* __restrict__ ret) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float gl = __fmul_rn(gamma, lam);
+    float a_next = 0.0f;
+    for (int t = k_steps - 1; t >= 0; --t) {
+        const int64_t at = (int64_t)t * ld + i;
+        const bool fin = tr.finished[at] != 0;
+        const float v = values[at];
+        const float nv = fin ? (tr.terminated[at] ? 0.0f : final_values[at]) : values[at + ld];
+        const float delta = __fsub_rn(__fadd_rn(tr.reward[at], __fmul_rn(gamma, nv)), v);
+        const float a = fin ? delta : __fadd_rn(delta, __fmul_rn(gl, a_next));
+        adv[at] = a;
+        ret[at] = __fadd_rn(a, v);
+        a_next = a;
     }
 }
 
@@ -1712,7 +1818,8 @@ static size_t mlp_smem(const MlpArgs& m, size_t base, int threads) {
 // dexsim_rollout_mlp (policy_kind == DEXSIM_POLICY_MLP_KIND)
 static int rollout_launch(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups, const uint16_t* group_of_env,
                           int32_t k_steps, int32_t policy_kind, const DexsimRolloutIO* rio, const DexsimTrajectory* traj,
-                          float* final_obs, void* stream, const MlpArgs* mlp = nullptr) {
+                          float* final_obs, void* stream, const MlpArgs* mlp = nullptr,
+                          const DexsimPolicyRecord* prec = nullptr) {
     int rc = check_state(st);
     if (rc) return rc;
     rc = check_params(p, true, groups, st->ep_return != nullptr);
@@ -1778,7 +1885,11 @@ static int rollout_launch(const DexsimState* st, const DexsimParams* p, const De
         kernel<<<(int)blocks, threads, msmem, s>>>(*st, *p, groups, group_of_env, k_steps, policy_kind, *rio, *mlp, tr...);
         return 0;
     };
-    if (mlp) {
+    if (mlp && prec) {
+        rc = final_obs ? launch_mlp_kernel(TrajectoryPolicy<TrajectoryFinal>{TrajectoryFinal{*traj, final_obs}, *prec})
+                       : launch_mlp_kernel(TrajectoryPolicy<DexsimTrajectory>{*traj, *prec});
+        if (rc) return rc;
+    } else if (mlp) {
         rc = traj && final_obs ? launch_mlp_kernel(TrajectoryFinal{*traj, final_obs})
            : traj              ? launch_mlp_kernel(*traj)
                                : launch_mlp_kernel();
@@ -1829,16 +1940,55 @@ int dexsim_rollout_record_final(const DexsimState* st, const DexsimParams* p, co
 
 int dexsim_sizeof_mlp_policy(void) { return (int)sizeof(DexsimMlpPolicy); }
 
-int dexsim_rollout_mlp(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
-                       const uint16_t* group_of_env, int32_t k_steps, const DexsimRolloutIO* rio,
-                       const DexsimMlpPolicy* policy, const DexsimTrajectory* traj, float* final_obs, void* stream) {
+// dexsim_rollout_mlp (prec == NULL) and dexsim_rollout_mlp_record: the checks of both, then rollout_launch's
+static int rollout_mlp(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups, const uint16_t* group_of_env,
+                       int32_t k_steps, const DexsimRolloutIO* rio, const DexsimMlpPolicy* policy,
+                       const DexsimTrajectory* traj, float* final_obs, const DexsimPolicyRecord* prec, void* stream) {
     MlpArgs m;
     const int rc = mlp_args(policy, m);
     if (rc) return rc;
     if (final_obs && !traj) return DEXSIM_E_NULL;
     if (rio && (rio->actions || rio->learner_mean || rio->learner_best || rio->learner_act_noise || rio->learner_upd_noise))
         return DEXSIM_E_PARAM;
-    return rollout_launch(st, p, groups, group_of_env, k_steps, DEXSIM_POLICY_MLP_KIND, rio, traj, final_obs, stream, &m);
+    if (prec) {
+        if (!aligned16(prec->obs) || !aligned16(prec->raw_action) || !aligned16(prec->log_prob)) return DEXSIM_E_ALIGN;
+        if (prec->log_prob && !policy->action_std) return DEXSIM_E_PARAM;   // a deterministic policy has no density
+    }
+    return rollout_launch(st, p, groups, group_of_env, k_steps, DEXSIM_POLICY_MLP_KIND, rio, traj, final_obs, stream, &m,
+                          prec);
+}
+
+int dexsim_rollout_mlp(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                       const uint16_t* group_of_env, int32_t k_steps, const DexsimRolloutIO* rio,
+                       const DexsimMlpPolicy* policy, const DexsimTrajectory* traj, float* final_obs, void* stream) {
+    return rollout_mlp(st, p, groups, group_of_env, k_steps, rio, policy, traj, final_obs, nullptr, stream);
+}
+
+int dexsim_sizeof_policy_record(void) { return (int)sizeof(DexsimPolicyRecord); }
+
+int dexsim_rollout_mlp_record(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                              const uint16_t* group_of_env, int32_t k_steps, const DexsimRolloutIO* rio,
+                              const DexsimMlpPolicy* policy, const DexsimTrajectory* traj, float* final_obs,
+                              const DexsimPolicyRecord* prec, void* stream) {
+    if (!traj || !prec) return DEXSIM_E_NULL;
+    return rollout_mlp(st, p, groups, group_of_env, k_steps, rio, policy, traj, final_obs, prec, stream);
+}
+
+int dexsim_gae(const DexsimTrajectory* traj, int64_t n, int64_t ld, int32_t k_steps, const float* values,
+               const float* final_values, float gamma, float lam, float* advantages, float* returns, void* stream) {
+    if (!traj || !traj->reward || !traj->terminated || !traj->finished || !values || !final_values || !advantages ||
+        !returns)
+        return DEXSIM_E_NULL;
+    if (n < 0 || ld < n || ld % 32 != 0 || k_steps < 1 || k_steps > traj->capacity) return DEXSIM_E_SIZE;
+    if (!aligned16(traj->reward) || !aligned16(traj->terminated) || !aligned16(traj->finished) || !aligned16(values) ||
+        !aligned16(final_values) || !aligned16(advantages) || !aligned16(returns))
+        return DEXSIM_E_ALIGN;
+    if (n == 0) return 0;
+    const int64_t blocks = (n + 255) / 256;
+    if (blocks > 0x7FFFFFFFll) return DEXSIM_E_SIZE;
+    gae_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(*traj, n, ld, k_steps, values, final_values, gamma, lam,
+                                                               advantages, returns);
+    return cuda_rc(cudaGetLastError());
 }
 
 int dexsim_mlp_policy_mean(const DexsimMlpPolicy* policy, const float* obs, int64_t n, int64_t ld, float* out, void* stream) {

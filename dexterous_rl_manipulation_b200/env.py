@@ -266,6 +266,7 @@ class BatchedManipulationEnv:
         # filled on first use: pinned host buffers (a batched env pins none it does not use), the rollout's optional outputs
         self._action_pin = self._pack_host = self._ep_log = self._ep_log_count = self._hist = self._learner_mean = None
         self._traj, self._traj_rows, self._traj_has_action = None, 0, False
+        self._traj_log_prob = self._traj_one_episode = False
         self._h_slots, self._host_keepalive = {}, {}
         self._step_out = None
         if not self.single:
@@ -1001,7 +1002,7 @@ class BatchedManipulationEnv:
         self._hist = torch.zeros(int(steps), self.ld, dtype=torch.uint8, device=self.device)
         self._hist_steps = int(steps)
 
-    def enable_trajectory(self, steps, final_observation=False):
+    def enable_trajectory(self, steps, final_observation=False, policy_record=False):
         """Allocate device buffers for ``steps`` rows of per-step trajectory that every later ``rollout()`` of at most
         that many steps fills as it steps (``dexsim_rollout_record``); ``trajectory`` returns them.  Row t of a call
         holds what the (t+1)-th step would return from ``step()`` on a same-step auto-reset env: the observation after
@@ -1011,7 +1012,12 @@ class BatchedManipulationEnv:
         ``final_observation=True`` also records, on every row where ``finished`` is set, the observation that ended the
         episode, before its reset (``dexsim_rollout_record_final``): what ``info["final_observation"]`` of a
         ``final_observation=True`` env's ``step()`` holds, and the ``next_obs`` of that transition.  Its buffer adds
-        ``steps x num_envs x 180`` bytes: 9.4 GB more for 1 Mi envs x 50 steps."""
+        ``steps x num_envs x 180`` bytes: 9.4 GB more for 1 Mi envs x 50 steps.
+        ``policy_record=True`` also records what the ``MlpPolicy`` that acted computed at every step
+        (``dexsim_rollout_mlp_record``): the network's input ``policy_obs`` (with the observation noise that reached it),
+        the action before the clip ``raw_action`` and its log-probability ``log_prob`` -- the behaviour-policy data of
+        on-policy training.  It adds ``steps x num_envs x 244`` bytes (12.8 GB for 1 Mi envs x 50 steps), and only an
+        ``MlpPolicy`` rollout can fill it: any other policy raises."""
         k, ld, dev = int(steps), self.ld, self.device
         if k < 1:
             raise ValueError("steps must be >= 1")
@@ -1020,7 +1026,10 @@ class BatchedManipulationEnv:
                       "truncated": z(k, ld, dtype=torch.uint8), "finished": z(k, ld, dtype=torch.uint8)}
         if final_observation:
             self._traj["final_observation"] = z(k, 45, ld)
+        if policy_record:
+            self._traj.update(policy_obs=z(k, 45, ld), raw_action=z(k, 15, ld), log_prob=z(k, ld))
         self._traj_rows, self._traj_has_action = 0, False
+        self._traj_log_prob = self._traj_one_episode = False
 
     @property
     def trajectory(self):
@@ -1029,7 +1038,11 @@ class BatchedManipulationEnv:
         float32 and ``terminated`` / ``truncated`` / ``finished`` [k, n] bool.  After
         ``enable_trajectory(steps, final_observation=True)`` also ``final_observation`` [k, n, 45]: the observation that
         ended the episode, valid where ``finished`` is True (other entries are not written).  With ``one_episode=True``
-        an env's rows after the step that ended its episode are not written.  The next ``rollout()`` overwrites them."""
+        an env's rows after the step that ended its episode are not written.  The next ``rollout()`` overwrites them.
+        After ``enable_trajectory(steps, policy_record=True)`` also ``policy_obs`` [k, n, 45] (the network's input at
+        step t, bit for bit), ``raw_action`` [k, n, 15] (mean + std * z before the clip; ``action`` is its clip) and,
+        when the policy has an ``action_std``, ``log_prob`` [k, n]: log N(raw_action; mean, diag(std^2)) summed over
+        the 15 joints, the density of the unclipped sample."""
         if self._traj is None:
             raise RuntimeError("enable_trajectory() first")
         k, n, tr = self._traj_rows, self.num_envs, self._traj
@@ -1038,6 +1051,11 @@ class BatchedManipulationEnv:
             out["final_observation"] = tr["final_observation"][:k, :, :n].transpose(1, 2)
         if self._traj_has_action:
             out["action"] = tr["action"][:k, :, :n].transpose(1, 2)
+        if "policy_obs" in tr:
+            out["policy_obs"] = tr["policy_obs"][:k, :, :n].transpose(1, 2)
+            out["raw_action"] = tr["raw_action"][:k, :, :n].transpose(1, 2)
+            if self._traj_log_prob:
+                out["log_prob"] = tr["log_prob"][:k, :n]
         for name in ("terminated", "truncated", "finished"):
             out[name] = tr[name][:k, :n].view(torch.bool)
         return out
@@ -1086,7 +1104,9 @@ class BatchedManipulationEnv:
         ``steps``.
         ``policy`` may also be an ``MlpPolicy``: every env acts on the observation ``step()`` would return for its
         current state (with the env's observation noise where its ``sigma_obs`` > 0), through the network, in the same
-        launch (``dexsim_rollout_mlp``); recorded actions are the policy's, before dynamics noise."""
+        launch (``dexsim_rollout_mlp``); recorded actions are the policy's, before dynamics noise.  After
+        ``enable_trajectory(steps, policy_record=True)`` only an ``MlpPolicy`` may act, and its ``action_std`` entries
+        must be finite and positive."""
         if self._next_step:
             raise NotImplementedError("rollout() resets finished episodes in the same step; it does not support "
                                       "autoreset_mode='next_step'")
@@ -1101,8 +1121,13 @@ class BatchedManipulationEnv:
                 raise ValueError("an MlpPolicy rollout takes no actions and no learner noise")
             if mlp.device != self.device:
                 raise ValueError(f"the policy lives on {mlp.device}, the env on {self.device}")
+            if self._traj is not None and "policy_obs" in self._traj and mlp.action_std is not None \
+                    and not mlp.std_has_density:
+                raise ValueError("policy_record needs action_std entries that are finite and > 0")
             kind = None
         else:
+            if self._traj is not None and "policy_obs" in self._traj:
+                raise ValueError("policy_record records an MlpPolicy's data: rollout with policy=MlpPolicy")
             kind = {"external": _L.POLICY_EXTERNAL, "random": _L.POLICY_RANDOM, "heuristic": _L.POLICY_HEURISTIC,
                     "learner": _L.POLICY_LEARNER}[policy]
         if kind == _L.POLICY_LEARNER and self._learner_mean is None:
@@ -1152,12 +1177,18 @@ class BatchedManipulationEnv:
                                                  tr["terminated"].data_ptr(), tr["truncated"].data_ptr(),
                                                  tr["finished"].data_ptr(), tr["obs"].shape[0])
                     fo = tr["final_observation"].data_ptr() if "final_observation" in tr else None
-                _lib.check(self._lib.dexsim_rollout_mlp(
-                    C.byref(self._state), C.byref(p), self._ptr(self._groups_dev), self._ptr(self._goe), int(k_steps),
-                    C.byref(rio), C.byref(mlp._struct), None if traj is None else C.byref(traj), fo, self._stream()),
-                    "dexsim_rollout_mlp")
+                mlp_args = (C.byref(self._state), C.byref(p), self._ptr(self._groups_dev), self._ptr(self._goe),
+                            int(k_steps), C.byref(rio), C.byref(mlp._struct), None if traj is None else C.byref(traj), fo)
+                if traj is not None and "policy_obs" in tr:
+                    lp = tr["log_prob"].data_ptr() if mlp.action_std is not None else None
+                    prec = _lib.DexsimPolicyRecord(tr["policy_obs"].data_ptr(), tr["raw_action"].data_ptr(), lp)
+                    _lib.check(self._lib.dexsim_rollout_mlp_record(*mlp_args, C.byref(prec), self._stream()),
+                               "dexsim_rollout_mlp_record")
+                else:
+                    _lib.check(self._lib.dexsim_rollout_mlp(*mlp_args, self._stream()), "dexsim_rollout_mlp")
                 if traj is not None:
                     self._traj_rows, self._traj_has_action = int(k_steps), True
+                    self._traj_log_prob = mlp.action_std is not None
             elif self._traj is None:
                 _lib.check(self._lib.dexsim_rollout(*args, self._stream()), "dexsim_rollout")
             else:
@@ -1171,9 +1202,45 @@ class BatchedManipulationEnv:
                 else:
                     _lib.check(self._lib.dexsim_rollout_record(*args, C.byref(traj), self._stream()), "dexsim_rollout_record")
                 self._traj_rows, self._traj_has_action = int(k_steps), kind != _L.POLICY_EXTERNAL
+            if self._traj is not None:
+                self._traj_one_episode = bool(one_episode)
             self._rollout_steps += int(k_steps)
             self._spawned = True
         return self.counters, self.ret_sums
+
+    def gae(self, values, final_values, gamma, lam):
+        """Generalized advantage estimation over the last recorded ``rollout()``, in one kernel (``dexsim_gae``).
+        ``values`` [k+1, n]: V of the input of step t, row k the value after the last step; ``final_values`` [k, n]:
+        V(``final_observation``) of row t, read only where the row is finished and not terminated (truncation and the
+        loop bound bootstrap from it, termination does not).  Both float32 on the env's device.  Returns
+        ``(advantages, returns)``, each [k, n] float32; an advantage never runs across a finished row.  A
+        ``one_episode=True`` recording leaves rows unwritten and raises here."""
+        if self._traj is None or self._traj_rows == 0:
+            raise RuntimeError("gae() runs on a recorded rollout: enable_trajectory() and rollout() first")
+        if self._traj_one_episode:
+            raise RuntimeError("gae() needs every row written: the last recording was one_episode=True")
+        k, n, ld = self._traj_rows, self.num_envs, self.ld
+        padded = []
+        for name, t, rows in (("values", values, k + 1), ("final_values", final_values, k)):
+            if not isinstance(t, torch.Tensor) or t.dtype != torch.float32:
+                raise TypeError(f"{name} must be a float32 torch tensor")
+            if t.device != self.device:
+                raise ValueError(f"{name} lives on {t.device}, the env on {self.device}")
+            if tuple(t.shape) != (rows, n):
+                raise ValueError(f"{name} must be [{rows}, {n}], got {list(t.shape)}")
+            buf = torch.zeros(rows, ld, dtype=torch.float32, device=self.device)
+            buf[:, :n] = t
+            padded.append(buf)
+        adv = torch.empty(k, ld, dtype=torch.float32, device=self.device)
+        ret = torch.empty(k, ld, dtype=torch.float32, device=self.device)
+        tr = self._traj
+        traj = _lib.DexsimTrajectory(tr["obs"].data_ptr(), None, tr["reward"].data_ptr(), tr["terminated"].data_ptr(),
+                                     tr["truncated"].data_ptr(), tr["finished"].data_ptr(), tr["obs"].shape[0])
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.dexsim_gae(C.byref(traj), n, ld, k, padded[0].data_ptr(), padded[1].data_ptr(),
+                                            C.c_float(gamma), C.c_float(lam), adv.data_ptr(), ret.data_ptr(),
+                                            self._stream()), "dexsim_gae")
+        return adv[:, :n], ret[:, :n]
 
     # ------------------------------------------------------------------ misc API of the reference env
     def render(self):

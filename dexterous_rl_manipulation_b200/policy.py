@@ -39,12 +39,16 @@ class MlpPolicy:
         self.hidden, self.activation = hidden, activation
         self.params = params.to(self.device).contiguous().clone()       # a fresh allocation: 16-byte aligned
         self.action_std = None
+        # whether the policy has a Gaussian density (the log_prob of a policy record): action_std given, every entry
+        # finite and > 0 -- decided here, on the host, once
+        self.std_has_density = False
         if action_std is not None:
             std = torch.as_tensor(action_std, dtype=torch.float32).reshape(-1)
             if std.numel() == 1:
                 std = std.expand(15)
             if std.numel() != 15:
                 raise ValueError("action_std must be a scalar or hold 15 entries")
+            self.std_has_density = bool(torch.isfinite(std.cpu()).all()) and bool((std.cpu() > 0).all())
             self.action_std = torch.zeros(16, dtype=torch.float32, device=self.device)
             self.action_std[:15] = std.to(self.device)
         self._struct = _lib.DexsimMlpPolicy(

@@ -433,6 +433,60 @@ int dexsim_rollout_mlp(const DexsimState* st, const DexsimParams* p, const Dexsi
 int dexsim_mlp_policy_mean(const DexsimMlpPolicy* policy, const float* obs, int64_t n, int64_t ld, float* out,
                            void* stream);
 
+/* ---- behaviour-policy data for on-policy training ----------------------------------------------------------------
+ * What a PPO-style learner needs of the policy that acted in a dexsim_rollout_mlp call, recorded next to the trajectory:
+ * device arrays of traj->capacity rows laid out [row, field, ld] like DexsimTrajectory, row t holding step t of the call
+ * (244 bytes per env and row with all three).  Each may be NULL = not recorded. */
+typedef struct DexsimPolicyRecord {
+    float* obs;          /* [capacity, 45, ld]: the network's input at step t */
+    float* raw_action;   /* [capacity, 15, ld]: mean + std * z before the clip (= mean when action_std is NULL) */
+    float* log_prob;     /* [capacity, ld]: log-density of raw_action under N(mean, diag(std^2)) */
+} DexsimPolicyRecord;
+int dexsim_sizeof_policy_record(void);
+
+/* dexsim_rollout_mlp with a recording (traj required, final_obs optional) that also fills `prec`.  Row t of the call:
+ *   - obs: all 45 inputs the network saw at step t, bit for bit: the observation of the env's state before the step,
+ *     plus the stream-3 noise where its group has sigma_obs > 0 -- what dexsim_step returned before that step (its
+ *     io->noisy_obs where noise is on).  Where sigma_obs == 0 it equals traj->obs row t-1 (row 0: the state the call
+ *     starts from);
+ *   - raw_action: a_j = mean_j + std_j * z_j, the product and the sum rounded separately (= mean_j without action_std);
+ *     traj->action row t is clip(raw_action, -1, 1) bit for bit;
+ *   - log_prob: lp = fmaf(-0.5f, s, c) with s = the ascending fmaf chain from 0 of z_j * z_j (j = 0 .. 14) and
+ *     c = (float)(-S - 7.5 * L), S = the ascending double sum from 0 of log((double)std_j), L = 1.8378770664093453
+ *     (double log(2 pi)), every double operation rounded on its own; c is computed once per CTA (the device's double log
+ *     is within 1 ulp, so c is exact to float32 unless the double value lies within an ulp of a float32 rounding tie).
+ *     This is the density of the UNCLIPPED sample: the convention of PPO implementations that clip outside the
+ *     distribution.  A deterministic policy (action_std NULL) has no density: log_prob must then be NULL.
+ * As in traj, an env's rows after a one_episode stop are not written, nor columns n .. ld-1, nor rows k_steps ...  Every
+ * other output equals dexsim_rollout_mlp with the same traj and final_obs.
+ * Returns, before anything touches the device: DEXSIM_E_NULL when traj or prec is NULL; DEXSIM_E_ALIGN when an array of
+ * prec is not 16-byte aligned; DEXSIM_E_PARAM when log_prob is set and policy->action_std is NULL; and every error of
+ * dexsim_rollout_mlp.
+ * Available since ABI 5 without a version bump: look the symbol up to detect it. */
+int dexsim_rollout_mlp_record(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                              const uint16_t* group_of_env, int32_t k_steps, const DexsimRolloutIO* rio,
+                              const DexsimMlpPolicy* policy, const DexsimTrajectory* traj, float* final_obs /* or NULL */,
+                              const DexsimPolicyRecord* prec, void* stream);
+
+/* Generalized advantage estimation (Schulman et al. 2016) over rows 0 .. k_steps-1 of a recording, one thread per env,
+ * reading reward, terminated and finished from `traj` (any recording call's; not one made with rio->one_episode, whose
+ * unwritten rows it would read).  values [k_steps + 1, ld]: V of the input of step t, row k_steps = V after the last
+ * step; final_values [k_steps, ld]: V(final observation of row t), read only where finished && !terminated; advantages
+ * and returns [k_steps, ld].  Device float32, 16-byte aligned.  With gl = gamma * lam (one rounding), for t = k_steps-1
+ * down to 0, every operation rounded on its own (no contraction):
+ *   nv = finished ? (terminated ? 0 : final_values[t]) : values[t+1]
+ *   delta = (reward[t] + gamma * nv) - values[t]
+ *   A = finished ? delta : delta + gl * A_next          (A_next = 0 below row k_steps-1; a select, so a non-finite
+ *   advantages[t] = A;  returns[t] = A + values[t]       A_next does not cross an episode boundary)
+ * A terminated row does not bootstrap.  A truncated one, and one ended by the loop bound (p->loop_max_steps), bootstraps
+ * from final_values: traj->obs holds the next episode's first observation there.  Columns n .. ld-1 are not written.
+ * Returns, before anything touches the device: DEXSIM_E_NULL when traj, traj->reward / terminated / finished or an
+ * array is NULL; DEXSIM_E_SIZE when n < 0, ld < n, ld % 32 != 0, k_steps < 1 or k_steps > traj->capacity;
+ * DEXSIM_E_ALIGN when an array is not 16-byte aligned.
+ * Available since ABI 5 without a version bump: look the symbol up to detect it. */
+int dexsim_gae(const DexsimTrajectory* traj, int64_t n, int64_t ld, int32_t k_steps, const float* values,
+               const float* final_values, float gamma, float lam, float* advantages, float* returns, void* stream);
+
 /* ---- single-env read-back: everything the reference's step()/reset() return for env `index`, packed into
  *      64 float64 on the device (one launch + one small D2H instead of a dozen scalar reads):
  *      [0..44] obs (noisy_obs if given), 45 reward, 46 terminated, 47 truncated, 48 num_contacts, 49 step_count,
