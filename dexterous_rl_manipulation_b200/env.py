@@ -63,6 +63,20 @@ def _round_up(x, m):
     return (x + m - 1) // m * m
 
 
+def check_group_of_env(group_of_env, num_envs, num_groups):
+    """An env -> group map as the kernels read it: uint16 [num_envs], every entry in [0, num_groups).  Raises
+    ValueError otherwise.  The library cannot look inside the device copy, and an entry past the table makes every
+    kernel read its group and add to its counters out of bounds, so this is the only check there is."""
+    a = np.asarray(group_of_env.cpu() if isinstance(group_of_env, torch.Tensor) else group_of_env)
+    if a.dtype == np.bool_ or not np.issubdtype(a.dtype, np.integer):
+        raise ValueError(f"group_of_env must hold integers, got dtype {a.dtype}")
+    if a.shape != (int(num_envs),):
+        raise ValueError(f"group_of_env must have shape ({int(num_envs)},), got {a.shape}")
+    if a.min() < 0 or a.max() >= num_groups:
+        raise ValueError(f"group_of_env entries must lie in [0, {num_groups}), got {int(a.min())} .. {int(a.max())}")
+    return a.astype(np.uint16)
+
+
 def _reward_spec(reward_type, reward_shaping):
     """(reward_type code, weights) from the reference's constructor arguments
     (envs/manipulation_env.py:65-74; rewards/reward_shaping.py:20-25)."""
@@ -228,9 +242,10 @@ class BatchedManipulationEnv:
         self._noisy_obs = None
         self._obs_noise = None
         self._dyn_noise = None
-        self._goe = self._goe_ptr = None
+        self._goe = self._goe_ptr = self._goe_host = None
+        self._goe_max = -1                 # largest entry of the map, kept on the host to check a new table against
         if group_of_env is not None:
-            self._set_group_of_env(group_of_env)
+            self._set_group_of_env(check_group_of_env(group_of_env, self.num_envs, self.num_groups))
         self._groups_dev = None
         self.counters = None
         self.ret_sums = None
@@ -341,17 +356,27 @@ class BatchedManipulationEnv:
             self._groups_dirty = True
 
     def set_groups(self, configs, sigma_obs=0.0, sigma_dyn=0.0, group_of_env=None):
-        """Several curriculum / object / noise cells in one batch; env -> group is
-        ``group_of_env`` or ``global env id % len(configs)``."""
-        self._group_cfgs = list(configs)
+        """Several curriculum / object / noise cells in one batch; env -> group is ``group_of_env`` or
+        ``(global env id mod 2^32) % len(configs)``.  A ``group_of_env`` given earlier (here or to the constructor)
+        stays in force when this call gives none; every entry of the map in force must be < ``len(configs)``."""
+        cfgs = list(configs)
+        if not 1 <= len(cfgs) <= _L.MAX_GROUPS:
+            raise ValueError(f"need 1..{_L.MAX_GROUPS} groups, got {len(cfgs)}")
+        goe = None if group_of_env is None else check_group_of_env(group_of_env, self.num_envs, len(cfgs))
+        if goe is None and self._goe is not None and self._goe_max >= len(cfgs):
+            raise ValueError(f"the group_of_env in force names group {self._goe_max}, but only {len(cfgs)} groups "
+                             "are given: pass a new group_of_env with them")
+        self._group_cfgs = cfgs
         self._group_sigma = (sigma_obs, sigma_dyn)
-        if group_of_env is not None:
-            self._set_group_of_env(group_of_env)
+        if goe is not None:
+            self._set_group_of_env(goe)
         self._groups_dirty = True
 
-    def _set_group_of_env(self, group_of_env):
+    def _set_group_of_env(self, goe):
+        """Keep a map check_group_of_env() returned, on the host and on the device."""
+        self._goe_host, self._goe_max = goe, int(goe.max())
         self._goe = torch.zeros(self.ld, dtype=torch.int16, device=self.device)
-        self._goe[:self.num_envs] = torch.as_tensor(group_of_env).to(torch.int16).to(self.device)
+        self._goe[:self.num_envs] = torch.from_numpy(goe.view(np.int16)).to(self.device)
         self._goe_ptr = self._goe.data_ptr()
 
     @property
@@ -366,6 +391,8 @@ class BatchedManipulationEnv:
         if self._group_cfgs is None:
             so, sd = self.observation_noise_std, self.dynamics_noise_std
         table = group_table(cfgs, so, sd)
+        if self._goe is not None and self._goe_max >= len(cfgs):       # every kernel would index past the table
+            raise ValueError(f"group_of_env names group {self._goe_max} of a {len(cfgs)}-group table")
         # noise cells of a multi-group batch (group_sigma_*): step() draws them in-kernel with each env's group value
         self._group_noise = (self._group_cfgs is not None and bool(np.any(np.asarray(so, np.float64) > 0.0)),
                              self._group_cfgs is not None and bool(np.any(np.asarray(sd, np.float64) > 0.0)))
@@ -407,8 +434,9 @@ class BatchedManipulationEnv:
         if self._group_cfgs is None:
             return self._curriculum_config
         if self._goe is not None:
-            return self._group_cfgs[int(self._goe[i])]
-        return self._group_cfgs[(self.env_gid0 + i) % len(self._group_cfgs)]
+            return self._group_cfgs[int(self._goe_host[i])]
+        # the kernels' row: the global id wraps at 2^32 like the Philox counter word
+        return self._group_cfgs[((self.env_gid0 + i) & 0xFFFFFFFF) % len(self._group_cfgs)]
 
     @property
     def object_position(self):

@@ -61,6 +61,14 @@ extern "C" {
 
 #define DEXSIM_MAX_GROUPS 256
 
+/* group_of_env, the env -> group map every entry point that takes `groups` also takes:
+ *   - a device array of uint16 with one entry per env; entries n .. ld-1 are never read;
+ *   - every entry must be < num_groups.  The library does not check this (it cannot look inside a device array
+ *     without a copy), and a larger entry makes the kernels read the group row and add to the counters and
+ *     return sums out of bounds;
+ *   - NULL means env i belongs to group (uint32_t)(env_gid0 + i) % num_groups: the global id wraps at 2^32, like
+ *     the Philox counter word. */
+
 /* policy kinds (policies/random_policy.py:40, policies/heuristic_policy.py:55-62) */
 #define DEXSIM_POLICY_EXTERNAL 0
 #define DEXSIM_POLICY_RANDOM 1

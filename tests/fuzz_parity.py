@@ -211,7 +211,7 @@ while time.time() < t_end:
     K = int(rng.integers(1, 260))
     gid0 = int(rng.choice([0, 5, 2 ** 31 - 50_000, 2 ** 32 - 30_000]))
     seed = int(rng.integers(0, 2 ** 63))
-    n_groups = int(rng.integers(1, 5))
+    n_groups = int(rng.choice([1, 2, 3, 4, 16, 17, 64, 65, 255, 256]))     # both sides of the 16 / 64 staging limits
     cfgs = []
     for _ in range(n_groups):
         kw = dict(object_size=float(rng.uniform(0.01, 0.3)), object_mass=float(rng.uniform(0.01, 2.0)),
@@ -226,21 +226,22 @@ while time.time() < t_end:
             kw["spawn_z_range"] = (0.0, float(rng.uniform(0.0, 0.3)))
         cfgs.append(CC(**kw))
     n_env = max(n, 2)
+    goe = rng.integers(0, n_groups, n_env).astype(np.uint16) if rng.integers(2) else None   # explicit env -> group map
     env = dx.BatchedManipulationEnv(n_env, "cuda", max_episode_steps=max_steps, reward_type="dense" if dense else "sparse",
-                                    track_episodes=True, groups=cfgs, seed=seed, env_gid0=gid0)
+                                    track_episodes=True, groups=cfgs, seed=seed, env_gid0=gid0, group_of_env=goe)
     env.reset(seed=seed)
     ob = oracle.OracleBatch(n_env, dense=dense, max_episode_steps=max_steps)
     groups = np.concatenate([oracle.make_group(c) for c in cfgs])
-    gidx = [((gid0 + i) & 0xFFFFFFFF) % n_groups for i in range(n_env)]
+    gidx = [((gid0 + i) & 0xFFFFFFFF) % n_groups if goe is None else int(goe[i]) for i in range(n_env)]
     draws = [oracle.reset_draws(seed, (gid0 + i) & 0xFFFFFFFF, 0, groups[gidx[i]:gidx[i] + 1]) for i in range(n_env)]
     ob.reset_predrawn(np.stack([d[0] for d in draws]), np.array([d[1] for d in draws]), np.array([d[2] for d in draws]),
                       np.array([d[3] for d in draws]), np.stack([d[4] for d in draws]))
     desc = dict(case=case, n=n_env, dense=dense, respawn=respawn, policy=policy, max_steps=max_steps, loop_max=loop_max, K=K,
-                gid0=gid0, groups=n_groups)
+                gid0=gid0, groups=n_groups, group_map=goe is not None)
     assert np.array_equal(env._obs[:, :n_env].t().cpu().numpy(), ob.observation()), ("reset", desc)
     env.rollout(K, policy=policy, respawn=respawn, loop_max_steps=loop_max)
     cnt_o, rs_o = ob.rollout(groups, K, seed, policy_kind=1 if policy == "random" else 2, respawn=respawn, env_gid0=gid0,
-                             loop_max_steps=loop_max)
+                             group_of_env=goe, loop_max_steps=loop_max)
     cnt = env.counters.cpu().numpy()
     ok = (np.array_equal(cnt[:, :16], cnt_o[:, :16]) and np.array_equal(cnt[:, 17], cnt_o[:, 17])
           and np.array_equal(env._obs[:, :n_env].t().cpu().numpy(), ob.observation(), equal_nan=True)
