@@ -119,7 +119,7 @@ EXPORTS = (
     "dexsim_reset_philox", "dexsim_step", "dexsim_rollout", "dexsim_rollout_record", "dexsim_rollout_record_final",
     "dexsim_sizeof_trajectory", "dexsim_sizeof_mlp_policy", "dexsim_rollout_mlp", "dexsim_mlp_policy_mean",
     "dexsim_sizeof_policy_record", "dexsim_rollout_mlp_record", "dexsim_gae",
-    "dexsim_fill_policy_actions",
+    "dexsim_fill_policy_actions", "dexsim_fill_mlp_actions",
     "dexsim_fill_normal", "dexsim_classify_summary", "dexsim_step_host", "dexsim_pack_env", "dexsim_pack_env_tagged", "dexsim_step_single",
     "dexsim_step_final", "dexsim_step_host_final", "dexsim_step_next_reset",
     "dexsim_expand_contact_rows",
@@ -177,6 +177,8 @@ def lib():
     L.dexsim_gae.argtypes = [C.POINTER(DexsimTrajectory), i64, i64, i32, vp, vp, C.c_float, C.c_float, vp, vp, vp]
     L.dexsim_mlp_policy_mean.argtypes = [C.POINTER(DexsimMlpPolicy), vp, i64, i64, vp, vp]
     L.dexsim_fill_policy_actions.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, vp, vp]
+    L.dexsim_fill_mlp_actions.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), vp, vp,
+                                          C.POINTER(DexsimMlpPolicy), vp, vp]
     L.dexsim_fill_normal.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimParams), i32, i32, C.c_float, vp, vp]
     L.dexsim_pack_env.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimStepIO), i64, i32, vp, vp]
     L.dexsim_pack_env_tagged.argtypes = [C.POINTER(DexsimState), C.POINTER(DexsimStepIO), i64, i32, vp, C.c_double, vp]

@@ -929,6 +929,38 @@ mlp_mean_kernel(const MlpArgs m, const float* __restrict__ obs, const int64_t n,
     for (int j = 0; j < NJ; ++j) out[j * ld + i] = mean[j];
 }
 
+// dexsim_fill_mlp_actions: the action the MLP branch of rollout_kernel takes in each env's current state, from the same
+// device functions in the same order (input, mean, stream-4 exploration keyed by the current step count, clip).  It
+// reads the state and writes nothing but out[0..14][i], i < n.  Two resident CTAs per SM, as in the rollout: uncapped, the
+// env registers plus the 16 + 15 accumulators take 165 registers, one CTA per SM.
+__global__ void __launch_bounds__(256, 2)
+fill_mlp_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
+                const uint16_t* __restrict__ group_of_env, const MlpArgs m, float* __restrict__ out) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float* sw = reinterpret_cast<float*>(smem_raw);
+    mlp_stage(m, sw);
+    __syncthreads();
+    const int64_t n = st.n, ld = st.ld;
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int64_t gid64 = p.env_gid0 + i;
+    const uint32_t gid = (uint32_t)gid64;
+    const float sigma_obs = groups[group_index(group_of_env, i, gid64, p.num_groups)].sigma_obs;
+    EnvRegs e;
+    load_env(st, i, e);
+    const uint32_t episode = st.episode[i];
+    float a[NJ];
+    mlp_mean(m, sw, sw + m.scratch_off + threadIdx.x, (int)blockDim.x, MlpEnvInput{e, p.seed, gid, episode, sigma_obs}, a);
+    if (m.action_std) {
+        float z[NJ];
+        normal_rows<NJ>(p.seed, gid, episode, (uint32_t)e.sc, STREAM_LEARNER_ACT, 1.0f, z);
+#pragma unroll
+        for (int j = 0; j < NJ; ++j) a[j] = __fadd_rn(a[j], __fmul_rn(sw[m.o_std + j], z[j]));
+    }
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) out[j * ld + i] = clip_f32(a[j], -1.0f, 1.0f);
+}
+
 // The rollout kernel receives the policy as the first element of its trailing pack: (MlpArgs) or (MlpArgs, trajectory).
 // The record_* calls forward past it.
 template <typename Tr> __device__ __forceinline__ void record_action(const MlpArgs&, const Tr& tr, int64_t ld, int t, int64_t i,
@@ -2026,6 +2058,26 @@ int dexsim_fill_policy_actions(const DexsimState* st, const DexsimParams* p, int
     if (st->n == 0) return 0;
     const int grid = (int)((st->n + 255) / 256 > 65535 ? 65535 : (st->n + 255) / 256);
     fill_policy_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(*st, *p, policy_kind, actions);
+    return cuda_rc(cudaGetLastError());
+}
+
+int dexsim_fill_mlp_actions(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                            const uint16_t* group_of_env, const DexsimMlpPolicy* policy, float* actions, void* stream) {
+    MlpArgs m;
+    int rc = mlp_args(policy, m);
+    if (rc) return rc;
+    rc = check_state(st);
+    if (rc) return rc;
+    rc = check_params(p, true, groups);
+    if (rc) return rc;
+    if (!actions) return DEXSIM_E_NULL;
+    if (st->n == 0) return 0;
+    const int64_t blocks = (st->n + 255) / 256;
+    if (blocks > 0x7FFFFFFFll) return DEXSIM_E_SIZE;
+    const size_t smem = mlp_smem(m, 0, 256);
+    const cudaError_t e = cudaFuncSetAttribute(fill_mlp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return cuda_rc(e);
+    fill_mlp_kernel<<<(int)blocks, 256, smem, (cudaStream_t)stream>>>(*st, *p, groups, group_of_env, m, actions);
     return cuda_rc(cudaGetLastError());
 }
 

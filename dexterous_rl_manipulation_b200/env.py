@@ -1117,6 +1117,35 @@ class BatchedManipulationEnv:
         self.episode_log_overflow = produced - kept
         return rec
 
+    def policy_actions(self, policy):
+        """The action ``rollout(policy=policy)`` would take in every env's current state: a fresh ``[num_envs, 15]``
+        float32 tensor on the env's device, bit for bit, that ``step()`` accepts as it is.  ``policy`` is an
+        ``MlpPolicy`` (``dexsim_fill_mlp_actions``: the network on the observation ``step()`` returned, noise included,
+        plus its stream-4 exploration) or ``"random"`` / ``"heuristic"`` (``dexsim_fill_policy_actions``).  The call
+        reads the state and changes nothing.  In ``autoreset_mode="next_step"`` an env whose reset is pending gets an
+        action too, which the next ``step()`` ignores as it ignores any."""
+        mlp = isinstance(policy, MlpPolicy)
+        if not mlp and not (isinstance(policy, str) and policy in ("random", "heuristic")):
+            raise ValueError(f"policy must be an MlpPolicy, 'random' or 'heuristic', got {policy!r}")
+        if mlp and policy.device != self.device:
+            raise ValueError(f"the policy lives on {policy.device}, the env on {self.device}")
+        if not self._did_reset:
+            raise RuntimeError("call reset() before policy_actions()")
+        with torch.cuda.device(self.device):
+            self._sync_groups()
+            out = torch.empty(15, self.ld, dtype=torch.float32, device=self.device)
+            if mlp:
+                _lib.check(self._lib.dexsim_fill_mlp_actions(C.byref(self._state), C.byref(self._params),
+                                                             self._ptr(self._groups_dev), self._ptr(self._goe),
+                                                             C.byref(policy._struct), out.data_ptr(), self._stream()),
+                           "dexsim_fill_mlp_actions")
+            else:
+                kind = _L.POLICY_RANDOM if policy == "random" else _L.POLICY_HEURISTIC
+                _lib.check(self._lib.dexsim_fill_policy_actions(C.byref(self._state), C.byref(self._params), kind,
+                                                                out.data_ptr(), self._stream()),
+                           "dexsim_fill_policy_actions")
+            return out[:, :self.num_envs].t().contiguous()
+
     def rollout(self, k_steps, policy="random", actions=None, dyn_noise=None, loop_max_steps=None,
                 success_is_terminated=None, respawn=True, zero_counters=False, one_episode=False,
                 learner_act_noise=None, learner_upd_noise=None):

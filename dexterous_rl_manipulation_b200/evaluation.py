@@ -10,6 +10,10 @@ analysis run unchanged on the output:
   run_robustness_sweep_batched  -> RobustnessTester.run_robustness_sweep (:330-407)
   evaluate_seeds_batched        -> SeedVarianceAnalyzer.evaluate_with_seeds (evaluation/seed_variance.py:44-78)
 
+Wherever a policy name is taken, an ``MlpPolicy`` is accepted too: it acts inside the same one-episode fused launch
+(``rollout(policy=mlp)``), reads the (possibly noisy) observation, and its episodes are replayed step by step through
+``env.policy_actions``.  Each rank of a multi-GPU run passes its own ``MlpPolicy`` on its own device.
+
 Reset draws follow the reference exactly (``rng="numpy"``: env (object o, episode e) is seeded with
 ``seed + e`` like evaluator.py:222, so all objects share the same initial joint / spawn draws); the
 policy randomness is Philox, because the reference's policies draw from process-global NumPy state
@@ -22,6 +26,7 @@ import torch
 
 from . import _lib
 from .env import BatchedManipulationEnv
+from .policy import MlpPolicy
 
 FAILURE_TYPES = _lib.LABELS_METRICS
 
@@ -61,6 +66,23 @@ def aggregate_metrics(episodes: Sequence[Dict], max_steps: int = 200) -> Dict:
         "mean_failure_length": mean(f_len),
         "mean_failure_contacts": mean(f_con),
     }
+
+
+def _check_policy(policy, device):
+    """Refuse, before anything is launched, an ``MlpPolicy`` on another device than ``device``."""
+    if isinstance(policy, MlpPolicy):
+        dev = torch.device(device)
+        if dev.type == "cuda" and dev.index is None:
+            dev = torch.device("cuda", torch.cuda.current_device())
+        if policy.device != dev:
+            raise ValueError(f"the policy lives on {policy.device}, the env on {dev}")
+
+
+def _replay_policy(policy) -> Dict:
+    """The policy entries of an episode's ``replay`` record: the name, or "mlp" and the network's hash."""
+    if isinstance(policy, MlpPolicy):
+        return {"policy": "mlp", "policy_sha256": policy.sha256()}
+    return {"policy": policy}
 
 
 def _label(code, table):
@@ -124,8 +146,11 @@ def evaluate_heldout_set_batched(heldout_set, policy: str = "heuristic", num_epi
                                  actions=None, shard: Optional[Tuple[int, int]] = None) -> Dict:
     """All (object, episode) pairs of Evaluator.evaluate_heldout_set as ONE batch.
 
-    ``policy``: "heuristic" | "random" (fused, Philox) or "external" with ``actions`` of shape
-    [max_episode_steps, n_objects * n_episodes, 15] (env index = object * n_episodes + episode).
+    ``policy``: "heuristic" | "random" (fused, Philox), an ``MlpPolicy`` on ``device`` (fused, the network acting on
+    every env's observation, its exploration keyed by ``policy_seed``), or "external" with ``actions`` of shape
+    [max_episode_steps, n_objects * n_episodes, 15] (env index = object * n_episodes + episode).  Every episode's
+    ``replay`` entry holds what ``replay_episode`` needs; for an MLP it records ``"policy": "mlp"`` and the network's
+    ``policy_sha256``.
 
     Multi-GPU: with ``torch.distributed`` initialised (or an explicit ``shard=(rank, world_size)``) every rank
     runs a contiguous slice of the batch on its own GPU and the per-episode records are all-gathered, so every
@@ -133,6 +158,7 @@ def evaluate_heldout_set_batched(heldout_set, policy: str = "heuristic", num_epi
     unseeded run draws different episode seeds on every rank)."""
     import torch.distributed as dist
     from .distributed import shard_range
+    _check_policy(policy, device)
     objs = heldout_set.heldout_objects
     n_obj, n_eps = len(objs), int(num_episodes_per_object)
     n = n_obj * n_eps
@@ -159,6 +185,7 @@ def _heldout_result(heldout_set, recs, n_eps, seeds, policy, policy_seed, reward
     objs = heldout_set.heldout_objects
     n_obj = len(objs)
     env_seeds = [seeds[i % n_eps] for i in range(n_obj * n_eps)]
+    replay_policy = _replay_policy(policy)
     size, mass, fric = ([o.size for o in objs], [o.mass for o in objs], [o.friction for o in objs])
     all_results, object_results = [], {}
     for o in range(n_obj):
@@ -169,7 +196,7 @@ def _heldout_result(heldout_set, recs, n_eps, seeds, policy, policy_seed, reward
             d["object_idx"], d["episode"] = o, e
             # everything needed to re-run exactly this episode with full capture (replay_episode)
             d["replay"] = {"object_idx": o, "reset_seed": env_seeds[o * n_eps + e], "env_gid": int(rec["env_gid"]),
-                           "philox_episode": int(rec["episode"]), "policy": policy, "policy_seed": int(policy_seed),
+                           "philox_episode": int(rec["episode"]), **replay_policy, "policy_seed": int(policy_seed),
                            "reward_type": reward_type, "max_episode_steps": int(max_episode_steps)}
             obj_results.append(d)
             all_results.append(d)
@@ -224,12 +251,14 @@ def evaluate_with_noise_batched(eval_config, policy: str = "heuristic", observat
     (evaluation/robustness_tests.py:260,282; envs/manipulation_env.py:156-161); every episode is one
     fused launch in one-episode mode followed by the reference's own reset(seed + episode).  ``num_replicas``
     independent copies of that experiment run side by side (replica r is seeded with seed + 1000 r).
-    Dynamics noise is drawn in-kernel; observation noise cannot change the trajectory of a policy that
-    ignores observations (all shipped policies do, SURVEY.md 3.5) and is only recorded in the output.
+    Dynamics noise is drawn in-kernel.  Observation noise reaches an ``MlpPolicy``, which acts on the noisy
+    observation; the shipped in-kernel policies ("heuristic", "random") ignore observations (SURVEY.md 3.5), so
+    for them it cannot change the trajectory and is only recorded in the output.
     With ``torch.distributed`` initialised (or ``shard=(rank, world_size)``) the replicas are spread over the ranks
     and the records all-gathered; every rank returns the complete, GPU-count-independent result."""
     import torch.distributed as dist
     from .distributed import shard_range
+    _check_policy(policy, device)
     distributed = shard is None and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
     rank, world = shard if shard is not None else ((dist.get_rank(), dist.get_world_size()) if distributed else (0, 1))
     if world > 1 and seed is None:
@@ -293,32 +322,29 @@ def evaluate_seeds_batched(heldout_set, seeds: Sequence[int], policy="heuristic"
             for s in seeds}
 
 
-def replay_episode(eval_config, reset_seed: int, env_gid: int, philox_episode: int = 0, policy: str = "heuristic",
+def replay_episode(eval_config, reset_seed: int, env_gid: int, philox_episode: int = 0, policy="heuristic",
                    policy_seed: int = 0, reward_type: str = "dense", max_episode_steps: int = 200, device="cuda",
                    dynamics_noise_std: float = 0.0) -> Dict:
     """Re-run ONE episode of a fused rollout step by step with full capture.  Trajectories are a pure
     function of (reset draws, Philox key, global env id, episode index), so any episode a rollout logged can
     be reproduced bit for bit later -- this is how failed episodes get the ``states`` / ``actions`` /
     ``contact_history`` that FailureLogger.log_episode stores (evaluation/failure_logger.py:48-119), without
-    the rollout kernel having to write trajectories for a million envs.
+    the rollout kernel having to write trajectories for a million envs.  ``policy``: "heuristic", "random" or the
+    ``MlpPolicy`` that ran the episode; every action comes from ``env.policy_actions``.
     Returns {"states": [T+1 x obs[45]], "actions": [T x a[15]], "contacts": [T+1 count-encoded rows],
     "episode": per-episode dict} in the layout evaluation/evaluator.py:118-173 records."""
-    import ctypes as C
-    kind = {"random": _lib.POLICY_RANDOM, "heuristic": _lib.POLICY_HEURISTIC}[policy]
+    _check_policy(policy, device)
     env = BatchedManipulationEnv(2, device, max_episode_steps=max_episode_steps, reward_type=reward_type, rng="numpy",
                                  groups=[eval_config], seed=policy_seed, env_gid0=int(env_gid),
                                  dynamics_noise_std=dynamics_noise_std, reward_components=False)
     obs, info = env.reset(seed=[int(reset_seed), int(reset_seed)])
     env._episode.fill_(int(philox_episode))
-    act = torch.zeros(15, env.ld, device=env.device)
     states = [obs[0].cpu().numpy().copy()]
     n0 = int(info["num_contacts"][0])
     contacts = [[1.0 if i < n0 else 0.0 for i in range(5)]]
     actions, total, steps, success = [], 0.0, 0, False
     for _ in range(int(max_episode_steps)):
-        _lib.check(env._lib.dexsim_fill_policy_actions(C.byref(env._state), C.byref(env._params), kind, act.data_ptr(),
-                                                       env._stream()), "dexsim_fill_policy_actions")
-        a = act[:, :2].t().contiguous()
+        a = env.policy_actions(policy)
         obs, rew, te, tr, info = env.step(a)
         actions.append(a[0].cpu().numpy().copy())
         states.append(obs[0].cpu().numpy().copy())
@@ -335,17 +361,29 @@ def replay_episode(eval_config, reset_seed: int, env_gid: int, philox_episode: i
     return {"states": states, "actions": actions, "contacts": contacts, "episode": episode}
 
 
-def log_failures_batched(result: Dict, heldout_set, failure_logger, device="cuda") -> int:
+def log_failures_batched(result: Dict, heldout_set, failure_logger, device="cuda", policy=None) -> int:
     """Feed every failed episode of an ``evaluate_heldout_set_batched`` result to an (unchanged)
     FailureLogger, re-creating its full trajectory by deterministic replay; returns the number logged.
-    Mirrors the logging branch of Evaluator.evaluate_episode (evaluation/evaluator.py:97-185)."""
+    Mirrors the logging branch of Evaluator.evaluate_episode (evaluation/evaluator.py:97-185).
+    Episodes of an ``MlpPolicy`` are replayed with ``policy``, which must be that network: when the result holds failed
+    such episodes and ``policy`` is missing or its ``sha256()`` differs from the recorded one, ValueError is raised before
+    anything is launched."""
+    mlp_hashes = {ep["replay"]["policy_sha256"] for ep in result["all_episodes"]
+                  if not ep["success"] and "replay" in ep and ep["replay"]["policy"] == "mlp"}
+    if mlp_hashes:
+        if not isinstance(policy, MlpPolicy):
+            raise ValueError("the result holds failed MlpPolicy episodes: pass the policy that ran them (policy=...)")
+        _check_policy(policy, device)
+        if mlp_hashes != {policy.sha256()}:
+            raise ValueError("the policy given is not the network that ran the result's episodes (policy_sha256 differs)")
     logged = 0
     for ep in result["all_episodes"]:
-        if ep["success"] or "replay" not in ep or ep["replay"]["policy"] not in ("random", "heuristic"):
+        if ep["success"] or "replay" not in ep or ep["replay"]["policy"] not in ("random", "heuristic", "mlp"):
             continue
         rp = ep["replay"]
         cfg = heldout_set.get_eval_config(rp["object_idx"])
-        tr = replay_episode(cfg, rp["reset_seed"], rp["env_gid"], rp["philox_episode"], rp["policy"], rp["policy_seed"],
+        tr = replay_episode(cfg, rp["reset_seed"], rp["env_gid"], rp["philox_episode"],
+                            policy if rp["policy"] == "mlp" else rp["policy"], rp["policy_seed"],
                             rp["reward_type"], rp["max_episode_steps"], device)
         if tr["episode"]["episode_steps"] != ep["episode_steps"] or tr["episode"]["final_contacts"] != ep["final_contacts"]:
             raise RuntimeError("replay diverged from the logged episode")

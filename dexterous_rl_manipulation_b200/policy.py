@@ -6,6 +6,7 @@
 returns the network's output for given observations with the rollout's arithmetic (include/dexsim.h).
 """
 import ctypes as C
+import hashlib
 
 import torch
 
@@ -91,6 +92,15 @@ class MlpPolicy:
             params = torch.cat([t.detach().to(torch.float32).reshape(-1).cpu()
                                 for m in linears for t in (m.weight, m.bias)])
         return params, hidden, "relu" if kinds == {nn.ReLU} else "tanh"
+
+    def sha256(self):
+        """Hex SHA-256 of what fixes the policy's actions: the hidden widths, the activation, the packed parameters and
+        ``action_std`` (or its absence).  Evaluation results carry it so that a saved result can be tied to its
+        network, and replays refuse a different one."""
+        h = hashlib.sha256(repr((self.hidden, self.activation)).encode())
+        h.update(self.params.cpu().numpy().tobytes())
+        h.update(b"std:" + self.action_std[:15].cpu().numpy().tobytes() if self.action_std is not None else b"no std")
+        return h.hexdigest()
 
     def mean(self, obs):
         """The network's output for ``obs`` [n, 45] (any device, cast to float32): [n, 15] on the policy's device,

@@ -39,10 +39,12 @@ def mlp(out, hidden=(64, 64)):
 
 
 def train(envs=131072, iters=40, steps=50, sigma_obs=(0.0, 0.02, 0.05), seed=0, epochs=4, minibatches=4, lr=3e-4,
-          gamma=0.99, lam=0.95, clip=0.2, max_episode_steps=200, device="cuda", log=print):
+          gamma=0.99, lam=0.95, clip=0.2, max_episode_steps=200, device="cuda", log=print, save=None):
     """Run PPO; returns one dict per iteration: mean episode return, surrogate / value losses of every minibatch,
     ``max_abs_log_ratio0`` (max |log pi(raw_action | policy_obs) - log_prob| over the batch before the first update:
-    0 up to float32 rounding, since the torch actor and the kernel evaluate the same network) and wall-clock seconds."""
+    0 up to float32 rounding, since the torch actor and the kernel evaluate the same network) and wall-clock seconds.
+    ``save``: a path to which the trained actor's ``state_dict`` and ``log_std`` are written after the last iteration
+    (``torch.save``; ``examples/evaluate_mlp.py`` loads it)."""
     torch.manual_seed(seed)
     groups = [dx.CurriculumConfig.easy()] * len(sigma_obs)
     env = dx.BatchedManipulationEnv(envs, device, reward_type="dense", max_episode_steps=max_episode_steps,
@@ -98,6 +100,8 @@ def train(envs=131072, iters=40, steps=50, sigma_obs=(0.0, 0.02, 0.05), seed=0, 
         if log:
             log(f"iter {it:3d}  episodes {episodes:8d}  mean return {mean_return:9.3f}  pg {pg_losses[-1]:+.4f}  "
                 f"v {v_losses[-1]:.4f}  |log ratio0| {max_abs_log_ratio0:.1e}  {stats['seconds']:.2f} s")
+    if save:
+        torch.save({"actor": {k: v.cpu() for k, v in actor.state_dict().items()}, "log_std": log_std.detach().cpu()}, save)
     return history
 
 
@@ -109,8 +113,9 @@ def main(argv=None):
     ap.add_argument("--sigma-obs", type=float, nargs="+", default=[0.0, 0.02, 0.05],
                     help="observation-noise std of each env group (env i is in group i %% len)")
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--save", metavar="PATH", help="write the trained actor and log_std here (torch.save)")
     args = ap.parse_args(argv)
-    train(args.envs, args.iters, args.steps, tuple(args.sigma_obs), args.seed)
+    train(args.envs, args.iters, args.steps, tuple(args.sigma_obs), args.seed, save=args.save)
 
 
 if __name__ == "__main__":

@@ -441,6 +441,22 @@ int dexsim_rollout_mlp(const DexsimState* st, const DexsimParams* p, const Dexsi
 int dexsim_mlp_policy_mean(const DexsimMlpPolicy* policy, const float* obs, int64_t n, int64_t ld, float* out,
                            void* stream);
 
+/* The action dexsim_rollout_mlp would take in every env's current state, bit for bit, for stepping with dexsim_step
+ * (Gymnasium-style loops, next-step auto-reset, deterministic replay of a logged episode).  For env i < st->n:
+ * actions[j][i] = clip(mean_j + std_j * z_j, -1, 1) (clip(mean_j, -1, 1) with action_std NULL), the input being the
+ * observation of the current state plus the stream-3 noise where the env's group (group_of_env[i], or with a NULL map
+ * ((uint32_t)(p->env_gid0 + i)) % p->num_groups) has sigma_obs > 0, and z the stream-4 normals keyed by the env's current
+ * (episode, step count).  `actions` is a device float32 array [15, ld].  The call only reads the state: it writes
+ * nothing but actions[0..14][0..n-1] -- no state array, no column n .. ld-1, no counter.
+ * Returns, before anything touches the device: DEXSIM_E_NULL / E_PARAM / E_ALIGN for the policy as dexsim_rollout_mlp;
+ * every error of the state, the params and the group table that dexsim_rollout_mlp returns (DEXSIM_E_NULL for a NULL st,
+ * p or groups, DEXSIM_E_SIZE for a bad n / ld, DEXSIM_E_GROUPS for num_groups outside 1 .. DEXSIM_MAX_GROUPS);
+ * DEXSIM_E_NULL for a NULL actions.
+ * Available since ABI 5 without a version bump: look the symbol up to detect it. */
+int dexsim_fill_mlp_actions(const DexsimState* st, const DexsimParams* p, const DexsimGroup* groups,
+                            const uint16_t* group_of_env, const DexsimMlpPolicy* policy,
+                            float* actions /* [15, ld] */, void* stream);
+
 /* ---- behaviour-policy data for on-policy training ----------------------------------------------------------------
  * What a PPO-style learner needs of the policy that acted in a dexsim_rollout_mlp call, recorded next to the trajectory:
  * device arrays of traj->capacity rows laid out [row, field, ld] like DexsimTrajectory, row t holding step t of the call
