@@ -230,6 +230,15 @@ __device__ __forceinline__ float obs_entry(const EnvRegs& e, const int row) {
     return ((e.cmask >> (row - DEXSIM_ROW_CONTACT)) & 1u) ? 1.0f : 0.0f;
 }
 
+// Observation noise (evaluation/robustness_tests.py:204-205) of the state `step` of an env: Philox block b of stream 3
+// gives the N(0, 1) draws z[0..3] of observation rows 4b .. 4b+3, the normals dexsim_fill_normal(STREAM_OBS) produces.
+__device__ __forceinline__ void obs_noise_block(uint64_t seed, uint32_t gid, uint32_t episode, uint32_t step, int b,
+                                                float* z) {
+    const U4 o = rng_block(seed, gid, episode, step, STREAM_OBS, (uint32_t)b);
+    normal_pair(o.x, o.y, z[0], z[1]);
+    normal_pair(o.z, o.w, z[2], z[3]);
+}
+
 }  // namespace dexsim
 
 #include "dexsim_step_tma.cuh"
@@ -464,10 +473,8 @@ step_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __res
             float* __restrict__ out = io.noisy_obs;
 #pragma unroll
             for (int b = 0; b < (NOBS + 3) / 4; ++b) {
-                const U4 o = rng_block(p.seed, (uint32_t)gid, episode, (uint32_t)e.sc, STREAM_OBS, (uint32_t)b);
                 float z[4];
-                normal_pair(o.x, o.y, z[0], z[1]);
-                normal_pair(o.z, o.w, z[2], z[3]);
+                obs_noise_block(p.seed, (uint32_t)gid, episode, (uint32_t)e.sc, b, z);
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
                     const int row = 4 * b + k;
@@ -683,10 +690,8 @@ finish_reset_kernel(const DexsimState st, const DexsimParams p, const DexsimGrou
             const float sigma = io.sigma_obs > 0.0f ? io.sigma_obs : groups[g].sigma_obs;
 #pragma unroll
             for (int b = 0; b < (NOBS + 3) / 4; ++b) {
-                const U4 o = rng_block(p.seed, (uint32_t)gid, episode, (uint32_t)e.sc, STREAM_OBS, (uint32_t)b);
                 float z[4];
-                normal_pair(o.x, o.y, z[0], z[1]);
-                normal_pair(o.z, o.w, z[2], z[3]);
+                obs_noise_block(p.seed, (uint32_t)gid, episode, (uint32_t)e.sc, b, z);
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
                     const int row = 4 * b + k;
@@ -710,15 +715,40 @@ finish_reset_kernel(const DexsimState st, const DexsimParams p, const DexsimGrou
 // Row t of a recorded rollout (DexsimTrajectory), stored from registers in three parts so that nothing of it stays live
 // across the step: the action as the policy produced it, the step's outcome, and the observation once the step and a
 // possible reset are done.  Every store of a warp is one 128-byte line of one row.
-__device__ __forceinline__ void record_action(const DexsimTrajectory& tr, int64_t ld, int t, int64_t i, const float* a) {
+//
+// A recording is a DexsimTrajectory, or one of two wrappers that hold it as `.tr`:
+//   TrajectoryFinal      also keeps the terminal observation of every episode it ends (dexsim_rollout_record_final):
+//                        `final_obs` [capacity, 45, ld] like tr.obs.
+//   TrajectoryPolicy<R>  a recording R plus the behaviour-policy record of the MLP rollout (dexsim_rollout_mlp_record).
+// Each is a distinct type, so that it instantiates rollout_kernel anew and the instantiations without it keep their code:
+// the hooks of what a type lacks compile to nothing (if constexpr).
+struct TrajectoryFinal {
+    DexsimTrajectory tr;
+    float* final_obs;
+};
+template <typename Tr> struct TrajectoryPolicy {
+    Tr tr;
+    DexsimPolicyRecord pr;
+};
+template <typename Rec> struct is_policy_record : std::false_type {};
+template <typename Tr> struct is_policy_record<TrajectoryPolicy<Tr>> : std::true_type {};
+
+template <typename Rec> __device__ __forceinline__ const DexsimTrajectory& traj_of(const Rec& rec) {
+    if constexpr (std::is_same<Rec, DexsimTrajectory>::value) return rec;
+    else return traj_of(rec.tr);
+}
+
+template <typename Rec> __device__ __forceinline__ void record_action(const Rec& rec, int64_t ld, int t, int64_t i, const float* a) {
+    const DexsimTrajectory& tr = traj_of(rec);
     if (!tr.action) return;
     float* out = tr.action + (int64_t)t * NJ * ld + i;
 #pragma unroll
     for (int j = 0; j < NJ; ++j) out[j * ld] = a[j];
 }
 
-__device__ __forceinline__ void record_outcome(const DexsimTrajectory& tr, int64_t ld, int t, int64_t i, const StepResult& r,
-                                               bool done) {
+template <typename Rec> __device__ __forceinline__ void record_outcome(const Rec& rec, int64_t ld, int t, int64_t i,
+                                                                       const StepResult& r, bool done) {
+    const DexsimTrajectory& tr = traj_of(rec);
     const int64_t at = (int64_t)t * ld + i;
     tr.reward[at] = (float)r.total;
     tr.terminated[at] = r.terminated ? 1 : 0;
@@ -726,41 +756,23 @@ __device__ __forceinline__ void record_outcome(const DexsimTrajectory& tr, int64
     tr.finished[at] = done ? 1 : 0;
 }
 
-__device__ __forceinline__ void record_obs(const DexsimTrajectory& tr, int64_t ld, int t, int64_t i, const EnvRegs& e) {
-    float* out = tr.obs + (int64_t)t * DEXSIM_OBS * ld + i;
+template <typename Rec> __device__ __forceinline__ void record_obs(const Rec& rec, int64_t ld, int t, int64_t i, const EnvRegs& e) {
+    float* out = traj_of(rec).obs + (int64_t)t * DEXSIM_OBS * ld + i;
 #pragma unroll
     for (int row = 0; row < DEXSIM_OBS; ++row) out[row * ld] = obs_entry(e, row);
 }
-
-// A recording that also keeps the terminal observation of every episode it ends (dexsim_rollout_record_final):
-// `final_obs` [capacity, 45, ld] like tr.obs.  A distinct type, so that it instantiates rollout_kernel anew and the
-// DexsimTrajectory instantiations keep their code: for them record_final_obs is empty.
-struct TrajectoryFinal {
-    DexsimTrajectory tr;
-    float* final_obs;
-};
-
-__device__ __forceinline__ void record_action(const TrajectoryFinal& f, int64_t ld, int t, int64_t i, const float* a) {
-    record_action(f.tr, ld, t, i, a);
-}
-
-__device__ __forceinline__ void record_outcome(const TrajectoryFinal& f, int64_t ld, int t, int64_t i, const StepResult& r,
-                                               bool done) {
-    record_outcome(f.tr, ld, t, i, r, done);
-}
-
-__device__ __forceinline__ void record_obs(const TrajectoryFinal& f, int64_t ld, int t, int64_t i, const EnvRegs& e) {
-    record_obs(f.tr, ld, t, i, e);
-}
-
-__device__ __forceinline__ void record_final_obs(const DexsimTrajectory&, int64_t, int, int64_t, const EnvRegs&) {}
 
 // Called where the episode has ended and `e` still holds the state after the step, before any reset: the observation
 // dexsim_step_final returns in final_obs.  Only finished lanes store, so a warp's store covers its finished lanes.
-__device__ __forceinline__ void record_final_obs(const TrajectoryFinal& f, int64_t ld, int t, int64_t i, const EnvRegs& e) {
-    float* out = f.final_obs + (int64_t)t * DEXSIM_OBS * ld + i;
+template <typename Rec> __device__ __forceinline__ void record_final_obs(const Rec& rec, int64_t ld, int t, int64_t i,
+                                                                         const EnvRegs& e) {
+    if constexpr (is_policy_record<Rec>::value) {
+        record_final_obs(rec.tr, ld, t, i, e);
+    } else if constexpr (std::is_same<Rec, TrajectoryFinal>::value) {
+        float* out = rec.final_obs + (int64_t)t * DEXSIM_OBS * ld + i;
 #pragma unroll
-    for (int row = 0; row < DEXSIM_OBS; ++row) out[row * ld] = obs_entry(e, row);
+        for (int row = 0; row < DEXSIM_OBS; ++row) out[row * ld] = obs_entry(e, row);
+    }
 }
 
 // ---- MLP policy (dexsim_rollout_mlp, dexsim_mlp_policy_mean) -------------------------------------------------------
@@ -895,15 +907,24 @@ struct MlpEnvInput {
 #pragma unroll
         for (int k = 0; k < 4; ++k) x[k] = 4 * b + k < NOBS ? obs_entry(e, 4 * b + k) : 0.0f;
         if (sigma > 0.0f) {
-            const U4 o = rng_block(seed, gid, episode, (uint32_t)e.sc, STREAM_OBS, (uint32_t)b);
             float z[4];
-            normal_pair(o.x, o.y, z[0], z[1]);
-            normal_pair(o.z, o.w, z[2], z[3]);
+            obs_noise_block(seed, gid, episode, (uint32_t)e.sc, b, z);
 #pragma unroll
             for (int k = 0; k < 4; ++k) x[k] = __fadd_rn(x[k], __fmul_rn(sigma, z[k]));
         }
     }
 };
+
+// The MLP's action in the env state of `xin` before the clip: the mean, plus std * z where the policy has a std, with z
+// the stream-4 normals keyed by the current step count (left in z for the caller's log-density).
+__device__ __forceinline__ void mlp_action(const MlpArgs& m, float* sw, const MlpEnvInput& xin, float* a, float* z) {
+    mlp_mean(m, sw, sw + m.scratch_off + threadIdx.x, (int)blockDim.x, xin, a);
+    if (m.action_std) {
+        normal_rows<NJ>(xin.seed, xin.gid, xin.episode, (uint32_t)xin.e.sc, STREAM_LEARNER_ACT, 1.0f, z);
+#pragma unroll
+        for (int j = 0; j < NJ; ++j) a[j] = __fadd_rn(a[j], __fmul_rn(sw[m.o_std + j], z[j]));
+    }
+}
 
 // Inputs of dexsim_mlp_policy_mean: column i of an [45, ld] array
 struct MlpColumnInput {
@@ -929,10 +950,9 @@ mlp_mean_kernel(const MlpArgs m, const float* __restrict__ obs, const int64_t n,
     for (int j = 0; j < NJ; ++j) out[j * ld + i] = mean[j];
 }
 
-// dexsim_fill_mlp_actions: the action the MLP branch of rollout_kernel takes in each env's current state, from the same
-// device functions in the same order (input, mean, stream-4 exploration keyed by the current step count, clip).  It
-// reads the state and writes nothing but out[0..14][i], i < n.  Two resident CTAs per SM, as in the rollout: uncapped, the
-// env registers plus the 16 + 15 accumulators take 165 registers, one CTA per SM.
+// dexsim_fill_mlp_actions: the action the MLP branch of rollout_kernel takes in each env's current state, through the
+// same mlp_action and clip.  It reads the state and writes nothing but out[0..14][i], i < n.  Two resident CTAs per SM,
+// as in the rollout: uncapped, the env registers plus the 16 + 15 accumulators take 165 registers, one CTA per SM.
 __global__ void __launch_bounds__(256, 2)
 fill_mlp_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __restrict__ groups,
                 const uint16_t* __restrict__ group_of_env, const MlpArgs m, float* __restrict__ out) {
@@ -949,112 +969,76 @@ fill_mlp_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* _
     EnvRegs e;
     load_env(st, i, e);
     const uint32_t episode = st.episode[i];
-    float a[NJ];
-    mlp_mean(m, sw, sw + m.scratch_off + threadIdx.x, (int)blockDim.x, MlpEnvInput{e, p.seed, gid, episode, sigma_obs}, a);
-    if (m.action_std) {
-        float z[NJ];
-        normal_rows<NJ>(p.seed, gid, episode, (uint32_t)e.sc, STREAM_LEARNER_ACT, 1.0f, z);
-#pragma unroll
-        for (int j = 0; j < NJ; ++j) a[j] = __fadd_rn(a[j], __fmul_rn(sw[m.o_std + j], z[j]));
-    }
+    float a[NJ], z[NJ];
+    mlp_action(m, sw, MlpEnvInput{e, p.seed, gid, episode, sigma_obs}, a, z);
 #pragma unroll
     for (int j = 0; j < NJ; ++j) out[j * ld + i] = clip_f32(a[j], -1.0f, 1.0f);
 }
 
-// The rollout kernel receives the policy as the first element of its trailing pack: (MlpArgs) or (MlpArgs, trajectory).
-// The record_* calls forward past it.
-template <typename Tr> __device__ __forceinline__ void record_action(const MlpArgs&, const Tr& tr, int64_t ld, int t, int64_t i,
-                                                                     const float* a) { record_action(tr, ld, t, i, a); }
-template <typename Tr> __device__ __forceinline__ void record_outcome(const MlpArgs&, const Tr& tr, int64_t ld, int t, int64_t i,
-                                                                      const StepResult& r, bool done) {
-    record_outcome(tr, ld, t, i, r, done);
-}
-template <typename Tr> __device__ __forceinline__ void record_obs(const MlpArgs&, const Tr& tr, int64_t ld, int t, int64_t i,
-                                                                  const EnvRegs& e) { record_obs(tr, ld, t, i, e); }
-template <typename Tr> __device__ __forceinline__ void record_final_obs(const MlpArgs&, const Tr& tr, int64_t ld, int t,
-                                                                        int64_t i, const EnvRegs& e) {
-    record_final_obs(tr, ld, t, i, e);
-}
-
+// The rollout kernel's trailing pack is (), (recording), (MlpArgs) or (MlpArgs, recording); mlp_of and recording_of take
+// it apart (recording_of gives an empty NoRecording where the pack has no recording).
 template <typename... T> struct first_is_mlp : std::false_type {};
 template <typename... T> struct first_is_mlp<MlpArgs, T...> : std::true_type {};
 template <typename... T> __device__ __forceinline__ const MlpArgs& mlp_of(const MlpArgs& m, const T&...) { return m; }
+struct NoRecording {};
+__device__ __forceinline__ NoRecording recording_of() { return {}; }
+__device__ __forceinline__ NoRecording recording_of(const MlpArgs&) { return {}; }
+template <typename Rec> __device__ __forceinline__ const Rec& recording_of(const Rec& rec) { return rec; }
+template <typename Rec> __device__ __forceinline__ const Rec& recording_of(const MlpArgs&, const Rec& rec) { return rec; }
 
 // ---- behaviour-policy record (dexsim_rollout_mlp_record) --------------------------------------------------------------
-// A recording (DexsimTrajectory or TrajectoryFinal) plus what an on-policy learner needs of the policy that acted: the
-// network's input, the action before the clip and its log-density.  A distinct type, so that it instantiates
-// rollout_kernel anew and the existing MLP instantiations keep their code: for them the three hooks below are empty.
+// What an on-policy learner needs of the policy that acted, recorded by a TrajectoryPolicy: the network's input, the
+// action before the clip and its log-density.  For every other recording the three hooks below are empty.
 // The log-density's constant c = float32(-sum_j log(double std_j) - 7.5 log(2 pi)) is computed once per CTA into the
 // padding slot std[15] of the staged weights (the mean never reads it).
-template <typename Tr> struct TrajectoryPolicy {
-    Tr tr;
-    DexsimPolicyRecord pr;
-};
 constexpr double LOG_2PI = 1.8378770664093453;   // double(log(2 pi)), the constant of include/dexsim.h
 
-template <typename Tr> __device__ __forceinline__ void record_action(const TrajectoryPolicy<Tr>& f, int64_t ld, int t, int64_t i,
-                                                                     const float* a) { record_action(f.tr, ld, t, i, a); }
-template <typename Tr> __device__ __forceinline__ void record_outcome(const TrajectoryPolicy<Tr>& f, int64_t ld, int t,
-                                                                      int64_t i, const StepResult& r, bool done) {
-    record_outcome(f.tr, ld, t, i, r, done);
-}
-template <typename Tr> __device__ __forceinline__ void record_obs(const TrajectoryPolicy<Tr>& f, int64_t ld, int t, int64_t i,
-                                                                  const EnvRegs& e) { record_obs(f.tr, ld, t, i, e); }
-template <typename Tr> __device__ __forceinline__ void record_final_obs(const TrajectoryPolicy<Tr>& f, int64_t ld, int t,
-                                                                        int64_t i, const EnvRegs& e) {
-    record_final_obs(f.tr, ld, t, i, e);
-}
-
-// The hooks take the rollout kernel's whole trailing pack, (MlpArgs) or (MlpArgs, recording), and do nothing unless the
-// recording is a TrajectoryPolicy.
-__device__ __forceinline__ void stage_log_prob_const(const MlpArgs&, float*) {}
-template <typename Tr> __device__ __forceinline__ void stage_log_prob_const(const MlpArgs&, const Tr&, float*) {}
-template <typename Tr> __device__ __forceinline__ void stage_log_prob_const(const MlpArgs& m, const TrajectoryPolicy<Tr>& f,
-                                                                            float* sw) {
-    if (!f.pr.log_prob) return;                  // uniform over the CTA: every thread returns or every thread syncs
-    if (threadIdx.x == 0) {
-        double s = 0.0;
-        for (int j = 0; j < NJ; ++j) s = __dadd_rn(s, log((double)sw[m.o_std + j]));
-        sw[m.o_std + NJ] = (float)__dsub_rn(-s, __dmul_rn(7.5, LOG_2PI));
+template <typename Rec> __device__ __forceinline__ void stage_log_prob_const(const MlpArgs& m, const Rec& rec, float* sw) {
+    if constexpr (is_policy_record<Rec>::value) {
+        if (!rec.pr.log_prob) return;            // uniform over the CTA: every thread returns or every thread syncs
+        if (threadIdx.x == 0) {
+            double s = 0.0;
+            for (int j = 0; j < NJ; ++j) s = __dadd_rn(s, log((double)sw[m.o_std + j]));
+            sw[m.o_std + NJ] = (float)__dsub_rn(-s, __dmul_rn(7.5, LOG_2PI));
+        }
+        __syncthreads();
     }
-    __syncthreads();
 }
 
 // Row t of the record: the 45 inputs of the network (regenerated from the registers and stream 3, as the mean read them)
 // and the action before the clip.
-template <typename Tr> __device__ __forceinline__ void record_policy(const MlpArgs&, const Tr&, int64_t, int, int64_t,
-                                                                     const MlpEnvInput&, const float*) {}
-template <typename Tr> __device__ __forceinline__ void record_policy(const MlpArgs&, const TrajectoryPolicy<Tr>& f, int64_t ld,
-                                                                     int t, int64_t i, const MlpEnvInput& xin,
-                                                                     const float* raw) {
-    if (f.pr.obs) {
-        float* out = f.pr.obs + (int64_t)t * NOBS * ld + i;
+template <typename Rec> __device__ __forceinline__ void record_policy(const Rec& rec, int64_t ld, int t, int64_t i,
+                                                                      const MlpEnvInput& xin, const float* raw) {
+    if constexpr (is_policy_record<Rec>::value) {
+        if (rec.pr.obs) {
+            float* out = rec.pr.obs + (int64_t)t * NOBS * ld + i;
 #pragma unroll
-        for (int b = 0; b < (NOBS + 3) / 4; ++b) {
-            float x[4];
-            xin.chunk(b, x);
+            for (int b = 0; b < (NOBS + 3) / 4; ++b) {
+                float x[4];
+                xin.chunk(b, x);
 #pragma unroll
-            for (int k = 0; k < 4; ++k)
-                if (4 * b + k < NOBS) out[(4 * b + k) * ld] = x[k];
+                for (int k = 0; k < 4; ++k)
+                    if (4 * b + k < NOBS) out[(4 * b + k) * ld] = x[k];
+            }
         }
-    }
-    if (f.pr.raw_action) {
-        float* out = f.pr.raw_action + (int64_t)t * NJ * ld + i;
+        if (rec.pr.raw_action) {
+            float* out = rec.pr.raw_action + (int64_t)t * NJ * ld + i;
 #pragma unroll
-        for (int j = 0; j < NJ; ++j) out[j * ld] = raw[j];
+            for (int j = 0; j < NJ; ++j) out[j * ld] = raw[j];
+        }
     }
 }
 
 // log N(raw; mean, diag(std^2)) = c - 0.5 sum_j z_j^2, the sum an ascending fmaf chain from 0
-template <typename Tr> __device__ __forceinline__ void record_log_prob(const MlpArgs&, const Tr&, int64_t, int, int64_t,
-                                                                       const float*, const float*) {}
-template <typename Tr> __device__ __forceinline__ void record_log_prob(const MlpArgs&, const TrajectoryPolicy<Tr>& f, int64_t ld,
-                                                                       int t, int64_t i, const float* z, const float* std16) {
-    if (!f.pr.log_prob) return;
-    float s = 0.0f;
+template <typename Rec> __device__ __forceinline__ void record_log_prob(const Rec& rec, int64_t ld, int t, int64_t i,
+                                                                        const float* z, const float* std16) {
+    if constexpr (is_policy_record<Rec>::value) {
+        if (!rec.pr.log_prob) return;
+        float s = 0.0f;
 #pragma unroll
-    for (int j = 0; j < NJ; ++j) s = __fmaf_rn(z[j], z[j], s);
-    f.pr.log_prob[(int64_t)t * ld + i] = __fmaf_rn(-0.5f, s, std16[NJ]);
+        for (int j = 0; j < NJ; ++j) s = __fmaf_rn(z[j], z[j], s);
+        rec.pr.log_prob[(int64_t)t * ld + i] = __fmaf_rn(-0.5f, s, std16[NJ]);
+    }
 }
 
 constexpr int ROLLOUT_MIN_BLOCKS = 2;
@@ -1072,6 +1056,7 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
     constexpr bool MLP = first_is_mlp<Traj...>::value;
     static_assert(sizeof...(Traj) == (REC ? 1 : 0) + (MLP ? 1 : 0), "a recording rollout takes one trajectory");
     static_assert(!(MLP && LEARNER), "the MLP and the learner never share a launch");
+    const auto& rec = recording_of(traj...);
     const float* __restrict__ actions = rio.actions;
     const float* __restrict__ dyn_noise = rio.dyn_noise;
     int64_t* __restrict__ counters = rio.counters;
@@ -1097,7 +1082,7 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
         sh_mlp = reinterpret_cast<float*>(smem_raw + ((groups_bytes + 15) & ~(size_t)15));
         mlp_stage(mlp_of(traj...), sh_mlp);
         __syncthreads();
-        stage_log_prob_const(traj..., sh_mlp);
+        stage_log_prob_const(mlp_of(traj...), rec, sh_mlp);
     }
     const DexsimGroup* gtab = staged ? sh_groups : groups;
     unsigned long long* cnt_base = staged ? sh_cnt : reinterpret_cast<unsigned long long*>(counters);
@@ -1135,16 +1120,12 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
             float a[NJ];
             if constexpr (MLP) {                           // dexsim_rollout_mlp: the observation this state returns from step()
                 const MlpArgs& m = mlp_of(traj...);
-                mlp_mean(m, sh_mlp, sh_mlp + m.scratch_off + threadIdx.x, (int)blockDim.x,
-                         MlpEnvInput{e, p.seed, gid, episode, grp.sigma_obs}, a);
-                if (m.action_std) {
-                    float z[NJ];
-                    normal_rows<NJ>(p.seed, gid, episode, (uint32_t)e.sc, STREAM_LEARNER_ACT, 1.0f, z);
-#pragma unroll
-                    for (int j = 0; j < NJ; ++j) a[j] = __fadd_rn(a[j], __fmul_rn(sh_mlp[m.o_std + j], z[j]));
-                    if constexpr (REC) record_log_prob(traj..., ld, t, i, z, sh_mlp + m.o_std);
+                float z[NJ];
+                mlp_action(m, sh_mlp, MlpEnvInput{e, p.seed, gid, episode, grp.sigma_obs}, a, z);
+                if constexpr (REC) {
+                    if (m.action_std) record_log_prob(rec, ld, t, i, z, sh_mlp + m.o_std);
+                    record_policy(rec, ld, t, i, MlpEnvInput{e, p.seed, gid, episode, grp.sigma_obs}, a);
                 }
-                if constexpr (REC) record_policy(traj..., ld, t, i, MlpEnvInput{e, p.seed, gid, episode, grp.sigma_obs}, a);
 #pragma unroll
                 for (int j = 0; j < NJ; ++j) a[j] = clip_f32(a[j], -1.0f, 1.0f);
             } else if (LEARNER) {                          // SimpleLearner.select_action, policies/simple_learner.py:60-69
@@ -1163,7 +1144,7 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
             } else {
                 policy_action(p.seed, gid, episode, (uint32_t)e.sc, policy_kind, a);
             }
-            if constexpr (REC) record_action(traj..., ld, t, i, a);     // the policy's action, before dynamics noise
+            if constexpr (REC) record_action(rec, ld, t, i, a);     // the policy's action, before dynamics noise
             if (dyn_noise) {                               // pre-drawn, already scaled by sigma
 #pragma unroll
                 for (int j = 0; j < NJ; ++j)
@@ -1203,7 +1184,7 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
             epstats_push(es, e.sc - 1, r.n_c);
             if (rio.hist && rio.step_base + t < rio.hist_steps) rio.hist[(rio.step_base + t) * ld + i] = (uint8_t)r.n_c;
             const bool done = r.terminated || r.truncated || (p.loop_max_steps > 0 && e.sc >= p.loop_max_steps);
-            if constexpr (REC) record_outcome(traj..., ld, t, i, r, done);
+            if constexpr (REC) record_outcome(rec, ld, t, i, r, done);
             if (done) {
                 if (LEARNER) lbest = -INFINITY;              // policy.reset() before the next episode
                 EpisodeLog log;
@@ -1211,16 +1192,16 @@ rollout_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* __
                 log.capacity = rio.ep_log_capacity; log.t_end = (uint32_t)(rio.step_base + t);
                 if (rio.one_episode) {          // run_episode semantics: stop here, the caller resets
                     finish_episode(e, p, gid, episode, ep_return, es, r.terminated, r.n_c, cnt, rs, &log);
-                    if constexpr (REC) record_obs(traj..., ld, t, i, e);   // the terminal observation
-                    if constexpr (REC) record_final_obs(traj..., ld, t, i, e);
+                    if constexpr (REC) record_obs(rec, ld, t, i, e);   // the terminal observation
+                    if constexpr (REC) record_final_obs(rec, ld, t, i, e);
                     break;
                 }
-                if constexpr (REC) record_final_obs(traj..., ld, t, i, e); // the terminal observation, before the reset
+                if constexpr (REC) record_final_obs(rec, ld, t, i, e); // the terminal observation, before the reset
                 finish_and_reset(e, p, grp, gid, episode, ep_return, es, r.terminated, r.n_c, cnt, rs,
                                  size, mass, friction, &log);
                 params_dirty = true;
             }
-            if constexpr (REC) record_obs(traj..., ld, t, i, e);       // after the auto-reset, as step() returns it
+            if constexpr (REC) record_obs(rec, ld, t, i, e);       // after the auto-reset, as step() returns it
         }
         store_env_full(st, i, e);
         st.episode[i] = episode;
@@ -1302,7 +1283,7 @@ __global__ void resolve_ties_kernel(const DexsimParams p, const uint16_t* __rest
         int la, lb, tie;
         classify_summary(s, p.loop_max_steps > 0 ? p.loop_max_steps : p.max_episode_steps, p.success_threshold, la, lb, tie, &cv);
         if (rio.counters) {
-            const int g = group_of_env ? (int)group_of_env[i] : (int)(rec.env_gid % (uint32_t)p.num_groups);
+            const int g = group_index(group_of_env, i, rec.env_gid, p.num_groups);
             unsigned long long* cnt = reinterpret_cast<unsigned long long*>(rio.counters) + (int64_t)g * DEXSIM_NCOUNTERS;
             if (la != rec.label_metrics) {
                 if (rec.label_metrics != DEXSIM_LABEL_NONE) atomicAdd(&cnt[DEXSIM_CNT_LABEL_METRICS + rec.label_metrics], ~0ull);

@@ -79,7 +79,7 @@ rollout_split_kernel(const DexsimState st, const DexsimParams p, const DexsimGro
 
     const int64_t gid64 = p.env_gid0 + i;
     const uint32_t gid = (uint32_t)gid64;
-    const int g = group_of_env ? (int)group_of_env[i] : (int)((uint32_t)gid64 % (uint32_t)p.num_groups);
+    const int g = group_index(group_of_env, i, gid64, p.num_groups);
     const DexsimGroup& grp = groups[g];                      // read only at resets
     unsigned long long* cnt = rio.counters ? reinterpret_cast<unsigned long long*>(rio.counters) + (int64_t)g * DEXSIM_NCOUNTERS : nullptr;
     double* rs = (rio.ret_sums && rio.counters) ? rio.ret_sums + 2 * g : nullptr;

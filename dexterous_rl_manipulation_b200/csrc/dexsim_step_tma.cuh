@@ -357,7 +357,7 @@ step_tma_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* _
                     if (fused_dyn || fused_obs) {
                         episode = reinterpret_cast<const uint32_t*>(sp + OFF_EPISODE)[col];
                         if (io.sigma_dyn < 0.0f || io.sigma_obs < 0.0f)
-                            g = group_of_env ? (int)group_of_env[i] : (int)((uint32_t)gid % (uint32_t)p.num_groups);
+                            g = group_index(group_of_env, i, gid, p.num_groups);
                     }
                     if (io.dyn_noise) {
 #pragma unroll
@@ -382,7 +382,7 @@ step_tma_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* _
                 if constexpr (NEXT) {
                     if (pending) {
                         // the reset the previous step left for this env, instead of a step: the action is ignored
-                        g = group_of_env ? (int)group_of_env[i] : (int)((uint32_t)gid % (uint32_t)p.num_groups);
+                        g = group_index(group_of_env, i, gid, p.num_groups);
                         episode = reinterpret_cast<const uint32_t*>(sp + OFF_EPISODE)[col];     // load_episode is on with auto-reset
                         next_step_reset(e, p, groups[g], (uint32_t)gid, episode, st, i, r);
                         st.thr[i] = e.thr; st.damp[i] = e.damp;
@@ -420,7 +420,7 @@ step_tma_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* _
                     const bool done = r.terminated || r.truncated || (p.loop_max_steps > 0 && e.sc >= p.loop_max_steps);
                     if (p.auto_reset && done) {
                         // episode end on the owning lane (counters, labels)
-                        g = group_of_env ? (int)group_of_env[i] : (int)((uint32_t)gid % (uint32_t)p.num_groups);
+                        g = group_index(group_of_env, i, gid, p.num_groups);
                         episode = reinterpret_cast<const uint32_t*>(sp + OFF_EPISODE)[col];     // load_episode is on with auto-reset
                         unsigned long long* cnt = nullptr;
                         double* rs = nullptr;
@@ -504,10 +504,8 @@ step_tma_kernel(const DexsimState st, const DexsimParams p, const DexsimGroup* _
                     const int64_t gid = p.env_gid0 + i;
 #pragma unroll
                     for (int b = 0; b < (NOBS + 3) / 4; ++b) {
-                        const U4 o = rng_block(p.seed, (uint32_t)gid, episode, (uint32_t)e.sc, STREAM_OBS, (uint32_t)b);
                         float z[4];
-                        normal_pair(o.x, o.y, z[0], z[1]);
-                        normal_pair(o.z, o.w, z[2], z[3]);
+                        obs_noise_block(p.seed, (uint32_t)gid, episode, (uint32_t)e.sc, b, z);
 #pragma unroll
                         for (int q = 0; q < 4; ++q) {
                             const int row = 4 * b + q;
